@@ -2,6 +2,7 @@
 """bench.py -- Groth16 proofs/s (nzcp, BN254) on N B200s, one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--shape live|example|small] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): the nzcp_liveTest shape -- n = 2^20, 835 000 constraints, 880 001 wires,
 513 public signals, ~4.6 M A/B coefficients -- as a SYNTHETIC R1CS + satisfying witnesses (the real circuit cannot be
@@ -198,6 +199,18 @@ def quiet_stdout():
         os.dup2(2, 1)
 
 
+def dump_proofs(out_dir, proofs, prefix=""):
+    """--dump-outputs: the B proofs of one step as float64 arrays pi_a (B, 2, 8), pi_b (B, 2, 2, 8) and pi_c (B, 2, 8), in
+    the coordinate order of the proof bytes (include/nzcp_prover.h).  Each coordinate is a plain field element split into
+    8 little-endian 32-bit limbs, which float64 holds exactly, so two builds can be compared bit for bit.  The inputs
+    (synthetic key, witnesses, r, s) are seeded, so the same arguments give the same proofs."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    v = np.frombuffer(b"".join(proofs), dtype="<u4").reshape(len(proofs), 8, 8).astype(np.float64)
+    for name, a in (("pi_a", v[:, 0:2]), ("pi_b", v[:, 2:6].reshape(-1, 2, 2, 8)), ("pi_c", v[:, 6:8])):
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.ascontiguousarray(a))
+
+
 def emit(line):
     out = _REAL_STDOUT or sys.stdout
     out.write(json.dumps(line) + "\n")
@@ -221,6 +234,8 @@ def main():
     ap.add_argument("--extras-msm-log", type=int, default=24, help="configs[4]: log2 points of the split G1 MSM")
     ap.add_argument("--tune", action="append", default=[], metavar="KNOB=VALUE",
                     help="library tuning knob (include/nzcp_prover.h nzcp_tuning_set), e.g. prover_rounds_h=0")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the proofs of the last timed step to DIR/pi_a.npy, pi_b.npy, pi_c.npy (see dump_proofs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -264,8 +279,10 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def step_device():
-        pool.prove_device_many(d_wit, r=R_FIXED, s=S_FIXED)
+        last["proofs"] = pool.prove_device_many(d_wit, r=R_FIXED, s=S_FIXED)
 
     lat = []
     host_wtns = [p.numpy() for p in pinned]
@@ -315,6 +332,8 @@ def main():
     l0 = pool.launch_count()          # per-prover counters, summed over the pool's provers
     ms_dev = timed(step_device, args.steps)
     launches = pool.launch_count() - l0
+    if args.dump_outputs:
+        dump_proofs(args.dump_outputs, [o["proof"] for o in last["proofs"]], "rank%d_" % rank if world > 1 else "")
     ms_e2e = timed(lambda: step_e2e(True), args.steps)
     clocks = sampler.stop()
     step_e2e_pageable()

@@ -74,6 +74,23 @@ def test_round2_line_additions(path):
         assert 0 < c4["kernel_ms_max_over_ranks"] <= c4["ms"]
 
 
+def test_dump_outputs_hold_the_proofs_exactly(tmp_path):
+    """bench.py --dump-outputs: the float64 limb arrays give back every byte of every proof, in order."""
+    import random
+
+    import numpy as np
+
+    import bench
+    rng = random.Random(3)
+    proofs = [bytes(rng.randrange(256) for _ in range(256)) for _ in range(3)]
+    bench.dump_proofs(str(tmp_path), proofs)
+    a, b, c = (np.load(tmp_path / (n + ".npy")) for n in ("pi_a", "pi_b", "pi_c"))
+    assert a.dtype == b.dtype == c.dtype == np.float64
+    assert a.shape == c.shape == (3, 2, 8) and b.shape == (3, 2, 2, 8)
+    limbs = np.concatenate([x.reshape(3, -1) for x in (a, b, c)], axis=1)
+    assert [row.astype("<u4").tobytes() for row in limbs] == proofs
+
+
 def test_round2_reference_arm_has_the_same_config():
     ref = os.path.join(ROOT, "profiles", "r02_ref_n1.json")
     main = os.path.join(ROOT, "profiles", "r02_bench_default.json")
