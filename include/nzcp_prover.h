@@ -196,6 +196,21 @@ int nzcp_selftest(int device, uint64_t seed, uint32_t n_cases, uint32_t* n_bad);
 /* Element-wise Fr/Fq ops on the device, for limb-exact parity tests: op 0 mul, 1 add, 2 sub (3..5: the portable code paths), 6 inverse by division steps, 7 Fermat inverse (Montgomery-form in/out),
  * field 0 = Fr, 1 = Fq. */
 int nzcp_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n, int device);
+/* Device Fq / Fq2 arithmetic on n little-endian records, one thread per record, through the functions the kernels call.
+ * Fq2 = c0 | c1.  op (input / output bytes per record):
+ *   0 fp_mul_wide: a | b -> 512-bit a * b (64 / 64); a, b < 2^255
+ *   1 fp_redc_wide<Fq>: T -> T / 2^256 mod q (64 / 32); T < q * 2^256
+ *   2 f_mulsub(Fq), the lazy-reduction body, and 3 its eager form fp_sub(fp_mul, fp_mul): a | b | c | d -> a b - c d (128 / 32)
+ *   4 f_mul(Fq2) as the kernels call it, 5 f2_mul_inline: a | b -> a b (128 / 64)
+ *   6 f_sqr(Fq2) (64 / 64), 7 f_inv(Fq2) Fermat (64 / 64), 8 f_inv_fast(Fq2) division steps (64 / 64)
+ *   9 f_mulsub(Fq2): a | b | c | d -> a b - c d (256 / 64)
+ * Ops 2-9 take and return Montgomery form.  Ops 0 and 1 reject inputs outside their domain with NZCP_E_ARG. */
+int nzcp_arith_op(int op, const uint8_t* in, uint8_t* out, size_t n, int device);
+/* Device XYZZ group law on n records (x, y, zz, zzz Montgomery, as nzcp_msm_plan_run_partial writes them: 128 B for G1,
+ * 256 B for G2; zz == 0 is infinity).  op: 0 xyzz_add(a, b), b XYZZ; 1 xyzz_madd(a, b), b affine in the zkey layout;
+ * 2 xyzz_madd(a, -b); 3 xyzz_dbl(a), b unused; 4 xyzz_to_affine(a) -> affine records.  Ops 0-3 write XYZZ records.
+ * A madd operand equal to (0, 0) is rejected with NZCP_E_ARG. */
+int nzcp_curve_op(int g2, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n, int device);
 
 /* Tuning knobs for experiments and tests (process-wide, read when a plan is created / a run is launched):
  *   "msm_rounds"  batched-affine pair rounds per MSM: -1 = automatic (by size), 0..3 forced

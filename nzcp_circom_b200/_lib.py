@@ -84,6 +84,8 @@ SIGNATURES = {
     "nzcp_msm_var": (C.c_int, [_U8P, _U8P, C.c_size_t, C.c_int, C.c_int, C.c_int, _U8P, C.POINTER(C.c_float)]),
     "nzcp_selftest": (C.c_int, [C.c_int, C.c_uint64, C.c_uint32, C.POINTER(C.c_uint32)]),
     "nzcp_field_op": (C.c_int, [C.c_int, C.c_int, _U8P, _U8P, _U8P, C.c_size_t, C.c_int]),
+    "nzcp_arith_op": (C.c_int, [C.c_int, _U8P, _U8P, C.c_size_t, C.c_int]),
+    "nzcp_curve_op": (C.c_int, [C.c_int, C.c_int, _U8P, _U8P, _U8P, C.c_size_t, C.c_int]),
     "nzcp_intpipe_modes": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double)]),
     "nzcp_intpipe_bench": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double)]),
     "nzcp_pipe_probe": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_double)]),

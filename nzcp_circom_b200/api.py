@@ -362,6 +362,24 @@ def field_op(field, op, a, b, n, device=0):
     return bytes(out)
 
 
+# nzcp_arith_op record sizes in bytes, per op: (input, output)
+ARITH_IO = ((64, 64), (64, 32), (128, 32), (128, 32), (128, 64), (128, 64), (64, 64), (64, 64), (64, 64), (256, 64))
+
+
+def arith_op(op, data, n, device=0):
+    """Device Fq / Fq2 arithmetic on n little-endian records (include/nzcp_prover.h nzcp_arith_op) -> output records."""
+    out = bytearray(ARITH_IO[op][1] * n)
+    check(_lib.load().nzcp_arith_op(int(op), addr(data), addr(out), int(n), int(device)))
+    return bytes(out)
+
+
+def curve_op(g2, op, a, b, n, device=0):
+    """Device XYZZ group law on n records (include/nzcp_prover.h nzcp_curve_op) -> XYZZ records, affine for op 4."""
+    out = bytearray((128 if g2 else 64) * n * (1 if op == 4 else 2))
+    check(_lib.load().nzcp_curve_op(int(bool(g2)), int(op), addr(a), addr(b), addr(out), int(n), int(device)))
+    return bytes(out)
+
+
 def intpipe_bench(device=0, iters=4096):
     """-> dict(imad_wide_per_s, imad_lo_per_s, fq_mul_per_s, sm_count): the integer-pipe roofline denominators."""
     out = (C.c_double * 4)()

@@ -78,6 +78,71 @@ __global__ void curve_op_kernel(const Affine<F>* a, const Affine<F>* b, Affine<F
   out[i] = xyzz_to_affine(acc);
 }
 
+// Record sizes (bytes) of nzcp_arith_op, per op: in, out.
+static const int kArithIn[10] = {64, 64, 128, 128, 128, 128, 64, 64, 64, 256};
+static const int kArithOut[10] = {64, 32, 32, 32, 64, 64, 64, 64, 64, 64};
+
+// One case per thread through the exact device functions the kernels call (the lazy-reduction bodies, the non-inlined
+// Fq2 product / square, the device inversions), so the suite can pin them limb for limb against a big-integer reference.
+__global__ void arith_op_kernel(int op, const uint32_t* in, uint32_t* out, size_t n, int in_w, int out_w) {
+#if defined(__CUDA_ARCH__)   // fp_mul_wide / fp_redc_wide exist only in the device pass
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t* x = in + i * in_w;
+  uint32_t* y = out + i * out_w;
+  auto fq = [&](int k) { return *reinterpret_cast<const Fq*>(x + 8 * k); };
+  auto fq2 = [&](int k) { return Fq2{fq(2 * k), fq(2 * k + 1)}; };
+  Fq r1;
+  Fq2 r2;
+  switch (op) {
+    case 0: fp_mul_wide(y, x, x + 8); return;
+    case 1: fp_redc_wide<FqParams>(y, x); return;
+    case 2: r1 = f_mulsub(fq(0), fq(1), fq(2), fq(3)); break;
+    case 3: r1 = fp_sub(fp_mul(fq(0), fq(1)), fp_mul(fq(2), fq(3))); break;
+    case 4: r2 = f_mul(fq2(0), fq2(1)); break;
+    case 5: r2 = f2_mul_inline(fq2(0), fq2(1)); break;
+    case 6: r2 = f_sqr(fq2(0)); break;
+    case 7: r2 = f_inv(fq2(0)); break;
+    case 8: r2 = f_inv_fast(fq2(0)); break;
+    default: r2 = f_mulsub(fq2(0), fq2(1), fq2(2), fq2(3)); break;
+  }
+  if (op <= 3) {
+    *reinterpret_cast<Fq*>(y) = r1;
+  } else {
+    *reinterpret_cast<Fq*>(y) = r2.c0;
+    *reinterpret_cast<Fq*>(y + 8) = r2.c1;
+  }
+#endif
+}
+
+// XYZZ group law on records: 0 add(a, b), 1 madd(a, affine b), 2 madd(a, -affine b), 3 dbl(a), 4 to_affine(a).
+template <class F>
+__global__ void xyzz_op_kernel(int op, const XYZZ<F>* a, const void* b, void* out, size_t n) {
+  size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  XYZZ<F> acc = a[i];
+  switch (op) {
+    case 0: xyzz_add(acc, reinterpret_cast<const XYZZ<F>*>(b)[i]); break;
+    case 1: xyzz_madd(acc, reinterpret_cast<const Affine<F>*>(b)[i], false); break;
+    case 2: xyzz_madd(acc, reinterpret_cast<const Affine<F>*>(b)[i], true); break;
+    case 3: acc = xyzz_dbl(acc); break;
+    default: reinterpret_cast<Affine<F>*>(out)[i] = xyzz_to_affine(acc); return;
+  }
+  reinterpret_cast<XYZZ<F>*>(out)[i] = acc;
+}
+
+template <class F>
+static void run_xyzz_op(int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n) {
+  const size_t xs = sizeof(XYZZ<F>), as = sizeof(Affine<F>);
+  const size_t bs = op == 0 ? xs : (op <= 2 ? as : 0), os = op == 4 ? as : xs;
+  DevBuf da(n * xs), db(n * bs), dout(n * os);
+  NZCP_CUDA(cudaMemcpy(da.p, a, n * xs, cudaMemcpyHostToDevice));
+  if (bs) NZCP_CUDA(cudaMemcpy(db.p, b, n * bs, cudaMemcpyHostToDevice));
+  xyzz_op_kernel<F><<<div_up(n, 128), 128>>>(op, da.as<XYZZ<F>>(), db.p, dout.p, n);
+  NZCP_LAUNCH_CHECK();
+  NZCP_CUDA(cudaMemcpy(out, dout.p, n * os, cudaMemcpyDeviceToHost));
+}
+
 template <class P>
 static uint32_t selftest_field(uint64_t seed, uint32_t n) {
   std::vector<Fp<P>> a(n), b(n);
@@ -653,6 +718,45 @@ int nzcp_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint8_t
       field_op_kernel<FqParams><<<div_up(n, 128), 128>>>(op, da.as<Fq>(), db.as<Fq>(), dout.as<Fq>(), n);
     NZCP_LAUNCH_CHECK();
     NZCP_CUDA(cudaMemcpy(out, dout.p, n * 32, cudaMemcpyDeviceToHost));
+  });
+}
+
+int nzcp_arith_op(int op, const uint8_t* in, uint8_t* out, size_t n, int device) {
+  return api_guard([&] {
+    if (!in || !out) throw ApiError(NZCP_E_ARG, "null argument");
+    if (op < 0 || op > 9) throw ApiError(NZCP_E_ARG, "bad op");
+    // ops 0 and 1 take raw integers: keep them inside the bounds their carry chains assume
+    for (size_t i = 0; i < n && op <= 1; i++) {
+      const uint32_t* w = reinterpret_cast<const uint32_t*>(in + 64 * i);
+      if (op == 0 && ((w[7] | w[15]) >> 31)) throw ApiError(NZCP_E_ARG, "fp_mul_wide operand >= 2^255");
+      if (op == 1 && fp_geq_mod<FqParams>(w + 8)) throw ApiError(NZCP_E_ARG, "fp_redc_wide input >= q * 2^256");
+    }
+    use_device(device);
+    if (!n) return;
+    const int iw = kArithIn[op], ow = kArithOut[op];
+    DevBuf din(n * iw), dout(n * ow);
+    NZCP_CUDA(cudaMemcpy(din.p, in, n * iw, cudaMemcpyHostToDevice));
+    arith_op_kernel<<<div_up(n, 128), 128>>>(op, din.as<uint32_t>(), dout.as<uint32_t>(), n, iw / 4, ow / 4);
+    NZCP_LAUNCH_CHECK();
+    NZCP_CUDA(cudaMemcpy(out, dout.p, n * ow, cudaMemcpyDeviceToHost));
+  });
+}
+
+int nzcp_curve_op(int g2, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n, int device) {
+  return api_guard([&] {
+    if (!a || !out || (op <= 2 && !b)) throw ApiError(NZCP_E_ARG, "null argument");
+    if (op < 0 || op > 4 || g2 < 0 || g2 > 1) throw ApiError(NZCP_E_ARG, "bad op/group");
+    // xyzz_madd's contract: the affine operand is never the point at infinity (0, 0)
+    const size_t as = g2 ? sizeof(G2Affine) : sizeof(G1Affine);
+    for (size_t i = 0; i < n && (op == 1 || op == 2); i++) {
+      const uint8_t* p = b + as * i;
+      bool zero = true;
+      for (size_t k = 0; k < as && zero; k++) zero = p[k] == 0;
+      if (zero) throw ApiError(NZCP_E_ARG, "madd operand is the point at infinity");
+    }
+    use_device(device);
+    if (!n) return;
+    if (g2) run_xyzz_op<Fq2>(op, a, b, out, n); else run_xyzz_op<Fq>(op, a, b, out, n);
   });
 }
 

@@ -90,6 +90,12 @@ def test_no_cpu_fallback(lib):
     with pytest.raises(NzcpError) as e:
         api.selftest()
     assert e.value.code == _lib.NZCP_E_CUDA
+    with pytest.raises(NzcpError) as e:
+        api.arith_op(2, bytes(128), 1)
+    assert e.value.code == _lib.NZCP_E_CUDA
+    with pytest.raises(NzcpError) as e:
+        api.curve_op(False, 3, bytes(128), None, 1)
+    assert e.value.code == _lib.NZCP_E_CUDA
 
 
 def test_zkey_format_errors_are_reported_before_touching_the_gpu(lib):
@@ -129,3 +135,38 @@ def test_null_and_bad_arguments_return_error_codes(lib):
     lib.nzcp_zkey_free(None)          # no-ops
     lib.nzcp_prover_free(None)
     lib.nzcp_synth_free(None)
+
+
+def test_arith_and_curve_ops_reject_bad_arguments(lib):
+    """The device arithmetic hooks check op, group and operand domain on the host, before any device is touched: a raw
+    operand of the wide product >= 2^255, a wide-reduction input >= q 2^256 and a madd operand at infinity never reach a
+    kernel.  Inputs just inside the bounds pass the checks (and then need a device)."""
+    import ctypes as C
+    out = (C.c_uint8 * 512)()
+    good = bytes(256)
+    for op in (-1, 10):
+        assert lib.nzcp_arith_op(op, good, out, 1, 0) == _lib.NZCP_E_ARG
+    for g2, op in ((0, -1), (0, 5), (2, 0), (-1, 0)):
+        assert lib.nzcp_curve_op(g2, op, good, good, out, 1, 0) == _lib.NZCP_E_ARG
+    assert lib.nzcp_arith_op(0, None, out, 1, 0) == _lib.NZCP_E_ARG
+    assert lib.nzcp_arith_op(0, good, None, 1, 0) == _lib.NZCP_E_ARG
+    assert lib.nzcp_curve_op(0, 0, good, None, out, 1, 0) == _lib.NZCP_E_ARG
+    assert lib.nzcp_curve_op(0, 3, None, None, out, 1, 0) == _lib.NZCP_E_ARG
+
+    def arith(op, *vals, width=32):
+        return lib.nzcp_arith_op(op, b"".join(v.to_bytes(width, "little") for v in vals), out, 1, 0)
+    mont = 1 << 256
+    # fp_mul_wide: a, b < 2^255 (either operand, second record of a batch too)
+    assert arith(0, 1 << 255, 1) == _lib.NZCP_E_ARG
+    assert arith(0, 1, mont - 1) == _lib.NZCP_E_ARG
+    assert lib.nzcp_arith_op(0, bytes(64) + le32(1) + le32(1 << 255), out, 2, 0) == _lib.NZCP_E_ARG
+    assert arith(0, (1 << 255) - 1, (1 << 255) - 1) != _lib.NZCP_E_ARG
+    # fp_redc_wide: T < q 2^256
+    assert arith(1, Q * mont, width=64) == _lib.NZCP_E_ARG
+    assert arith(1, (1 << 512) - 1, width=64) == _lib.NZCP_E_ARG
+    assert arith(1, Q * mont - 1, width=64) != _lib.NZCP_E_ARG
+    # xyzz_madd: the affine operand must not be (0, 0); the XYZZ side may be infinity
+    for g2, (xs, as_) in enumerate(((128, 64), (256, 128))):
+        for op in (1, 2):
+            assert lib.nzcp_curve_op(g2, op, bytes(xs), bytes(as_), out, 1, 0) == _lib.NZCP_E_ARG
+            assert lib.nzcp_curve_op(g2, op, bytes(xs), b"\x01" + bytes(as_ - 1), out, 1, 0) != _lib.NZCP_E_ARG

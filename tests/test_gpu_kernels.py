@@ -7,6 +7,7 @@ import random
 
 import pytest
 
+from arith_cases import inverse_edge_values, mul_targeted, targets
 from nzcp_circom_b200 import api
 from nzcp_circom_b200._lib import NzcpError
 from oracle import bn254 as ob
@@ -34,6 +35,10 @@ def test_field_ops_limb_exact(lib, field, p):
     ev = _edge_values(p)
     a = [x for x in ev for _ in ev] + [rng.randrange(p) for _ in range(4000)]
     b = [y for _ in ev for y in ev] + [rng.randrange(p) for _ in range(4000)]
+    # operands solved so that the Montgomery product lands on 0, 1, p-1 .. p-64, ...: the final subtraction's edge
+    tgt = [mul_targeted(rng, y, p) for y in targets(p) for _ in range(4)]
+    a += [x for x, _ in tgt]
+    b += [y for _, y in tgt]
     ab = b"".join(le32(x) for x in a)
     bb = b"".join(le32(x) for x in b)
     rinv = pow(MONT, -1, p)
@@ -42,6 +47,18 @@ def test_field_ops_limb_exact(lib, field, p):
         exp = b"".join(le32(fn(x, y)) for x, y in zip(a, b))
         assert api.field_op(field, op, ab, bb, n) == exp            # IMAD carry-chain PTX path
         assert api.field_op(field, op + 3, ab, bb, n) == exp        # portable path compiled for the device
+
+
+@pytest.mark.parametrize("field,p", [(0, R), (1, Q)])
+def test_field_inverses_device(lib, field, p):
+    """Ops 6 (division steps, what the pair rounds run) and 7 (Fermat ladder, what xyzz_to_affine runs)."""
+    rng = random.Random(41 + field)
+    vals = inverse_edge_values(p) + [rng.randrange(p) for _ in range(1 << 16)]
+    a = b"".join(le32(x) for x in vals)
+    # Montgomery in, Montgomery out: x = aR  ->  a^-1 R = R^2 / x
+    exp = b"".join(le32(0 if x == 0 else pow(x, -1, p) * MONT * MONT % p) for x in vals)
+    assert api.field_op(field, 6, a, a, len(vals)) == exp
+    assert api.field_op(field, 7, a, a, len(vals)) == exp
 
 
 def _mont_bytes(vals):
