@@ -22,6 +22,8 @@
  *                       build_multiexp.js (yarn.lock:1132-1135); the *_partial / sum_partials pair is the per-rank half of
  *                       the split MSM of BASELINE.json configs[4]
  *   nzcp_zkey_selfcheck no snarkjs equivalent: the format facts of SURVEY.md 8c-3, for the first real key
+ *   nzcp_ptau_prepare*  snarkjs powersoftau_preparephase2.js preparePhase2(oldPtauFilename, newPTauFilename) and the group
+ *                       ifft of ffjavascript engine_fft.js it runs per level (yarn.lock:987-999, 408-416)
  *   nzcp_field_op       wasmcurves build_f1m.js f1m_mul / f1m_add / f1m_sub (yarn.lock:1132-1135)
  *   nzcp_synth_*        snarkjs zkey_new.js with a known tau in place of the ptau file /root/reference/Makefile:31 names;
  *                       shapes from circuits/nzcp_exampleTest.circom:4 and circuits/nzcp_liveTest.circom:4
@@ -130,6 +132,21 @@ int nzcp_zkey_selfcheck(const uint8_t* bytes, size_t len, int device, nzcp_zkey_
 int nzcp_zkey_new_size(const uint8_t* r1cs, size_t r1cs_len, const uint8_t* ptau, size_t ptau_len, size_t* out_size);
 int nzcp_zkey_new(const uint8_t* r1cs, size_t r1cs_len, const uint8_t* ptau, size_t ptau_len, int device, uint8_t* out,
                   size_t cap, size_t* written);
+
+/* snarkjs `powersoftau prepare phase2` (powersoftau_preparephase2.js preparePhase2(oldPtau, newPtau)): the file `zkey new`
+ * needs from the output of a phase-1 ceremony.  Sections 2-7 are copied, the header gets ceremonyPower = power, and the
+ * Lagrange-basis sections 12 (from tauG1, levels 0 .. power+1), 13 (tauG2), 14 (alphaTauG1) and 15 (betaTauG1) (levels
+ * 0 .. power) are computed by an inverse FFT over curve points on `device`; sections 12-15 already in the input are
+ * ignored.  As in snarkjs, the top tauG1 level takes the point at infinity for the tauG1 power the file lacks (see
+ * csrc/ptau.cu).  Output: 11 sections in the order 1-7, 12-15.
+ * Both functions reject before any device work: a file that is not a ptau (NZCP_E_FORMAT) or not over bn128
+ * (NZCP_E_CURVE); power outside 1..27 (NZCP_E_FORMAT; power 28 needs snarkjs's coset branch and is NZCP_E_ARG); a missing
+ * section 2-7 ("Missing section N") or a section 2-6 whose size does not match the power (NZCP_E_FORMAT); an input point
+ * with a coordinate >= q or off its curve (NZCP_E_RANGE).  nzcp_ptau_prepare_size is host-only.
+ * section_ms (optional): device time of output sections 12, 13, 14, 15. */
+int nzcp_ptau_prepare_size(const uint8_t* ptau, size_t len, size_t* out_size);
+int nzcp_ptau_prepare(const uint8_t* ptau, size_t len, int device, uint8_t* out, size_t cap, size_t* written,
+                      float section_ms[4]);
 
 /* Work buffers + streams for proofs against `zk`.  Several provers may share one zkey (one per host thread). */
 int nzcp_prover_create(nzcp_zkey* zk, nzcp_prover** out);   /* = mode 0 */
@@ -253,6 +270,9 @@ int nzcp_host_msm_sim(const uint8_t* bases, const uint8_t* scalars, size_t n_poi
                       int adds_per_thread, uint8_t* out);
 /* Fr.w[k] of ffjavascript (plain form). */
 int nzcp_host_root_of_unity(int k, uint8_t* out_plain);
+/* nzcp_ptau_prepare with the kernels' load, stage indexing and butterflies run one thread after the other on the CPU,
+ * for power <= 4 (larger powers: NZCP_E_ARG).  Same validation, same output bytes. */
+int nzcp_host_ptau_prepare(const uint8_t* ptau, size_t len, uint8_t* out, size_t cap, size_t* written);
 
 /* ---- synthetic circuits of the NZCP shape (no circom / snarkjs in this environment; SURVEY.md 8d) ---- */
 typedef struct nzcp_synth nzcp_synth;

@@ -335,6 +335,27 @@ def zkey_new(r1cs, ptau, device=0):
     return out
 
 
+PTAU_SECTIONS = (12, 13, 14, 15)
+
+
+def ptau_prepare(ptau, device=0, timings=None):
+    """snarkjs `powersoftau prepare phase2`: a phase-1 .ptau (path | bytes-like | {"type": "mem"}) -> bytearray with the
+    prepared file (Lagrange-basis sections 12-15 added; csrc/ptau.cu).  The inverse FFTs run on `device`.  `timings`: a
+    dict that receives the device milliseconds of each output section, keyed 12, 13, 14, 15."""
+    lib = _lib.load()
+    pb = _as_bytes_like(ptau)
+    size = C.c_size_t()
+    check(lib.nzcp_ptau_prepare_size(addr(pb), _nbytes(pb), C.byref(size)))
+    out = bytearray(size.value)
+    written = C.c_size_t()
+    ms = (C.c_float * 4)()
+    check(lib.nzcp_ptau_prepare(addr(pb), _nbytes(pb), int(device), addr(out), len(out), C.byref(written), ms))
+    assert written.value == len(out)
+    if timings is not None:
+        timings.update(zip(PTAU_SECTIONS, [float(x) for x in ms]))
+    return out
+
+
 def zkey_selfcheck(zkey, device=0):
     """Format self-checks of SURVEY.md 8c-3 on a .zkey image (path | bytes-like | {"type": "mem"}) -> dict; ["ok"] is
     the verdict.  Meant for the first REAL snarkjs-made key: it pins the section-4 `coef * R^2` convention, the moduli
@@ -422,6 +443,19 @@ def host_msm_sim(bases, scalars, n_points, g2=False, window_bits=8, rounds=1, ad
     check(_lib.load().nzcp_host_msm_sim(addr(bases), addr(scalars), int(n_points), int(bool(g2)), int(window_bits),
                                         int(rounds), int(adds_per_thread), addr(out)))
     return bytes(out)
+
+
+def host_ptau_prepare(ptau):
+    """CPU run of ptau_prepare's load / stage / butterfly code (power <= 4) -> the same bytes."""
+    lib = _lib.load()
+    pb = _as_bytes_like(ptau)
+    size = C.c_size_t()
+    check(lib.nzcp_ptau_prepare_size(addr(pb), _nbytes(pb), C.byref(size)))
+    out = bytearray(size.value)
+    written = C.c_size_t()
+    check(lib.nzcp_host_ptau_prepare(addr(pb), _nbytes(pb), addr(out), len(out), C.byref(written)))
+    assert written.value == len(out)
+    return out
 
 
 def tuning_set(name, value):

@@ -268,6 +268,85 @@ HDN inline XYZZ<F> xyzz_mul(const XYZZ<F>& p, const uint32_t* k) {
   return r;
 }
 
+// Bits pos .. pos+4 of a 256-bit little-endian scalar; bits below 0 read as 0.
+HD uint32_t scalar_bits5(const uint32_t* v, int pos) {
+  if (pos < 0) return (v[0] << 1) & 31u;
+  const int l = pos >> 5;
+  uint64_t w = v[l];
+  if (l < 7) w |= (uint64_t)v[l + 1] << 32;
+  return (uint32_t)(w >> (pos & 31)) & 31u;
+}
+
+// acc += k * P for an affine P and a plain scalar k < r.  k > (r-1)/2 is folded to (r - k) * (-P), so the -1 / small
+// negative coefficients circom emits cost one addition.  The rest is a signed 4-bit fixed window (radix-16 Booth digits
+// d_i = b(4i-1) + b(4i) + 2 b(4i+1) + 4 b(4i+2) - 8 b(4i+3), in [-8, 8]) over a table of 1..8 * P: 4 doublings and at most
+// one addition per digit.  The digits of every lane of a warp fall at the same positions, so the additions do not
+// diverge the way a per-bit double-and-add does (one lane or another has a set bit at almost every position).
+template <class F>
+HD void scalar_mul_accumulate(XYZZ<F>& acc, const Affine<F>& P, Fr k) {
+  if (P.is_inf() || k.is_zero()) return;
+  bool neg = false;
+  {
+    Fr nk = fp_sub(Fr::zero(), k);       // r - k (plain integers: canonical subtraction mod r)
+    bool gt = false;
+#pragma unroll
+    for (int i = 7; i >= 0; i--) {
+      if (k.v[i] != nk.v[i]) { gt = k.v[i] > nk.v[i]; break; }
+    }
+    if (gt) { k = nk; neg = true; }
+  }
+  int top = 255;
+  while (top > 0 && !((k.v[top >> 5] >> (top & 31)) & 1)) top--;
+  if (top == 0) {                        // k == 1
+    xyzz_madd(acc, P, neg);
+    return;
+  }
+  XYZZ<F> tab[8];                        // tab[j] = (j + 1) * P
+  tab[0] = XYZZ<F>::from_affine(P);
+  tab[1] = xyzz_dbl_affine(P);
+  for (int j = 2; j < 8; j++) {
+    tab[j] = tab[j - 1];
+    xyzz_madd(tab[j], P, false);
+  }
+  XYZZ<F> r = XYZZ<F>::inf();
+  for (int i = (top + 1) >> 2; i >= 0; i--) {   // k < r/2 < 2^253: no digit above bit 252 + 1
+    for (int d = 0; d < 4; d++) r = xyzz_dbl(r);
+    const uint32_t w = scalar_bits5(k.v, 4 * i - 1);
+    const int d = (int)((w + 1) >> 1) - (int)((w >> 4) << 4);
+    if (d) {
+      XYZZ<F> t = tab[(d < 0 ? -d : d) - 1];
+      if (d < 0) t = xyzz_neg(t);
+      xyzz_add(r, t);
+    }
+  }
+  if (neg) r = xyzz_neg(r);
+  xyzz_add(acc, r);
+}
+
+// Curve membership of an affine point in Montgomery form: canonical coordinates and y^2 = x^3 + b, or the (0,0) marker.
+template <class F> struct CoordCanon;
+template <> struct CoordCanon<Fq> {
+  HD static bool ok(const Fq& a) { return !fp_geq_mod<FqParams>(a.v); }
+};
+template <> struct CoordCanon<Fq2> {
+  HD static bool ok(const Fq2& a) { return !fp_geq_mod<FqParams>(a.c0.v) && !fp_geq_mod<FqParams>(a.c1.v); }
+};
+
+template <class F>
+HD bool point_ok(const Affine<F>& p, const F& b, bool* inf) {
+  *inf = p.is_inf();
+  if (*inf) return true;
+  if (!CoordCanon<F>::ok(p.x) || !CoordCanon<F>::ok(p.y)) return false;
+  const F lhs = f_sqr(p.y);
+  const F rhs = f_add(f_mul(f_sqr(p.x), p.x), b);
+  return lhs == rhs;
+}
+
+template <class F>
+HD F curve_b(const Affine<F>& gen) {   // b = y^2 - x^3 of the generator (Montgomery form)
+  return f_sub(f_sqr(gen.y), f_mul(f_sqr(gen.x), gen.x));
+}
+
 // Montgomery-form affine; infinity -> (0,0).
 template <class F>
 HDN inline Affine<F> xyzz_to_affine(const XYZZ<F>& p) {

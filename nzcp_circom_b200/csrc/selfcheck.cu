@@ -18,24 +18,6 @@ namespace nzcp {
 G1Affine g1_generator();  // synth.cu
 G2Affine g2_generator();
 
-template <class F> struct CoordCanon;
-template <> struct CoordCanon<Fq> {
-  HD static bool ok(const Fq& a) { return !fp_geq_mod<FqParams>(a.v); }
-};
-template <> struct CoordCanon<Fq2> {
-  HD static bool ok(const Fq2& a) { return !fp_geq_mod<FqParams>(a.c0.v) && !fp_geq_mod<FqParams>(a.c1.v); }
-};
-
-template <class F>
-HD bool point_ok(const Affine<F>& p, const F& b, bool* inf) {
-  *inf = p.is_inf();
-  if (*inf) return true;
-  if (!CoordCanon<F>::ok(p.x) || !CoordCanon<F>::ok(p.y)) return false;
-  const F lhs = f_sqr(p.y);
-  const F rhs = f_add(f_mul(f_sqr(p.x), p.x), b);
-  return lhs == rhs;
-}
-
 // counts[0] += points off the curve (or with a non-canonical coordinate), counts[1] += infinity markers
 template <class F>
 __global__ void __launch_bounds__(128) curve_check_kernel(const Affine<F>* __restrict__ pts, size_t n, F b, unsigned long long* counts) {
@@ -47,11 +29,6 @@ __global__ void __launch_bounds__(128) curve_check_kernel(const Affine<F>* __res
     if (bad_mask) atomicAdd(&counts[0], (unsigned long long)__popc(bad_mask));
     if (inf_mask) atomicAdd(&counts[1], (unsigned long long)__popc(inf_mask));
   }
-}
-
-template <class F>
-static F curve_b(const Affine<F>& gen) {   // b = y^2 - x^3 of the generator (Montgomery form)
-  return f_sub(f_sqr(gen.y), f_mul(f_sqr(gen.x), gen.x));
 }
 
 template <class F>

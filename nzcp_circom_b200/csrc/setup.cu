@@ -25,11 +25,12 @@
 // Sections are written in zkey_new.js's own order: 1, 2, 4, 3, 9, 8, 5, 6, 7, 10.
 //
 // B200 design: the four sparse point combinations are one kernel each, one thread per wire walking its term list
-// (CSR by wire built on the host): k * P by double-and-add from the top set bit, with k > r/2 folded to (r - k) * (-P) so
-// the -1 / small-negative coefficients circom emits cost one addition, not 254 doublings.  One-time work per circuit.
+// (CSR by wire built on the host): k * P over signed 4-bit windows of k (ec.cuh scalar_mul_accumulate), with k > r/2
+// folded to (r - k) * (-P) so the -1 / small-negative coefficients circom emits cost one addition, not 254 doublings.
+// One-time work per circuit.
 #include <memory>
 
-#include "api_util.cuh"
+#include "binfile.cuh"
 
 namespace nzcp {
 
@@ -37,26 +38,6 @@ G1Affine g1_generator();  // synth.cu
 G2Affine g2_generator();
 
 namespace {
-
-uint32_t rd32u(const uint8_t* p) { uint32_t v; memcpy(&v, p, 4); return v; }
-uint64_t rd64u(const uint8_t* p) { uint64_t v; memcpy(&v, p, 8); return v; }
-
-struct Sect { const uint8_t* p = nullptr; uint64_t len = 0; };
-
-void parse_bin(const uint8_t* b, size_t len, const char* magic, Sect* secs, int max_id) {
-  if (len < 12 || memcmp(b, magic, 4) != 0) throw ApiError(NZCP_E_FORMAT, std::string(magic) + " file: Invalid File format");
-  if (rd32u(b + 4) > 1) throw ApiError(NZCP_E_FORMAT, "Version not supported");
-  size_t pos = 12;
-  for (uint32_t i = 0, n = rd32u(b + 8); i < n; i++) {
-    if (pos + 12 > len) throw ApiError(NZCP_E_FORMAT, "truncated section table");
-    const uint32_t id = rd32u(b + pos);
-    const uint64_t sl = rd64u(b + pos + 4);
-    pos += 12;
-    if (sl > len - pos) throw ApiError(NZCP_E_FORMAT, "section exceeds file size");
-    if (id <= (uint32_t)max_id && !secs[id].p) { secs[id].p = b + pos; secs[id].len = sl; }
-    pos += sl;
-  }
-}
 
 struct R1cs {
   uint32_t n_wires = 0, n_pub_out = 0, n_pub_in = 0, n_prv_in = 0, n_constraints = 0, n_public = 0;
@@ -140,50 +121,7 @@ struct Combo {      // one sparse point combination: CSR by wire
   std::vector<Term> terms;
 };
 
-struct Writer {
-  uint8_t* p;
-  size_t cap, pos = 0;
-  Writer(uint8_t* b, size_t c) : p(b), cap(c) {}
-  void need(size_t n) { if (pos + n > cap) throw ApiError(NZCP_E_ARG, "output buffer too small"); }
-  void u32(uint32_t v) { need(4); memcpy(p + pos, &v, 4); pos += 4; }
-  void u64(uint64_t v) { need(8); memcpy(p + pos, &v, 8); pos += 8; }
-  void raw(const void* s, size_t n) { need(n); memcpy(p + pos, s, n); pos += n; }
-  void zeros(size_t n) { need(n); memset(p + pos, 0, n); pos += n; }
-  uint8_t* reserve(size_t n) { need(n); uint8_t* q = p + pos; pos += n; return q; }
-  void section(uint32_t id, uint64_t len) { u32(id); u64(len); }
-};
-
 }  // namespace
-
-// k * P for an affine P: left-to-right double-and-add from the top set bit; k > (r-1)/2 is folded to (r - k) * (-P).
-template <class F>
-__device__ __forceinline__ void scalar_mul_accumulate(XYZZ<F>& acc, const Affine<F>& P, Fr k) {
-  if (P.is_inf() || k.is_zero()) return;
-  bool neg = false;
-  {
-    // half = (r - 1) / 2; compare k > half
-    Fr nk = fp_sub(Fr::zero(), k);       // r - k (plain integers: canonical subtraction mod r)
-    bool gt = false;
-#pragma unroll
-    for (int i = 7; i >= 0; i--) {
-      if (k.v[i] != nk.v[i]) { gt = k.v[i] > nk.v[i]; break; }
-    }
-    if (gt) { k = nk; neg = true; }
-  }
-  int top = 255;
-  while (top > 0 && !((k.v[top >> 5] >> (top & 31)) & 1)) top--;
-  if (top == 0) {                        // k == 1
-    xyzz_madd(acc, P, neg);
-    return;
-  }
-  XYZZ<F> r = XYZZ<F>::from_affine(P);
-  for (int b = top - 1; b >= 0; b--) {
-    r = xyzz_dbl(r);
-    if ((k.v[b >> 5] >> (b & 31)) & 1) xyzz_madd(r, P, false);
-  }
-  if (neg) r = xyzz_neg(r);
-  xyzz_add(acc, r);
-}
 
 template <class F>
 __global__ void __launch_bounds__(128)

@@ -5,7 +5,8 @@ yarn.lock:987-999).  The reference's tests build the prover input at /root/refer
 (`{ toBeSigned: bufferToBitArray(bytes), toBeSignedLen }`) and read public signals as witness[1..513] at
 test/nzcp.js:41-48; `publicSignals` below is that same slice, in the same order, as decimal strings.
 
-`zKey` groups newZKey / exportVerificationKey the way snarkjs's main.js does (snarkjs.zKey.newZKey, ...).
+`zKey` groups newZKey / exportVerificationKey the way snarkjs's main.js does (snarkjs.zKey.newZKey, ...);
+`powersOfTau.preparePhase2` is snarkjs.powersOfTau.preparePhase2.
 
 Same names, argument meaning and error text as snarkjs:
   prove(zkeyFileName, witnessFileName, logger=None)   file args: path | bytes-like | {"type": "mem", "data": ...}
@@ -289,6 +290,28 @@ def exportVerificationKey(zkeyFileName):
     ic0 = secs[3][0]
     vk["IC"] = [g1(ic0 + 64 * i) for i in range(n_public + 1)]
     return vk
+
+
+def preparePhase2(oldPtauFilename, newPTauFilename=None, logger=None, *, device=0):
+    """snarkjs powersOfTau.preparePhase2(oldPtauFilename, newPTauFilename): adds the Lagrange-basis sections 12-15 that
+    `zkey new` reads, computed on the GPU.  `newPTauFilename`: a path to write, a {"type": "mem"} object that receives
+    `.data`, or None.  Returns the prepared .ptau image."""
+    timings = {} if logger else None
+    data = api.ptau_prepare(oldPtauFilename, device=device, timings=timings)
+    if logger:
+        for sid, ms in timings.items():
+            logger.debug("section %d: %.3f ms" % (sid, ms))
+    if isinstance(newPTauFilename, dict):
+        newPTauFilename["data"] = data
+    elif newPTauFilename is not None:
+        with open(newPTauFilename, "wb") as f:
+            f.write(data)
+    return data
+
+
+class powersOfTau:
+    """snarkjs.powersOfTau namespace: the one entry this library computes."""
+    preparePhase2 = staticmethod(preparePhase2)
 
 
 class zKey:
