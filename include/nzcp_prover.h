@@ -24,6 +24,9 @@
  *   nzcp_zkey_selfcheck no snarkjs equivalent: the format facts of SURVEY.md 8c-3, for the first real key
  *   nzcp_ptau_prepare*  snarkjs powersoftau_preparephase2.js preparePhase2(oldPtauFilename, newPTauFilename) and the group
  *                       ifft of ffjavascript engine_fft.js it runs per level (yarn.lock:987-999, 408-416)
+ *   nzcp_zkey_contribute*, nzcp_zkey_beacon
+ *                       snarkjs zkey_contribute.js phase2contribute and zkey_beacon.js beacon, with the ChaCha of
+ *                       ffjavascript random.js (yarn.lock:987-999, 408-416)
  *   nzcp_field_op       wasmcurves build_f1m.js f1m_mul / f1m_add / f1m_sub (yarn.lock:1132-1135)
  *   nzcp_synth_*        snarkjs zkey_new.js with a known tau in place of the ptau file /root/reference/Makefile:31 names;
  *                       shapes from circuits/nzcp_exampleTest.circom:4 and circuits/nzcp_liveTest.circom:4
@@ -147,6 +150,31 @@ int nzcp_zkey_new(const uint8_t* r1cs, size_t r1cs_len, const uint8_t* ptau, siz
 int nzcp_ptau_prepare_size(const uint8_t* ptau, size_t len, size_t* out_size);
 int nzcp_ptau_prepare(const uint8_t* ptau, size_t len, int device, uint8_t* out, size_t cap, size_t* written,
                       float section_ms[4]);
+
+/* snarkjs `zkey contribute` / `zkey beacon` (zkey_contribute.js phase2contribute, zkey_beacon.js beacon): one phase-2
+ * contribution k to a Groth16 key.  delta1 and delta2 of the header become k * delta, every point of sections 8 (L) and 9
+ * (H) becomes k^-1 * P on `device`, sections 1 and 3-7 are copied, and section 10 gets a new record after the earlier
+ * ones (type 0 contribute, 1 beacon; parameter tag 1 = name if name is non-empty, tags 2 / 3 = num_iterations_exp /
+ * beacon hash).  Output: 10 sections in the order 1..10.  `hash` receives the 64-byte contribution hash snarkjs prints.
+ * contribute: k comes from ffjavascript's ChaCha seeded by BLAKE2b-512(64 OS-random bytes || entropy); `seed` (32 bytes,
+ * test hook; NULL in use) seeds the ChaCha directly instead.  beacon: from SHA-256 iterated 2^num_iterations_exp times
+ * over beacon_hash.  See csrc/contribute.cu for the restated algorithm.
+ * All functions reject before any device work: a file that is not a zkey or has no header (NZCP_E_FORMAT); protocol != 1
+ * (NZCP_E_NOT_GROTH16); moduli other than bn128's (NZCP_E_CURVE); section 2 not 660 bytes, a missing section 2-10
+ * ("Missing section N"), a section 8 / 9 size that does not match nVars - nPublic - 1 / domainSize, a section 10 that is
+ * truncated, has trailing bytes, unsorted ("Parameters in the contribution must be sorted") or unknown ("Parameter not
+ * recognized") parameters (NZCP_E_FORMAT); a point of sections 8 / 9 or the header delta1 / delta2 with a coordinate >= q
+ * or off its curve (NZCP_E_RANGE); a name longer than 64 bytes (NZCP_E_ARG; snarkjs would cut it at 64 characters); a
+ * beacon hash of 0 or >= 256 bytes or num_iterations_exp outside 10..63 (NZCP_E_ARG, snarkjs's messages).
+ * nzcp_zkey_contribute_size is host-only; beacon_hash_len = 0 sizes a contribute record.
+ * section_ms (optional): device time of sections 8 and 9. */
+int nzcp_zkey_contribute_size(const uint8_t* zkey, size_t len, const char* name, size_t beacon_hash_len, size_t* out_size);
+int nzcp_zkey_contribute(const uint8_t* zkey, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
+                         const uint8_t* seed, int device, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64],
+                         float section_ms[2]);
+int nzcp_zkey_beacon(const uint8_t* zkey, size_t len, const char* name, const uint8_t* beacon_hash, size_t beacon_hash_len,
+                     uint32_t num_iterations_exp, int device, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64],
+                     float section_ms[2]);
 
 /* Work buffers + streams for proofs against `zk`.  Several provers may share one zkey (one per host thread). */
 int nzcp_prover_create(nzcp_zkey* zk, nzcp_prover** out);   /* = mode 0 */
@@ -273,6 +301,12 @@ int nzcp_host_root_of_unity(int k, uint8_t* out_plain);
 /* nzcp_ptau_prepare with the kernels' load, stage indexing and butterflies run one thread after the other on the CPU,
  * for power <= 4 (larger powers: NZCP_E_ARG).  Same validation, same output bytes. */
 int nzcp_host_ptau_prepare(const uint8_t* ptau, size_t len, uint8_t* out, size_t cap, size_t* written);
+
+/* nzcp_zkey_contribute (beacon_hash == NULL) or nzcp_zkey_beacon with the kernel's per-point code run on the CPU, for
+ * sections 8 + 9 of at most 4096 points (more: NZCP_E_ARG).  Same validation, same output bytes and hash. */
+int nzcp_host_zkey_contribute(const uint8_t* zkey, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
+                              const uint8_t* seed, const uint8_t* beacon_hash, size_t beacon_hash_len,
+                              uint32_t num_iterations_exp, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]);
 
 /* ---- synthetic circuits of the NZCP shape (no circom / snarkjs in this environment; SURVEY.md 8d) ---- */
 typedef struct nzcp_synth nzcp_synth;

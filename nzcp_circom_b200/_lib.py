@@ -76,6 +76,11 @@ SIGNATURES = {
     "nzcp_zkey_new": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, C.c_int, _U8P, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nzcp_ptau_prepare_size": (C.c_int, [_U8P, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nzcp_ptau_prepare": (C.c_int, [_U8P, C.c_size_t, C.c_int, _U8P, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_float)]),
+    "nzcp_zkey_contribute_size": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "nzcp_zkey_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, C.c_int, _U8P, C.c_size_t,
+                                       C.POINTER(C.c_size_t), _U8P, C.POINTER(C.c_float)]),
+    "nzcp_zkey_beacon": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, C.c_uint32, C.c_int, _U8P, C.c_size_t,
+                                   C.POINTER(C.c_size_t), _U8P, C.POINTER(C.c_float)]),
     "nzcp_msm_plan_create": (C.c_int, [_U8P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(_P),
                                        C.POINTER(C.c_float)]),
     "nzcp_msm_plan_free": (None, [_P]),
@@ -95,6 +100,8 @@ SIGNATURES = {
     "nzcp_host_scalar_mul": (C.c_int, [C.c_int, _U8P, _U8P, _U8P]),
     "nzcp_host_root_of_unity": (C.c_int, [C.c_int, _U8P]),
     "nzcp_host_ptau_prepare": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "nzcp_host_zkey_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, _U8P, C.c_size_t,
+                                            C.c_uint32, _U8P, C.c_size_t, C.POINTER(C.c_size_t), _U8P]),
     "nzcp_host_msm_sim": (C.c_int, [_U8P, _U8P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, _U8P]),
     "nzcp_tuning_set": (C.c_int, [C.c_char_p, C.c_int]),
     "nzcp_synth_points": (C.c_int, [C.c_uint64, C.c_size_t, C.c_int, C.c_int, _U8P]),

@@ -356,6 +356,61 @@ def ptau_prepare(ptau, device=0, timings=None):
     return out
 
 
+CONTRIBUTE_SECTIONS = (8, 9)
+
+
+def _utf8(v):
+    if v is None:
+        return None
+    b = v.encode() if isinstance(v, str) else bytes(v)
+    if b"\0" in b:
+        raise NzcpError(_lib.NZCP_E_ARG, "zkey: contribution name contains a NUL byte")
+    return b
+
+
+def _contribute_out(lib, zb, name, beacon_len):
+    size = C.c_size_t()
+    check(lib.nzcp_zkey_contribute_size(addr(zb), _nbytes(zb), name, beacon_len, C.byref(size)))
+    return bytearray(size.value)
+
+
+def zkey_contribute(zkey, name=None, entropy=None, seed=None, device=0, timings=None):
+    """snarkjs `zkey contribute`: a Groth16 key (path | bytes-like | {"type": "mem"}) -> (bytearray with the new key,
+    64-byte contribution hash).  The random key comes from BLAKE2b(64 OS-random bytes || entropy) (str: UTF-8); `seed`
+    (32 bytes, tests) seeds the ChaCha directly instead.  Sections 8 and 9 are rescaled on `device`; `timings` receives
+    their device milliseconds, keyed 8 and 9."""
+    lib = _lib.load()
+    zb = _as_bytes_like(zkey)
+    nb, eb = _utf8(name), _utf8(entropy) or b""
+    if seed is not None and len(bytes(seed)) != 32:
+        raise NzcpError(_lib.NZCP_E_ARG, "seed must be 32 bytes")
+    out = _contribute_out(lib, zb, nb, 0)
+    written, h, ms = C.c_size_t(), bytearray(64), (C.c_float * 2)()
+    check(lib.nzcp_zkey_contribute(addr(zb), _nbytes(zb), nb, addr(eb) if eb else None, len(eb),
+                                   None if seed is None else bytes(seed), int(device), addr(out), len(out),
+                                   C.byref(written), addr(h), ms))
+    assert written.value == len(out)
+    if timings is not None:
+        timings.update(zip(CONTRIBUTE_SECTIONS, [float(x) for x in ms]))
+    return out, bytes(h)
+
+
+def zkey_beacon(zkey, beacon_hash, num_iterations_exp, name=None, device=0, timings=None):
+    """snarkjs `zkey beacon`: as zkey_contribute, with the random key derived from `beacon_hash` (bytes) hashed with
+    SHA-256 2^num_iterations_exp times (10..63)."""
+    lib = _lib.load()
+    zb = _as_bytes_like(zkey)
+    nb, hb = _utf8(name), bytes(beacon_hash)
+    out = _contribute_out(lib, zb, nb, len(hb))
+    written, h, ms = C.c_size_t(), bytearray(64), (C.c_float * 2)()
+    check(lib.nzcp_zkey_beacon(addr(zb), _nbytes(zb), nb, hb, len(hb), int(num_iterations_exp), int(device), addr(out),
+                               len(out), C.byref(written), addr(h), ms))
+    assert written.value == len(out)
+    if timings is not None:
+        timings.update(zip(CONTRIBUTE_SECTIONS, [float(x) for x in ms]))
+    return out, bytes(h)
+
+
 def zkey_selfcheck(zkey, device=0):
     """Format self-checks of SURVEY.md 8c-3 on a .zkey image (path | bytes-like | {"type": "mem"}) -> dict; ["ok"] is
     the verdict.  Meant for the first REAL snarkjs-made key: it pins the section-4 `coef * R^2` convention, the moduli
@@ -456,6 +511,22 @@ def host_ptau_prepare(ptau):
     check(lib.nzcp_host_ptau_prepare(addr(pb), _nbytes(pb), addr(out), len(out), C.byref(written)))
     assert written.value == len(out)
     return out
+
+
+def host_zkey_contribute(zkey, name=None, entropy=None, seed=None, beacon_hash=None, num_iterations_exp=0):
+    """CPU run of zkey_contribute (beacon_hash None) or zkey_beacon, sections 8 + 9 of at most 4096 points -> the same
+    (bytearray, hash)."""
+    lib = _lib.load()
+    zb = _as_bytes_like(zkey)
+    nb, eb = _utf8(name), _utf8(entropy) or b""
+    hb = None if beacon_hash is None else bytes(beacon_hash)
+    out = _contribute_out(lib, zb, nb, len(hb) if hb else 0)
+    written, h = C.c_size_t(), bytearray(64)
+    check(lib.nzcp_host_zkey_contribute(addr(zb), _nbytes(zb), nb, addr(eb) if eb else None, len(eb),
+                                        None if seed is None else bytes(seed), hb, len(hb) if hb is not None else 0,
+                                        int(num_iterations_exp), addr(out), len(out), C.byref(written), addr(h)))
+    assert written.value == len(out)
+    return out, bytes(h)
 
 
 def tuning_set(name, value):

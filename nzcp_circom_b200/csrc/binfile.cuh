@@ -1,6 +1,10 @@
-// binfileutils containers (snarkjs .r1cs / .ptau / .zkey): the section-table reader and the output writer shared by the
-// setup entry points (setup.cu `zkey new`, ptau.cu `powersoftau prepare phase2`).
+// binfileutils containers (snarkjs .r1cs / .ptau / .zkey): the section-table reader, the output writer and the point check
+// shared by the setup entry points (setup.cu `zkey new`, ptau.cu `powersoftau prepare phase2`, contribute.cu `zkey
+// contribute` / `zkey beacon`).
 #pragma once
+#include <algorithm>
+#include <thread>
+
 #include "api_util.cuh"
 
 namespace nzcp {
@@ -38,5 +42,38 @@ struct Writer {
   uint8_t* reserve(size_t n) { need(n); uint8_t* q = p + pos; pos += n; return q; }
   void section(uint32_t id, uint64_t len) { u32(id); u64(len); }
 };
+
+// Every point of a section of n affine points must be the (0,0) marker or have canonical coordinates and lie on the curve
+// y^2 = x^3 + b.  Scanned by all host threads; throws NZCP_E_RANGE naming the first offending point ("<what>: section
+// <sec> point <i> ...").
+template <class F>
+void check_points(const char* what, const uint8_t* p, uint64_t n, int sec, const F& b) {
+  // first offending point of each thread's chunk; 1 = coordinate >= q, 2 = off the curve
+  const unsigned nt = std::max(1u, std::min(64u, std::thread::hardware_concurrency()));
+  const uint64_t chunk = (n + nt - 1) / nt;
+  std::vector<uint64_t> first(nt, UINT64_MAX);
+  std::vector<int> kind(nt, 0);
+  auto scan = [&](unsigned t) {
+    for (uint64_t i = t * chunk; i < std::min(n, (t + 1) * chunk); i++) {
+      Affine<F> a;
+      memcpy(&a, p + i * sizeof(Affine<F>), sizeof(Affine<F>));
+      bool inf;
+      if (a.is_inf()) continue;
+      const int k = !(CoordCanon<F>::ok(a.x) && CoordCanon<F>::ok(a.y)) ? 1 : !point_ok(a, b, &inf) ? 2 : 0;
+      if (k) { first[t] = i; kind[t] = k; return; }
+    }
+  };
+  if (n < 4096) {
+    for (unsigned t = 0; t < nt; t++) scan(t);
+  } else {
+    std::vector<std::thread> th;
+    for (unsigned t = 0; t < nt; t++) th.emplace_back(scan, t);
+    for (auto& t : th) t.join();
+  }
+  for (unsigned t = 0; t < nt; t++)
+    if (kind[t])
+      throw ApiError(NZCP_E_RANGE, std::string(what) + ": section " + std::to_string(sec) + " point " + std::to_string(first[t]) +
+                                       (kind[t] == 1 ? " has a coordinate >= q" : " is not on the curve"));
+}
 
 }  // namespace nzcp

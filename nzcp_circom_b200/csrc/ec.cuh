@@ -356,6 +356,16 @@ HDN inline Affine<F> xyzz_to_affine(const XYZZ<F>& p) {
   return Affine<F>{f_mul(p.x, iz2), f_mul(p.y, iz3)};
 }
 
+// Montgomery-form affine through the division-step inversion (fp_inv_fast): the per-point conversion of the kernels that
+// write one affine point per thread.
+template <class F>
+HD Affine<F> to_affine_fast(const XYZZ<F>& p) {
+  if (p.is_inf()) return Affine<F>::inf();
+  const F iz3 = f_inv_fast(p.zzz);
+  const F iz2 = f_sqr(f_mul(iz3, p.zz));
+  return Affine<F>{f_mul(p.x, iz2), f_mul(p.y, iz3)};
+}
+
 typedef Affine<Fq> G1Affine;
 typedef Affine<Fq2> G2Affine;
 typedef XYZZ<Fq> G1XYZZ;

@@ -25,9 +25,7 @@
 //          2^(s+1) whatever the level, so one table w_top^(-k), k < 2^power, serves every level of every section.
 // Sections are computed one after the other (their times are reported apart); all of them are validated on the host
 // first: container, sizes, canonical coordinates and curve membership of every input point.
-#include <algorithm>
 #include <memory>
-#include <thread>
 
 #include "binfile.cuh"
 
@@ -55,14 +53,6 @@ HD uint64_t bitrev_bits(uint64_t x, int bits) {
   for (int i = 0; i < bits; i++, x >>= 1) r = (r << 1) | (x & 1);
   return r;
 #endif
-}
-
-template <class F>
-HD Affine<F> to_affine_fast(const XYZZ<F>& p) {
-  if (p.is_inf()) return Affine<F>::inf();
-  const F iz3 = f_inv_fast(p.zzz);
-  const F iz2 = f_sqr(f_mul(iz3, p.zz));
-  return Affine<F>{f_mul(p.x, iz2), f_mul(p.y, iz3)};
 }
 
 // tw[k] = w^k, plain form, for a Montgomery-form w
@@ -141,36 +131,6 @@ struct PtauIn {
   Sect s[16];
 };
 
-template <class F>
-void check_points(const uint8_t* p, uint64_t n, int sec, const F& b) {
-  // first offending point of the section, scanned by all host threads; 1 = coordinate >= q, 2 = off the curve
-  const unsigned nt = std::max(1u, std::min(64u, std::thread::hardware_concurrency()));
-  const uint64_t chunk = (n + nt - 1) / nt;
-  std::vector<uint64_t> first(nt, UINT64_MAX);
-  std::vector<int> kind(nt, 0);
-  auto scan = [&](unsigned t) {
-    for (uint64_t i = t * chunk; i < std::min(n, (t + 1) * chunk); i++) {
-      Affine<F> a;
-      memcpy(&a, p + i * sizeof(Affine<F>), sizeof(Affine<F>));
-      bool inf;
-      if (a.is_inf()) continue;
-      const int k = !(CoordCanon<F>::ok(a.x) && CoordCanon<F>::ok(a.y)) ? 1 : !point_ok(a, b, &inf) ? 2 : 0;
-      if (k) { first[t] = i; kind[t] = k; return; }
-    }
-  };
-  if (n < 4096) {
-    for (unsigned t = 0; t < nt; t++) scan(t);
-  } else {
-    std::vector<std::thread> th;
-    for (unsigned t = 0; t < nt; t++) th.emplace_back(scan, t);
-    for (auto& t : th) t.join();
-  }
-  for (unsigned t = 0; t < nt; t++)
-    if (kind[t])
-      throw ApiError(NZCP_E_RANGE, "ptau: section " + std::to_string(sec) + " point " + std::to_string(first[t]) +
-                                       (kind[t] == 1 ? " has a coordinate >= q" : " is not on the curve"));
-}
-
 // Everything preparePhase2 needs from its input, validated before any device work.
 PtauIn parse_ptau_in(const uint8_t* b, size_t len) {
   PtauIn p;
@@ -191,11 +151,11 @@ PtauIn parse_ptau_in(const uint8_t* b, size_t len) {
       throw ApiError(NZCP_E_FORMAT, "ptau: section " + std::to_string(id) + " size does not match the header power");
   const Fq b1 = curve_b(g1_generator());
   const Fq2 b2 = curve_b(g2_generator());
-  check_points<Fq>(p.s[2].p, 2 * n - 1, 2, b1);
-  check_points<Fq2>(p.s[3].p, n, 3, b2);
-  check_points<Fq>(p.s[4].p, n, 4, b1);
-  check_points<Fq>(p.s[5].p, n, 5, b1);
-  check_points<Fq2>(p.s[6].p, 1, 6, b2);
+  check_points<Fq>("ptau", p.s[2].p, 2 * n - 1, 2, b1);
+  check_points<Fq2>("ptau", p.s[3].p, n, 3, b2);
+  check_points<Fq>("ptau", p.s[4].p, n, 4, b1);
+  check_points<Fq>("ptau", p.s[5].p, n, 5, b1);
+  check_points<Fq2>("ptau", p.s[6].p, 1, 6, b2);
   return p;
 }
 

@@ -5,8 +5,8 @@ yarn.lock:987-999).  The reference's tests build the prover input at /root/refer
 (`{ toBeSigned: bufferToBitArray(bytes), toBeSignedLen }`) and read public signals as witness[1..513] at
 test/nzcp.js:41-48; `publicSignals` below is that same slice, in the same order, as decimal strings.
 
-`zKey` groups newZKey / exportVerificationKey the way snarkjs's main.js does (snarkjs.zKey.newZKey, ...);
-`powersOfTau.preparePhase2` is snarkjs.powersOfTau.preparePhase2.
+`zKey` groups newZKey / contribute / beacon / exportVerificationKey the way snarkjs's main.js does
+(snarkjs.zKey.newZKey, ...); `powersOfTau.preparePhase2` is snarkjs.powersOfTau.preparePhase2.
 
 Same names, argument meaning and error text as snarkjs:
   prove(zkeyFileName, witnessFileName, logger=None)   file args: path | bytes-like | {"type": "mem", "data": ...}
@@ -292,21 +292,59 @@ def exportVerificationKey(zkeyFileName):
     return vk
 
 
+def _write_out(dest, data):
+    if isinstance(dest, dict):
+        dest["data"] = data
+    elif dest is not None:
+        with open(dest, "wb") as f:
+            f.write(data)
+
+
+def _log_sections(logger, timings):
+    if logger:
+        for sid, ms in timings.items():
+            logger.debug("section %d: %.3f ms" % (sid, ms))
+
+
 def preparePhase2(oldPtauFilename, newPTauFilename=None, logger=None, *, device=0):
     """snarkjs powersOfTau.preparePhase2(oldPtauFilename, newPTauFilename): adds the Lagrange-basis sections 12-15 that
     `zkey new` reads, computed on the GPU.  `newPTauFilename`: a path to write, a {"type": "mem"} object that receives
     `.data`, or None.  Returns the prepared .ptau image."""
     timings = {} if logger else None
     data = api.ptau_prepare(oldPtauFilename, device=device, timings=timings)
-    if logger:
-        for sid, ms in timings.items():
-            logger.debug("section %d: %.3f ms" % (sid, ms))
-    if isinstance(newPTauFilename, dict):
-        newPTauFilename["data"] = data
-    elif newPTauFilename is not None:
-        with open(newPTauFilename, "wb") as f:
-            f.write(data)
+    _log_sections(logger, timings)
+    _write_out(newPTauFilename, data)
     return data
+
+
+def contribute(zkeyNameOld, zkeyNameNew, name, entropy, logger=None, *, seed=None, device=0):
+    """snarkjs zKey.contribute(zkeyNameOld, zkeyNameNew, name, entropy): one phase-2 contribution to delta; sections 8
+    and 9 are rescaled on the GPU.  Empty entropy means OS randomness alone (snarkjs would prompt for it).
+    `zkeyNameNew`: a path to write, a {"type": "mem"} object that receives `.data`, or None.  Returns the 64-byte
+    contribution hash.  `seed` (32 bytes) replaces the randomness: for tests only."""
+    timings = {} if logger else None
+    data, h = api.zkey_contribute(zkeyNameOld, name=name or None, entropy=entropy or None, seed=seed, device=device,
+                                  timings=timings)
+    _log_sections(logger, timings)
+    _write_out(zkeyNameNew, data)
+    return h
+
+
+def beacon(zkeyNameOld, zkeyNameNew, name, beaconHashStr, numIterationsExp, logger=None, *, device=0):
+    """snarkjs zKey.beacon(zkeyNameOld, zkeyNameNew, name, beaconHashStr, numIterationsExp): the final, publicly
+    reproducible contribution, its key derived from the hex string beaconHashStr hashed 2^numIterationsExp times.
+    Output and return value as contribute."""
+    try:
+        hb = bytes.fromhex(beaconHashStr)
+    except (TypeError, ValueError):
+        hb = b""
+    if not hb or len(hb) * 2 != len(beaconHashStr):
+        raise NzcpError(_lib.NZCP_E_ARG, "Invalid Beacon Hash. (It must be a valid hexadecimal sequence)")
+    timings = {} if logger else None
+    data, h = api.zkey_beacon(zkeyNameOld, hb, int(numIterationsExp), name=name or None, device=device, timings=timings)
+    _log_sections(logger, timings)
+    _write_out(zkeyNameNew, data)
+    return h
 
 
 class powersOfTau:
@@ -315,6 +353,8 @@ class powersOfTau:
 
 
 class zKey:
-    """snarkjs.zKey namespace: the two entries that border the proving path."""
+    """snarkjs.zKey namespace: the setup entries this library computes and the key export."""
     newZKey = staticmethod(newZKey)
+    contribute = staticmethod(contribute)
+    beacon = staticmethod(beacon)
     exportVerificationKey = staticmethod(exportVerificationKey)
