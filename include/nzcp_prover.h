@@ -27,6 +27,9 @@
  *   nzcp_zkey_contribute*, nzcp_zkey_beacon
  *                       snarkjs zkey_contribute.js phase2contribute and zkey_beacon.js beacon, with the ChaCha of
  *                       ffjavascript random.js (yarn.lock:987-999, 408-416)
+ *   nzcp_zkey_circuit_hash, nzcp_zkey_verify*
+ *                       snarkjs zkey_new.js's circuit hash, zkey_verify_fromr1cs.js verifyFromR1cs and
+ *                       zkey_verify_frominit.js verifyFromInit (yarn.lock:987-999); the pairings stay with the caller
  *   nzcp_field_op       wasmcurves build_f1m.js f1m_mul / f1m_add / f1m_sub (yarn.lock:1132-1135)
  *   nzcp_synth_*        snarkjs zkey_new.js with a known tau in place of the ptau file /root/reference/Makefile:31 names;
  *                       shapes from circuits/nzcp_exampleTest.circom:4 and circuits/nzcp_liveTest.circom:4
@@ -176,6 +179,62 @@ int nzcp_zkey_beacon(const uint8_t* zkey, size_t len, const char* name, const ui
                      uint32_t num_iterations_exp, int device, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64],
                      float section_ms[2]);
 
+/* snarkjs `zkey verify` (zkey_verify_fromr1cs.js verifyFromR1cs, zkey_verify_frominit.js verifyFromInit) and the circuit
+ * hash of zkey_new.js (csrc/verify.cu restates both).
+ * nzcp_zkey_circuit_hash: the csHash snarkjs's newZKey writes into section 10, from an initial key (`zkey new` output) and
+ * the prepared ptau it was made from; ms (optional): [0] device time of the hash kernels, [1] host BLAKE2b time.
+ * nzcp_zkey_verify_from_init checks `zkey` against the initial key `init`; nzcp_zkey_verify_from_r1cs first builds the
+ * initial key from the .r1cs and the ptau (nzcp_zkey_new in host memory, with its circuit hash).
+ * The verdict is split: the pairings are left to the caller.  The library decides every other check in snarkjs's order and
+ * stops at the first that fails (report->failed_step != 0, report->message).  Each pairing check before that point is
+ * returned as a claim e(a, d) = e(b, c), in order.  The verdict is the first false claim, else the library's failure, else
+ * true (nzcp_circom_b200/verifier.py checks the claims, as groth16.verify does).  The C ABI alone does not give it.
+ * Steps (failed_step and claim.step): 1 a point of the key's header, section 10 records or sections 8 / 9 that is not
+ * canonical and on its curve, or delta2 / a g2_spx outside the order-r subgroup (snarkjs checks none of this); 2 "INVALID(i):
+ * Inconsistent transcript"; 3 claim "INVALID(i): public key G1 and G2 do not have the same ration"; 4 claim "INVALID(i):
+ * deltaAfter does not fillow the public key"; 5 "INVALID(i): Key of the beacon does not match. g1_s" / "... g1_sx"; 6
+ * "Different circuit parameters"; 7 "Invalid alpha1" / beta1 / beta2 / gamma2 / delta1; 8 claim "Invalid delta2"; 9
+ * "Circuit does not match"; 10 "IC" / "Coeffs" / "A" / "B1" / "B2" " section is not identical"; 11 claim "L section does not
+ * match"; 12 claim "H section does not match".  (snarkjs's spellings.)
+ * Deviation: the L check draws full-width scalars (snarkjs: 32-bit).  seed (32 bytes, test hook; NULL in use) replaces the
+ * OS randomness that seeds the L and H scalars.
+ * Errors (before any device work): the zkey / ptau / r1cs rejections of nzcp_zkey_contribute and nzcp_zkey_new, a beacon
+ * record without its parameters, an initial key whose sections 3 / 5-7 do not match its header or whose domainSize is not
+ * a power of two, and cirPower = power with N > 2^14, where snarkjs's hashHPoints reads past ptau section 2 (NZCP_E_ARG).
+ * nzcp_zkey_verify_size (host-only) gives the claim and record counts the buffers must hold (2 n + 3 and n).
+ * section_ms (optional): [0] device time of the hash kernels, [1] host BLAKE2b of the circuit hash, [2] the L MSMs,
+ * [3] the H scalar transform, NTT and MSMs. */
+typedef struct nzcp_zkey_verify_claim {
+  int32_t step, record;      /* record: section-10 index for steps 3 and 4, else -1 */
+  uint8_t a[64], b[64];      /* G1, plain x, y (all zero = infinity) */
+  uint8_t c[128], d[128];    /* G2, plain x.c0 x.c1 y.c0 y.c1 */
+} nzcp_zkey_verify_claim;
+typedef struct nzcp_zkey_contribution {
+  uint8_t hash[64];          /* BLAKE2b-512(hashPubKey(record)): the contribution hash snarkjs prints */
+  uint32_t type;             /* 0 contribute, 1 beacon */
+  uint32_t num_iterations_exp, name_len, beacon_hash_len;
+  char name[256];            /* parameter tag 1, not NUL-terminated */
+  uint8_t beacon_hash[256];  /* parameter tag 3 */
+} nzcp_zkey_contribution;
+typedef struct nzcp_zkey_verify_report {
+  int32_t failed_step;       /* 0: every check the library decides passed */
+  int32_t failed_record;     /* section-10 index for steps 2 and 5, else -1 */
+  char message[256];
+  uint32_t n_contributions, n_claims;
+  uint8_t cs_hash[64];       /* the circuit hash computed from the initial key and the ptau */
+} nzcp_zkey_verify_report;
+int nzcp_zkey_circuit_hash(const uint8_t* init, size_t init_len, const uint8_t* ptau, size_t ptau_len, int device,
+                           uint8_t hash[64], float ms[2]);
+int nzcp_zkey_verify_size(const uint8_t* zkey, size_t len, size_t* n_claims, size_t* n_records);
+int nzcp_zkey_verify_from_init(const uint8_t* init, size_t init_len, const uint8_t* ptau, size_t ptau_len, const uint8_t* zkey,
+                               size_t zkey_len, const uint8_t* seed, int device, nzcp_zkey_verify_claim* claims,
+                               size_t claims_cap, nzcp_zkey_contribution* records, size_t records_cap,
+                               nzcp_zkey_verify_report* report, float section_ms[4]);
+int nzcp_zkey_verify_from_r1cs(const uint8_t* r1cs, size_t r1cs_len, const uint8_t* ptau, size_t ptau_len, const uint8_t* zkey,
+                               size_t zkey_len, const uint8_t* seed, int device, nzcp_zkey_verify_claim* claims,
+                               size_t claims_cap, nzcp_zkey_contribution* records, size_t records_cap,
+                               nzcp_zkey_verify_report* report, float section_ms[4]);
+
 /* Work buffers + streams for proofs against `zk`.  Several provers may share one zkey (one per host thread). */
 int nzcp_prover_create(nzcp_zkey* zk, nzcp_prover** out);   /* = mode 0 */
 /* mode 0 = latency (one proof at a time), mode 1 = throughput (meant to run beside other provers on the same GPU;
@@ -307,6 +366,10 @@ int nzcp_host_ptau_prepare(const uint8_t* ptau, size_t len, uint8_t* out, size_t
 int nzcp_host_zkey_contribute(const uint8_t* zkey, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
                               const uint8_t* seed, const uint8_t* beacon_hash, size_t beacon_hash_len,
                               uint32_t num_iterations_exp, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]);
+
+/* nzcp_zkey_circuit_hash with the kernels' per-point code (H differences, point encoding) run on the CPU, for a domain of
+ * at most 4096 (more: NZCP_E_ARG).  Same validation, same hash. */
+int nzcp_host_zkey_circuit_hash(const uint8_t* init, size_t init_len, const uint8_t* ptau, size_t ptau_len, uint8_t hash[64]);
 
 /* ---- synthetic circuits of the NZCP shape (no circom / snarkjs in this environment; SURVEY.md 8d) ---- */
 typedef struct nzcp_synth nzcp_synth;

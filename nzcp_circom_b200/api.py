@@ -321,9 +321,11 @@ def msm_sum_partials(d_partials, count, g2=False, device=0):
     return bytes(out)
 
 
-def zkey_new(r1cs, ptau, device=0):
+def zkey_new(r1cs, ptau, device=0, *, circuit_hash=False):
     """snarkjs `zkey new`: .r1cs + prepared .ptau (path | bytes-like | {"type": "mem"}) -> bytearray with the .zkey image
-    (gamma = delta = 1, no contributions).  The sparse point combinations run on `device` (csrc/setup.cu)."""
+    (gamma = delta = 1, no contributions).  The sparse point combinations run on `device` (csrc/setup.cu).
+    circuit_hash=True stamps the circuit hash snarkjs writes into section 10 (zkey_circuit_hash); only such a key passes
+    `zkey verify`.  The default leaves it zero, as before; it is meant to flip to True in a later release."""
     lib = _lib.load()
     rb, pb = _as_bytes_like(r1cs), _as_bytes_like(ptau)
     size = C.c_size_t()
@@ -332,7 +334,93 @@ def zkey_new(r1cs, ptau, device=0):
     written = C.c_size_t()
     check(lib.nzcp_zkey_new(addr(rb), _nbytes(rb), addr(pb), _nbytes(pb), int(device), addr(out), len(out), C.byref(written)))
     assert written.value == len(out)
+    if circuit_hash:
+        # section 10 (csHash, u32 0) is the last section zkey_new writes
+        out[-68:-4] = zkey_circuit_hash(out, pb, device=device)
     return out
+
+
+def zkey_circuit_hash(init_zkey, ptau, device=0, timings=None):
+    """The circuit hash snarkjs's newZKey writes into section 10 (csrc/verify.cu), from an initial key (`zkey new`
+    output) and the prepared ptau it was made from -> 64 bytes.  `timings` receives "hash_kernels" (device ms) and
+    "blake2b" (host ms)."""
+    lib = _lib.load()
+    zb, pb = _as_bytes_like(init_zkey), _as_bytes_like(ptau)
+    h, ms = bytearray(64), (C.c_float * 2)()
+    check(lib.nzcp_zkey_circuit_hash(addr(zb), _nbytes(zb), addr(pb), _nbytes(pb), int(device), addr(h), ms))
+    if timings is not None:
+        timings.update(hash_kernels=float(ms[0]), blake2b=float(ms[1]))
+    return bytes(h)
+
+
+def host_zkey_circuit_hash(init_zkey, ptau):
+    """zkey_circuit_hash with the kernels' per-point code run on the CPU (domain <= 4096); test hook."""
+    zb, pb = _as_bytes_like(init_zkey), _as_bytes_like(ptau)
+    h = bytearray(64)
+    check(_lib.load().nzcp_host_zkey_circuit_hash(addr(zb), _nbytes(zb), addr(pb), _nbytes(pb), addr(h)))
+    return bytes(h)
+
+
+VERIFY_TIMINGS = ("hash_kernels", "blake2b", "l_msm", "h_ntt_msm")
+CLAIM_MESSAGES = {3: "INVALID(%d): public key G1 and G2 do not have the same ration",
+                  4: "INVALID(%d): deltaAfter does not fillow the public key",
+                  8: "Invalid delta2", 11: "L section does not match", 12: "H section does not match"}
+
+
+def _plain_g1(b):
+    x, y = int.from_bytes(bytes(b[:32]), "little"), int.from_bytes(bytes(b[32:]), "little")
+    return None if x == 0 and y == 0 else (x, y)
+
+
+def _plain_g2(b):
+    c = [int.from_bytes(bytes(b[32 * i:32 * i + 32]), "little") for i in range(4)]
+    return None if not any(c) else ((c[0], c[1]), (c[2], c[3]))
+
+
+def zkey_verify(zkey, ptau, *, r1cs=None, init=None, seed=None, device=0, timings=None):
+    """snarkjs `zkey verify`: checks `zkey` against the circuit, given as the .r1cs (verifyFromR1cs) or as the initial key
+    (verifyFromInit), and the prepared ptau (all: path | bytes-like | {"type": "mem"}).  The library runs every check but
+    the pairings on the GPU and returns the pairing claims that precede its first failure; they are checked here, in order,
+    on the CPU (verifier.same_ratio).  -> dict(ok, message, cs_hash, contributions=[dict(type, name, hash,
+    beacon_hash, num_iterations_exp)]).  `seed` (32 bytes, tests) replaces the OS randomness of the L / H scalars;
+    `timings` receives VERIFY_TIMINGS in ms plus "pairings" (host ms)."""
+    import time
+    from . import verifier
+    if (r1cs is None) == (init is None):
+        raise NzcpError(_lib.NZCP_E_ARG, "zkey_verify: give exactly one of r1cs and init")
+    if seed is not None and len(bytes(seed)) != 32:
+        raise NzcpError(_lib.NZCP_E_ARG, "seed must be 32 bytes")
+    lib = _lib.load()
+    zb, pb = _as_bytes_like(zkey), _as_bytes_like(ptau)
+    n_claims, n_recs = C.c_size_t(), C.c_size_t()
+    check(lib.nzcp_zkey_verify_size(addr(zb), _nbytes(zb), C.byref(n_claims), C.byref(n_recs)))
+    claims = (_lib.VerifyClaim * n_claims.value)()
+    recs = (_lib.Contribution * max(1, n_recs.value))()
+    rep, ms = _lib.VerifyReport(), (C.c_float * 4)()
+    sd = None if seed is None else bytes(seed)
+    if r1cs is not None:
+        cb = _as_bytes_like(r1cs)
+        fn = lib.nzcp_zkey_verify_from_r1cs
+    else:
+        cb = _as_bytes_like(init)
+        fn = lib.nzcp_zkey_verify_from_init
+    check(fn(addr(cb), _nbytes(cb), addr(pb), _nbytes(pb), addr(zb), _nbytes(zb), sd, int(device), claims,
+             n_claims.value, recs, n_recs.value, C.byref(rep), ms))
+    t0 = time.perf_counter()
+    message = None
+    for k in claims[:rep.n_claims]:
+        if not verifier.same_ratio(_plain_g1(k.a), _plain_g1(k.b), _plain_g2(k.c), _plain_g2(k.d)):
+            message = CLAIM_MESSAGES[k.step] % k.record if "%d" in CLAIM_MESSAGES[k.step] else CLAIM_MESSAGES[k.step]
+            break
+    if timings is not None:
+        timings.update(zip(VERIFY_TIMINGS, [float(x) for x in ms]))
+        timings["pairings"] = (time.perf_counter() - t0) * 1e3
+    if message is None and rep.failed_step:
+        message = rep.message.decode(errors="replace")
+    contributions = [{"type": r.type, "name": bytes(r.name[:r.name_len]).decode(errors="replace"), "hash": bytes(r.hash),
+                      "beacon_hash": bytes(r.beacon_hash[:r.beacon_hash_len]), "num_iterations_exp": r.num_iterations_exp}
+                     for r in recs[:n_recs.value]]
+    return {"ok": message is None, "message": message, "cs_hash": bytes(rep.cs_hash), "contributions": contributions}
 
 
 PTAU_SECTIONS = (12, 13, 14, 15)

@@ -20,8 +20,9 @@
 //   section 3 (IC) = K[0..nPublic], section 8 (C) = K[nPublic+1..]   (gamma = delta = 1 at `zkey new` time)
 //   section 9   H[i] = tauG1 Lagrange level cirPower+1, entry 2i+1
 //   section 10  csHash + 0 contributions.  The circuit hash (BLAKE2b-512 over an uncompressed-point transcript) is NOT
-//               computed: the section is written zero-filled.  `groth16 prove`, `zkey export verificationkey` and this
-//               library do not read it; `zkey verify` / `zkey contribute` do and will refuse the file.
+//               computed here: the section is written zero-filled.  `groth16 prove`, `zkey export verificationkey` and
+//               `zkey contribute` do not check it; `zkey verify` refuses such a key.  verify.cu computes it from this
+//               output and the ptau (nzcp_zkey_circuit_hash; api.zkey_new(..., circuit_hash=True) stamps it).
 // Sections are written in zkey_new.js's own order: 1, 2, 4, 3, 9, 8, 5, 6, 7, 10.
 //
 // B200 design: the four sparse point combinations are one kernel each, one thread per wire walking its term list
@@ -30,21 +31,9 @@
 // One-time work per circuit.
 #include <memory>
 
-#include "binfile.cuh"
+#include "mpc.cuh"
 
 namespace nzcp {
-
-G1Affine g1_generator();  // synth.cu
-G2Affine g2_generator();
-
-namespace {
-
-struct R1cs {
-  uint32_t n_wires = 0, n_pub_out = 0, n_pub_in = 0, n_prv_in = 0, n_constraints = 0, n_public = 0;
-  const uint8_t* cons = nullptr;
-  uint64_t cons_len = 0;
-  uint64_t n_terms[3] = {0, 0, 0};   // A, B, C terms in total
-};
 
 R1cs parse_r1cs(const uint8_t* b, size_t len) {
   Sect s[4];
@@ -81,11 +70,6 @@ R1cs parse_r1cs(const uint8_t* b, size_t len) {
   return r;
 }
 
-struct Ptau {
-  uint32_t power = 0;
-  Sect s[16];
-};
-
 Ptau parse_ptau(const uint8_t* b, size_t len) {
   Ptau p;
   parse_bin(b, len, "ptau", p.s, 15);
@@ -110,6 +94,8 @@ uint32_t circuit_power(const R1cs& r) {
   while (v >> (lg + 1)) lg++;      // floor(log2(v)); snarkjs log2(0) = 0
   return lg + 1;
 }
+
+namespace {
 
 struct Term {
   uint32_t point;   // Lagrange point index (constraint number) | source << 30
@@ -163,6 +149,8 @@ void run_combo(const Combo& cb, const Fr* d_coefs, const void* d_src0, const voi
     NZCP_CUDA(cudaMemcpy(host_out, d_out, (size_t)n_wires * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
   }
 }
+
+}  // namespace
 
 size_t zkey_new_size(const R1cs& r, uint32_t cir_power) {
   const uint64_t n = (uint64_t)1 << cir_power, m = r.n_wires, np = r.n_public;
@@ -322,7 +310,6 @@ void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b
   if (written) *written = w.pos;
 }
 
-}  // namespace
 }  // namespace nzcp
 
 using namespace nzcp;

@@ -5,8 +5,8 @@ yarn.lock:987-999).  The reference's tests build the prover input at /root/refer
 (`{ toBeSigned: bufferToBitArray(bytes), toBeSignedLen }`) and read public signals as witness[1..513] at
 test/nzcp.js:41-48; `publicSignals` below is that same slice, in the same order, as decimal strings.
 
-`zKey` groups newZKey / contribute / beacon / exportVerificationKey the way snarkjs's main.js does
-(snarkjs.zKey.newZKey, ...); `powersOfTau.preparePhase2` is snarkjs.powersOfTau.preparePhase2.
+`zKey` groups newZKey / contribute / beacon / verifyFromR1cs / verifyFromInit / exportVerificationKey the way snarkjs's
+main.js does (snarkjs.zKey.newZKey, ...); `powersOfTau.preparePhase2` is snarkjs.powersOfTau.preparePhase2.
 
 Same names, argument meaning and error text as snarkjs:
   prove(zkeyFileName, witnessFileName, logger=None)   file args: path | bytes-like | {"type": "mem", "data": ...}
@@ -235,13 +235,14 @@ def verify(vk_verifier, publicSignals, proof, logger=None):
     return verifier.verify(vk_verifier, publicSignals, proof, logger)
 
 
-def newZKey(r1csName, ptauName, zkeyName=None, logger=None, *, device=0):
+def newZKey(r1csName, ptauName, zkeyName=None, logger=None, *, device=0, circuit_hash=False):
     """snarkjs zKey.newZKey(r1csName, ptauName, zkeyName): the circuit-specific key from an .r1cs and a prepared .ptau,
     computed on the GPU.  `zkeyName`: a path to write, a {"type": "mem"} object that receives `.data`, or None.
-    Returns the .zkey image (snarkjs returns the circuit hash, which is not computed here -- csrc/setup.cu)."""
+    Returns the .zkey image (snarkjs returns the circuit hash).  circuit_hash=True computes the circuit hash and writes it
+    into section 10 as snarkjs does, which `zkey verify` requires; the default still leaves it zero (api.zkey_new)."""
     if logger:
         logger.info("Reading r1cs / ptau, combining points on the GPU")
-    data = api.zkey_new(r1csName, ptauName, device=device)
+    data = api.zkey_new(r1csName, ptauName, device=device, circuit_hash=circuit_hash)
     if isinstance(zkeyName, dict):
         zkeyName["data"] = data
     elif zkeyName is not None:
@@ -347,6 +348,45 @@ def beacon(zkeyNameOld, zkeyNameNew, name, beaconHashStr, numIterationsExp, logg
     return h
 
 
+def _format_hash(h, title):
+    """misc.js formatHash: the title, then the hash in four lines of four 8-hex-digit groups."""
+    hx = h.hex()
+    rows = ["\t\t" + " ".join(hx[32 * r + 8 * c:32 * r + 8 * c + 8] for c in range(4)) for r in range(4)]
+    return "\n".join([title] + rows)
+
+
+def _verify(res, logger):
+    if logger:
+        if not res["ok"]:
+            logger.error(res["message"])
+        else:
+            logger.info(_format_hash(res["cs_hash"], "Circuit Hash: "))
+            for i in range(len(res["contributions"]) - 1, -1, -1):
+                c = res["contributions"][i]
+                logger.info("-------------------------")
+                logger.info(_format_hash(c["hash"], "contribution #%d %s:" % (i + 1, c["name"])))
+                if c["type"] == 1:
+                    logger.info("Beacon generator: %s" % c["beacon_hash"].hex())
+                    logger.info("Beacon iterations Exp: %d" % c["num_iterations_exp"])
+            logger.info("-------------------------")
+            logger.info("ZKey Ok!")
+    return res["ok"]
+
+
+def verifyFromR1cs(r1csFileName, pTauFileName, zkeyFileName, logger=None, *, seed=None, device=0):
+    """snarkjs zKey.verifyFromR1cs: rebuilds the initial key (newZKey with its circuit hash) and checks `zkeyFileName`
+    against it (verifyFromInit).  Returns a bool; the logger gets snarkjs's messages.  `seed` (32 bytes) replaces the OS
+    randomness of the L / H checks: for tests only."""
+    return _verify(api.zkey_verify(zkeyFileName, pTauFileName, r1cs=r1csFileName, seed=seed, device=device), logger)
+
+
+def verifyFromInit(initFileName, pTauFileName, zkeyFileName, logger=None, *, seed=None, device=0):
+    """snarkjs zKey.verifyFromInit: every contribution of `zkeyFileName` chains onto the one before, and the key is the
+    initial key `initFileName` with the contributed delta (sections 8 and 9 through random linear combinations on the GPU,
+    pairings on the CPU).  Returns a bool, as verifyFromR1cs."""
+    return _verify(api.zkey_verify(zkeyFileName, pTauFileName, init=initFileName, seed=seed, device=device), logger)
+
+
 class powersOfTau:
     """snarkjs.powersOfTau namespace: the one entry this library computes."""
     preparePhase2 = staticmethod(preparePhase2)
@@ -357,4 +397,6 @@ class zKey:
     newZKey = staticmethod(newZKey)
     contribute = staticmethod(contribute)
     beacon = staticmethod(beacon)
+    verifyFromR1cs = staticmethod(verifyFromR1cs)
+    verifyFromInit = staticmethod(verifyFromInit)
     exportVerificationKey = staticmethod(exportVerificationKey)

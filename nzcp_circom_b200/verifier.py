@@ -234,6 +234,11 @@ def pairing_product_is_one(pairs):
     return final_exp(f) == F12_ONE
 
 
+def same_ratio(a, b, c, d):
+    """snarkjs sameRatio(a, b, c, d): e(a, d) == e(b, c) -- the pairing half of `zkey verify` (api.zkey_verify)."""
+    return pairing_product_is_one([(a, d), (g1_neg(b), c)])
+
+
 # ---------------------------------------------------------------------------------------- snarkjs-shaped verify
 class _BadPoint(ValueError):
     pass
