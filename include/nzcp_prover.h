@@ -24,6 +24,9 @@
  *   nzcp_zkey_selfcheck no snarkjs equivalent: the format facts of SURVEY.md 8c-3, for the first real key
  *   nzcp_ptau_prepare*  snarkjs powersoftau_preparephase2.js preparePhase2(oldPtauFilename, newPTauFilename) and the group
  *                       ifft of ffjavascript engine_fft.js it runs per level (yarn.lock:987-999, 408-416)
+ *   nzcp_ptau_new*, nzcp_ptau_contribute*, nzcp_ptau_beacon
+ *                       snarkjs powersoftau_new.js newAccumulator, powersoftau_contribute.js contribute and
+ *                       powersoftau_beacon.js beacon, with keypair.js createPTauKey (yarn.lock:987-999)
  *   nzcp_zkey_contribute*, nzcp_zkey_beacon
  *                       snarkjs zkey_contribute.js phase2contribute and zkey_beacon.js beacon, with the ChaCha of
  *                       ffjavascript random.js (yarn.lock:987-999, 408-416)
@@ -153,6 +156,36 @@ int nzcp_zkey_new(const uint8_t* r1cs, size_t r1cs_len, const uint8_t* ptau, siz
 int nzcp_ptau_prepare_size(const uint8_t* ptau, size_t len, size_t* out_size);
 int nzcp_ptau_prepare(const uint8_t* ptau, size_t len, int device, uint8_t* out, size_t cap, size_t* written,
                       float section_ms[4]);
+
+/* snarkjs `powersoftau new` (powersoftau_new.js newAccumulator): a fresh phase-1 file of 2^power, power 1..28 (else
+ * NZCP_E_ARG): header (n8, q, power, ceremonyPower = power), sections 2-6 the G1 / G2 generators (tau = alpha = beta = 1),
+ * section 7 no contributions.  Host only.  `hash` (optional, NULL: skipped; it costs a BLAKE2b pass over ~384 * 2^power
+ * bytes) receives the first challenge hash, snarkjs's "First Contribution Hash".  nzcp_ptau_new_size gives the file size. */
+int nzcp_ptau_new_size(uint32_t power, size_t* out_size);
+int nzcp_ptau_new(uint32_t power, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]);
+
+/* snarkjs `powersoftau contribute` / `powersoftau beacon` (powersoftau_contribute.js contribute, powersoftau_beacon.js
+ * beacon): one phase-1 contribution (tau, alpha, beta) drawn by keypair.js createPTauKey from the rng and the challenge
+ * (the last record's nextChallenge, or the first challenge hash).  Point i of sections 2 (tauG1), 3 (tauG2), 4 (alphaTauG1),
+ * 5 (betaTauG1) and 6 (betaG2) becomes (first * tau^i) * P_i with first = 1, 1, alpha, beta, beta, on `device`; section 7
+ * gets a new record after the earlier ones (type 0 contribute, 1 beacon; parameters as nzcp_zkey_contribute).  Output:
+ * sections 1-7 in id order, header rewritten with ceremonyPower = power; sections 12-15 of a prepared input are dropped.
+ * `hash` receives the 64-byte response hash snarkjs returns.  The rng is that of nzcp_zkey_contribute / nzcp_zkey_beacon
+ * (`seed`: 32 bytes, test hook, NULL in use).  See csrc/ptau_contribute.cu for the restated algorithm.
+ * All functions reject before any device work: a file that is not a ptau or has no header (NZCP_E_FORMAT); not over bn128
+ * (NZCP_E_CURVE); power outside 1..28, a missing section 2-7 ("Missing section N"), a section 2-6 whose size does not match
+ * the power, a section 7 that is truncated, has trailing bytes, unsorted or unknown parameters (NZCP_E_FORMAT); power !=
+ * ceremonyPower (NZCP_E_ARG, "This file has been reduced. You cannot contribute into a reduced file."); an input point with
+ * a coordinate >= q or off its curve (NZCP_E_RANGE); a name longer than 64 bytes, a beacon hash of 0 or >= 256 bytes or
+ * num_iterations_exp outside 10..63 (NZCP_E_ARG, as nzcp_zkey_contribute).  nzcp_ptau_contribute_size is host-only.
+ * ms (optional): [0]-[4] key-kernel device time of sections 2-6, [5] encode-kernel device time, [6] host BLAKE2b time. */
+int nzcp_ptau_contribute_size(const uint8_t* ptau, size_t len, const char* name, size_t beacon_hash_len, size_t* out_size);
+int nzcp_ptau_contribute(const uint8_t* ptau, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
+                         const uint8_t* seed, int device, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64],
+                         float ms[7]);
+int nzcp_ptau_beacon(const uint8_t* ptau, size_t len, const char* name, const uint8_t* beacon_hash, size_t beacon_hash_len,
+                     uint32_t num_iterations_exp, int device, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64],
+                     float ms[7]);
 
 /* snarkjs `zkey contribute` / `zkey beacon` (zkey_contribute.js phase2contribute, zkey_beacon.js beacon): one phase-2
  * contribution k to a Groth16 key.  delta1 and delta2 of the header become k * delta, every point of sections 8 (L) and 9
@@ -364,6 +397,12 @@ int nzcp_host_ptau_prepare(const uint8_t* ptau, size_t len, uint8_t* out, size_t
 /* nzcp_zkey_contribute (beacon_hash == NULL) or nzcp_zkey_beacon with the kernel's per-point code run on the CPU, for
  * sections 8 + 9 of at most 4096 points (more: NZCP_E_ARG).  Same validation, same output bytes and hash. */
 int nzcp_host_zkey_contribute(const uint8_t* zkey, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
+                              const uint8_t* seed, const uint8_t* beacon_hash, size_t beacon_hash_len,
+                              uint32_t num_iterations_exp, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]);
+
+/* nzcp_ptau_contribute (beacon_hash == NULL) or nzcp_ptau_beacon with the kernels' per-point code (key, encodings) run
+ * on the CPU, for power <= 4 (more: NZCP_E_ARG).  Same validation, same output bytes and hash. */
+int nzcp_host_ptau_contribute(const uint8_t* ptau, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
                               const uint8_t* seed, const uint8_t* beacon_hash, size_t beacon_hash_len,
                               uint32_t num_iterations_exp, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]);
 

@@ -92,6 +92,13 @@ SIGNATURES = {
     "nzcp_zkey_new": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, C.c_int, _U8P, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nzcp_ptau_prepare_size": (C.c_int, [_U8P, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nzcp_ptau_prepare": (C.c_int, [_U8P, C.c_size_t, C.c_int, _U8P, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_float)]),
+    "nzcp_ptau_new_size": (C.c_int, [C.c_uint32, C.POINTER(C.c_size_t)]),
+    "nzcp_ptau_new": (C.c_int, [C.c_uint32, _U8P, C.c_size_t, C.POINTER(C.c_size_t), _U8P]),
+    "nzcp_ptau_contribute_size": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "nzcp_ptau_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, C.c_int, _U8P, C.c_size_t,
+                                       C.POINTER(C.c_size_t), _U8P, C.POINTER(C.c_float)]),
+    "nzcp_ptau_beacon": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, C.c_uint32, C.c_int, _U8P, C.c_size_t,
+                                   C.POINTER(C.c_size_t), _U8P, C.POINTER(C.c_float)]),
     "nzcp_zkey_contribute_size": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nzcp_zkey_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, C.c_int, _U8P, C.c_size_t,
                                        C.POINTER(C.c_size_t), _U8P, C.POINTER(C.c_float)]),
@@ -125,6 +132,8 @@ SIGNATURES = {
     "nzcp_host_root_of_unity": (C.c_int, [C.c_int, _U8P]),
     "nzcp_host_ptau_prepare": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nzcp_host_zkey_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, _U8P, C.c_size_t,
+                                            C.c_uint32, _U8P, C.c_size_t, C.POINTER(C.c_size_t), _U8P]),
+    "nzcp_host_ptau_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, _U8P, C.c_size_t,
                                             C.c_uint32, _U8P, C.c_size_t, C.POINTER(C.c_size_t), _U8P]),
     "nzcp_host_zkey_circuit_hash": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, _U8P]),
     "nzcp_host_msm_sim": (C.c_int, [_U8P, _U8P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, _U8P]),

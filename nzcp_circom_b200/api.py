@@ -499,6 +499,80 @@ def zkey_beacon(zkey, beacon_hash, num_iterations_exp, name=None, device=0, timi
     return out, bytes(h)
 
 
+def ptau_new(power, first_challenge=True):
+    """snarkjs `powersoftau new`: a fresh phase-1 .ptau of 2^power (1..28) -> (bytearray, 64-byte first challenge hash, or
+    None with first_challenge=False, which skips a BLAKE2b pass over ~384 * 2^power bytes).  Host only."""
+    lib = _lib.load()
+    size = C.c_size_t()
+    check(lib.nzcp_ptau_new_size(int(power), C.byref(size)))
+    out = bytearray(size.value)
+    written, h = C.c_size_t(), bytearray(64) if first_challenge else None
+    check(lib.nzcp_ptau_new(int(power), addr(out), len(out), C.byref(written), addr(h)))
+    assert written.value == len(out)
+    return out, None if h is None else bytes(h)
+
+
+PTAU_CONTRIBUTE_TIMINGS = (2, 3, 4, 5, 6, "encode", "blake2b")
+
+
+def _ptau_contribute_out(lib, pb, name, beacon_len):
+    size = C.c_size_t()
+    check(lib.nzcp_ptau_contribute_size(addr(pb), _nbytes(pb), name, beacon_len, C.byref(size)))
+    return bytearray(size.value)
+
+
+def ptau_contribute(ptau, name=None, entropy=None, seed=None, device=0, timings=None):
+    """snarkjs `powersoftau contribute`: a phase-1 .ptau (path | bytes-like | {"type": "mem"}) -> (bytearray with the new
+    file, 64-byte response hash).  The random key comes from BLAKE2b(64 OS-random bytes || entropy) (str: UTF-8); `seed`
+    (32 bytes, tests) seeds the ChaCha directly instead.  Sections 2-6 are multiplied on `device`; `timings` receives the
+    key-kernel device ms keyed 2..6, "encode" (encode kernels, device ms) and "blake2b" (host ms)."""
+    lib = _lib.load()
+    pb = _as_bytes_like(ptau)
+    nb, eb = _utf8(name), _utf8(entropy) or b""
+    if seed is not None and len(bytes(seed)) != 32:
+        raise NzcpError(_lib.NZCP_E_ARG, "seed must be 32 bytes")
+    out = _ptau_contribute_out(lib, pb, nb, 0)
+    written, h, ms = C.c_size_t(), bytearray(64), (C.c_float * 7)()
+    check(lib.nzcp_ptau_contribute(addr(pb), _nbytes(pb), nb, addr(eb) if eb else None, len(eb),
+                                   None if seed is None else bytes(seed), int(device), addr(out), len(out),
+                                   C.byref(written), addr(h), ms))
+    assert written.value == len(out)
+    if timings is not None:
+        timings.update(zip(PTAU_CONTRIBUTE_TIMINGS, [float(x) for x in ms]))
+    return out, bytes(h)
+
+
+def ptau_beacon(ptau, beacon_hash, num_iterations_exp, name=None, device=0, timings=None):
+    """snarkjs `powersoftau beacon`: as ptau_contribute, with the random key derived from `beacon_hash` (bytes) hashed
+    with SHA-256 2^num_iterations_exp times (10..63)."""
+    lib = _lib.load()
+    pb = _as_bytes_like(ptau)
+    nb, hb = _utf8(name), bytes(beacon_hash)
+    out = _ptau_contribute_out(lib, pb, nb, len(hb))
+    written, h, ms = C.c_size_t(), bytearray(64), (C.c_float * 7)()
+    check(lib.nzcp_ptau_beacon(addr(pb), _nbytes(pb), nb, hb, len(hb), int(num_iterations_exp), int(device), addr(out),
+                               len(out), C.byref(written), addr(h), ms))
+    assert written.value == len(out)
+    if timings is not None:
+        timings.update(zip(PTAU_CONTRIBUTE_TIMINGS, [float(x) for x in ms]))
+    return out, bytes(h)
+
+
+def host_ptau_contribute(ptau, name=None, entropy=None, seed=None, beacon_hash=None, num_iterations_exp=0):
+    """CPU run of ptau_contribute (beacon_hash None) or ptau_beacon, power <= 4 -> the same (bytearray, hash)."""
+    lib = _lib.load()
+    pb = _as_bytes_like(ptau)
+    nb, eb = _utf8(name), _utf8(entropy) or b""
+    hb = None if beacon_hash is None else bytes(beacon_hash)
+    out = _ptau_contribute_out(lib, pb, nb, len(hb) if hb else 0)
+    written, h = C.c_size_t(), bytearray(64)
+    check(lib.nzcp_host_ptau_contribute(addr(pb), _nbytes(pb), nb, addr(eb) if eb else None, len(eb),
+                                        None if seed is None else bytes(seed), hb, len(hb) if hb is not None else 0,
+                                        int(num_iterations_exp), addr(out), len(out), C.byref(written), addr(h)))
+    assert written.value == len(out)
+    return out, bytes(h)
+
+
 def zkey_selfcheck(zkey, device=0):
     """Format self-checks of SURVEY.md 8c-3 on a .zkey image (path | bytes-like | {"type": "mem"}) -> dict; ["ok"] is
     the verdict.  Meant for the first REAL snarkjs-made key: it pins the section-4 `coef * R^2` convention, the moduli

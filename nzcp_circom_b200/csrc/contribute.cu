@@ -26,10 +26,6 @@
 // sections 8 and 9, 2 x 2^27 points at most (8.6 GB each, resident in HBM one at a time): one thread per point,
 // x[i] = to_affine_fast(k^-1 * x[i]) with the signed 4-bit window of ec.cuh scalar_mul_accumulate.  The scalar is the
 // same for the whole launch, so every lane takes the same additions at the same digits.
-#include <sys/random.h>
-
-#include <memory>
-
 #include "mpc.cuh"
 
 namespace nzcp {
@@ -47,31 +43,6 @@ __global__ void __launch_bounds__(128) zkey_scale_kernel(G1Affine* __restrict__ 
 }
 
 namespace {
-
-// What the caller asks for: a contribution (beacon_len == 0) or a beacon.
-struct Args {
-  const char* name = nullptr;
-  size_t name_len = 0;
-  const uint8_t* entropy = nullptr;
-  size_t entropy_len = 0;
-  const uint8_t* seed = nullptr;
-  const uint8_t* beacon = nullptr;
-  size_t beacon_len = 0;
-  uint32_t exp = 0;
-};
-
-void check_name(const char* name, size_t* len) {
-  *len = name ? strlen(name) : 0;
-  if (*len > 64) throw ApiError(NZCP_E_ARG, "zkey: contribution name longer than 64 bytes");
-}
-
-void check_beacon_len(size_t len) {
-  if (len >= 256) throw ApiError(NZCP_E_ARG, "Maximum lenght of beacon hash is 255 bytes");
-}
-
-size_t params_len(size_t name_len, size_t beacon_len) {
-  return (name_len ? 2 + name_len : 0) + (beacon_len ? 2 + 2 + beacon_len : 0);
-}
 
 size_t contribute_size(const ZkeyIn& z, size_t name_len, size_t beacon_len) {
   size_t total = 12 + 10 * 12 + 4 + kHeaderLen;
@@ -105,15 +76,10 @@ void scale_section_host(const uint8_t* src, uint64_t n, const Fr& k, uint8_t* ds
 }
 
 // device < 0: the host hook.
-void contribute_impl(const uint8_t* b, size_t len, Args a, int device, uint8_t* out, size_t cap, size_t* written,
+void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, uint8_t* out, size_t cap, size_t* written,
                      uint8_t* hash_out, float* section_ms) {
-  check_name(a.name, &a.name_len);
-  check_beacon_len(a.beacon_len);
+  check_contrib_args("zkey", a);
   const bool beacon = a.beacon != nullptr;
-  if (beacon) {
-    if (a.beacon_len == 0) throw ApiError(NZCP_E_ARG, "Invalid Beacon Hash. (It must be a valid hexadecimal sequence)");
-    if (a.exp < 10 || a.exp > 63) throw ApiError(NZCP_E_ARG, "Invalid numIterationsExp. (Must be between 10 and 63)");
-  }
   const ZkeyIn z = parse_zkey_in(b, len);
   const size_t total = contribute_size(z, a.name_len, beacon ? a.beacon_len : 0);
   if (cap < total) throw ApiError(NZCP_E_ARG, "output buffer too small");
@@ -124,22 +90,7 @@ void contribute_impl(const uint8_t* b, size_t len, Args a, int device, uint8_t* 
 
   // ---- the rng
   uint8_t seed[64];
-  if (beacon) {
-    beacon_seed(a.beacon, a.beacon_len, a.exp, seed);
-  } else if (a.seed) {
-    memcpy(seed, a.seed, 32);
-  } else {
-    uint8_t os[64];
-    for (size_t got = 0; got < sizeof os;) {
-      const ssize_t r = getrandom(os + got, sizeof os - got, 0);
-      if (r <= 0) throw ApiError(NZCP_E_INTERNAL, "zkey contribute: no OS randomness");
-      got += (size_t)r;
-    }
-    Blake2b512 h;
-    h.update(os, sizeof os);
-    if (a.entropy_len) h.update(a.entropy, a.entropy_len);
-    h.final(seed);
-  }
+  contrib_seed(a, seed);
   ChaCha rng(seed);
 
   // ---- the contribution (host: O(1) multiplications)
@@ -182,14 +133,7 @@ void contribute_impl(const uint8_t* b, size_t len, Args a, int device, uint8_t* 
   memcpy(fixed + 384, &type, 4);
   memcpy(fixed + 388, &plen, 4);
   std::vector<uint8_t> rec(fixed, fixed + kRecFixed);
-  if (a.name_len) {
-    rec.insert(rec.end(), {1, (uint8_t)a.name_len});
-    rec.insert(rec.end(), a.name, a.name + a.name_len);
-  }
-  if (beacon) {
-    rec.insert(rec.end(), {2, (uint8_t)a.exp, 3, (uint8_t)a.beacon_len});
-    rec.insert(rec.end(), a.beacon, a.beacon + a.beacon_len);
-  }
+  append_params(rec, a);
   if (hash_out) {
     Blake2b512 ch;
     hash_pub_key(ch, rec.data());
@@ -243,7 +187,7 @@ int nzcp_zkey_contribute_size(const uint8_t* zkey, size_t len, const char* name,
   return api_guard([&] {
     if (!zkey || !out_size) throw ApiError(NZCP_E_ARG, "null argument");
     size_t name_len;
-    check_name(name, &name_len);
+    check_name("zkey", name, &name_len);
     check_beacon_len(beacon_hash_len);
     *out_size = contribute_size(parse_zkey_in(zkey, len), name_len, beacon_hash_len);
   });
@@ -255,7 +199,7 @@ int nzcp_zkey_contribute(const uint8_t* zkey, size_t len, const char* name, cons
   return api_guard([&] {
     if (!zkey || !out || (entropy_len && !entropy)) throw ApiError(NZCP_E_ARG, "null argument");
     if (device < 0) throw ApiError(NZCP_E_ARG, "device index out of range");
-    Args a;
+    ContribArgs a;
     a.name = name;
     a.entropy = entropy;
     a.entropy_len = entropy_len;
@@ -270,7 +214,7 @@ int nzcp_zkey_beacon(const uint8_t* zkey, size_t len, const char* name, const ui
   return api_guard([&] {
     if (!zkey || !out || !beacon_hash) throw ApiError(NZCP_E_ARG, "null argument");
     if (device < 0) throw ApiError(NZCP_E_ARG, "device index out of range");
-    Args a;
+    ContribArgs a;
     a.name = name;
     a.beacon = beacon_hash;
     a.beacon_len = beacon_hash_len;
@@ -284,7 +228,7 @@ int nzcp_host_zkey_contribute(const uint8_t* zkey, size_t len, const char* name,
                               uint32_t num_iterations_exp, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]) {
   return api_guard([&] {
     if (!zkey || !out || (entropy_len && !entropy)) throw ApiError(NZCP_E_ARG, "null argument");
-    Args a;
+    ContribArgs a;
     a.name = name;
     a.entropy = entropy;
     a.entropy_len = entropy_len;

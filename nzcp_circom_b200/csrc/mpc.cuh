@@ -1,7 +1,13 @@
-// Host code shared by the phase-2 ceremony entry points (contribute.cu `zkey contribute` / `zkey beacon`, verify.cu
-// `zkey verify`, setup.cu `zkey new`): BLAKE2b-512 and SHA-256, ffjavascript's ChaCha, F/G.fromRng, the uncompressed point
-// encoding of hashPubKey, the .zkey / section-10 reader, and the .r1cs / .ptau readers and the key writer of setup.cu.
+// Code shared by the ceremony entry points (contribute.cu `zkey contribute` / `zkey beacon`, verify.cu `zkey verify`,
+// setup.cu `zkey new`, ptau_contribute.cu `powersoftau new` / `contribute` / `beacon`): BLAKE2b-512 and SHA-256,
+// ffjavascript's ChaCha, F/G.fromRng, the uncompressed and compressed point encodings (host and device) with the chunked
+// point hasher, the .zkey / contribution-record reader, and the .r1cs / .ptau readers and the key writer of setup.cu.
 #pragma once
+#include <sys/random.h>
+
+#include <chrono>
+#include <memory>
+
 #include "binfile.cuh"
 
 namespace nzcp {
@@ -35,7 +41,7 @@ namespace {
 // ------------------------------------------------------------------------------------------------ hashes (host)
 struct Blake2b512 {   // RFC 7693, unkeyed, 64-byte digest
   uint64_t h[8], t = 0;
-  uint8_t buf[128];
+  uint8_t buf[128] = {};   // zero at init, as the RFC's blake2b_ctx: partial() serializes stale bytes too
   size_t n = 0;
   static constexpr uint64_t kIv[8] = {0x6a09e667f3bcc908ull, 0xbb67ae8584caa73bull, 0x3c6ef372fe94f82bull,
                                       0xa54ff53a5f1d36f1ull, 0x510e527fade682d1ull, 0x9b05688c2b3e6c1full,
@@ -88,6 +94,17 @@ struct Blake2b512 {   // RFC 7693, unkeyed, 64-byte digest
     memset(buf + n, 0, 128 - n);
     compress(true);
     memcpy(out, h, 64);
+  }
+  // The state as blake2b-wasm's getPartialHash returns it: RFC 7693's blake2b_ctx, 216 bytes: b[128] (stale bytes past c
+  // kept), h[8] and t[2] as u64 LE, c and outlen (64) as u32 LE.  c = 128 when a full block waits (lazy compression).
+  void partial(uint8_t out[216]) const {
+    const uint64_t tt[2] = {t, 0};
+    const uint32_t c = (uint32_t)n, outlen = 64;
+    memcpy(out, buf, 128);
+    memcpy(out + 128, h, 64);
+    memcpy(out + 192, tt, 16);
+    memcpy(out + 208, &c, 4);
+    memcpy(out + 212, &outlen, 4);
   }
 };
 
@@ -283,6 +300,76 @@ void beacon_seed(const uint8_t* beacon, size_t len, uint32_t exp, uint8_t seed[3
   memcpy(seed, cur.data(), 32);
 }
 
+// ------------------------------------------------------------------------------------------------ contribute / beacon
+// What a caller of `contribute` (beacon == nullptr) or `beacon` asks for.
+struct ContribArgs {
+  const char* name = nullptr;
+  size_t name_len = 0;
+  const uint8_t* entropy = nullptr;
+  size_t entropy_len = 0;
+  const uint8_t* seed = nullptr;
+  const uint8_t* beacon = nullptr;
+  size_t beacon_len = 0;
+  uint32_t exp = 0;
+};
+
+// kind: "zkey" or "ptau", for the message.  A name longer than 64 bytes is rejected (snarkjs cuts it at 64 characters,
+// and a cut in bytes could split a UTF-8 sequence).
+void check_name(const char* kind, const char* name, size_t* len) {
+  *len = name ? strlen(name) : 0;
+  if (*len > 64) throw ApiError(NZCP_E_ARG, std::string(kind) + ": contribution name longer than 64 bytes");
+}
+
+void check_beacon_len(size_t len) {
+  if (len >= 256) throw ApiError(NZCP_E_ARG, "Maximum lenght of beacon hash is 255 bytes");
+}
+
+void check_contrib_args(const char* kind, ContribArgs& a) {
+  check_name(kind, a.name, &a.name_len);
+  check_beacon_len(a.beacon_len);
+  if (a.beacon) {
+    if (a.beacon_len == 0) throw ApiError(NZCP_E_ARG, "Invalid Beacon Hash. (It must be a valid hexadecimal sequence)");
+    if (a.exp < 10 || a.exp > 63) throw ApiError(NZCP_E_ARG, "Invalid numIterationsExp. (Must be between 10 and 63)");
+  }
+}
+
+size_t params_len(size_t name_len, size_t beacon_len) {
+  return (name_len ? 2 + name_len : 0) + (beacon_len ? 2 + 2 + beacon_len : 0);
+}
+
+// The record's parameters: tag 1 name (if any), tag 2 numIterationsExp and tag 3 beaconHash (beacon only).
+void append_params(std::vector<uint8_t>& rec, const ContribArgs& a) {
+  if (a.name_len) {
+    rec.insert(rec.end(), {1, (uint8_t)a.name_len});
+    rec.insert(rec.end(), a.name, a.name + a.name_len);
+  }
+  if (a.beacon) {
+    rec.insert(rec.end(), {2, (uint8_t)a.exp, 3, (uint8_t)a.beacon_len});
+    rec.insert(rec.end(), a.beacon, a.beacon + a.beacon_len);
+  }
+}
+
+// The ChaCha seed: beacon_seed for a beacon; else BLAKE2b-512(64 OS-random bytes || entropy) (misc.js getRandomRng), or the
+// 32-byte test seed.
+void contrib_seed(const ContribArgs& a, uint8_t seed[64]) {
+  if (a.beacon) {
+    beacon_seed(a.beacon, a.beacon_len, a.exp, seed);
+  } else if (a.seed) {
+    memcpy(seed, a.seed, 32);
+  } else {
+    uint8_t os[64];
+    for (size_t got = 0; got < sizeof os;) {
+      const ssize_t r = getrandom(os + got, sizeof os - got, 0);
+      if (r <= 0) throw ApiError(NZCP_E_INTERNAL, "contribute: no OS randomness");
+      got += (size_t)r;
+    }
+    Blake2b512 h;
+    h.update(os, sizeof os);
+    if (a.entropy_len) h.update(a.entropy, a.entropy_len);
+    h.final(seed);
+  }
+}
+
 // hashToG2 (zkey_utils.js): G2.fromRng(ChaCha(transcript[0..32) as 8 BE words)), times the G2 cofactor 2q - r.
 G2Affine hash_to_g2(const uint8_t transcript[64]) {
   uint32_t h2[8];
@@ -350,23 +437,24 @@ struct ZkeyIn {
   std::vector<size_t> rec_len;
 };
 
-// readMPCParams (zkey_utils.js): csHash, nContributions, then the records; parameters tag-prefixed, strictly increasing
-void parse_mpc(ZkeyIn& z) {
-  const uint8_t* p = z.s[10].p;
-  const uint64_t len = z.s[10].len;
-  if (len < 68) throw ApiError(NZCP_E_FORMAT, "zkey: section 10 is truncated");
-  const uint32_t n = rd32u(p + 64);
-  uint64_t pos = 68;
+// readMPCParams (zkey_utils.js) / readContributions (powersoftau_utils.js): `head` bytes (the zkey's csHash), u32
+// nContributions, then the records: rec_fixed bytes whose last u32 is paramLength, then the parameters, tag-prefixed and
+// strictly increasing.  `what` names the section in the messages.
+void parse_records(const uint8_t* p, uint64_t len, uint64_t head, size_t rec_fixed, const std::string& what,
+                   std::vector<const uint8_t*>& recs, std::vector<size_t>& rec_len) {
+  if (len < head + 4) throw ApiError(NZCP_E_FORMAT, what + " is truncated");
+  const uint32_t n = rd32u(p + head);
+  uint64_t pos = head + 4;
   for (uint32_t c = 0; c < n; c++) {
-    if (len - pos < kRecFixed) throw ApiError(NZCP_E_FORMAT, "zkey: section 10 is truncated");
+    if (len - pos < rec_fixed) throw ApiError(NZCP_E_FORMAT, what + " is truncated");
     const uint64_t start = pos;
-    const uint32_t plen = rd32u(p + pos + kRecFixed - 4);
-    pos += kRecFixed;
+    const uint32_t plen = rd32u(p + pos + rec_fixed - 4);
+    pos += rec_fixed;
     const uint64_t end = pos + plen;
     int last = 0;
     while (pos < end) {
       auto need = [&](uint64_t k) {
-        if (pos + k > len) throw ApiError(NZCP_E_FORMAT, "zkey: section 10 is truncated");
+        if (pos + k > len) throw ApiError(NZCP_E_FORMAT, what + " is truncated");
       };
       need(1);
       const int tag = p[pos++];
@@ -385,11 +473,13 @@ void parse_mpc(ZkeyIn& z) {
       }
     }
     if (pos != end) throw ApiError(NZCP_E_FORMAT, "Parametes do not match");   // snarkjs's spelling
-    z.recs.push_back(p + start);
-    z.rec_len.push_back(end - start);
+    recs.push_back(p + start);
+    rec_len.push_back(end - start);
   }
-  if (pos != len) throw ApiError(NZCP_E_FORMAT, "zkey: section 10 has trailing bytes");
+  if (pos != len) throw ApiError(NZCP_E_FORMAT, what + " has trailing bytes");
 }
+
+void parse_mpc(ZkeyIn& z) { parse_records(z.s[10].p, z.s[10].len, 64, kRecFixed, "zkey: section 10", z.recs, z.rec_len); }
 
 // check_pts = false: the caller checks the points of sections 2, 8 and 9 itself.
 ZkeyIn parse_zkey_in(const uint8_t* b, size_t len, bool check_pts = true) {
@@ -435,6 +525,163 @@ struct Events {
   ~Events() {
     if (a) cudaEventDestroy(a);
     if (b) cudaEventDestroy(b);
+  }
+};
+
+// ------------------------------------------------------------------------------------------------ point encodings (device)
+HD uint32_t bswap32(uint32_t v) { return (v >> 24) | ((v >> 8) & 0xff00u) | ((v << 8) & 0xff0000u) | (v << 24); }
+HD void put_be(const Fq& a, uint32_t* w) {
+  const Fq p = fp_from_mont(a);
+  for (int j = 0; j < 8; j++) w[j] = bswap32(p.v[7 - j]);
+}
+HD void put_be(const Fq2& a, uint32_t* w) {   // c1 first
+  put_be(a.c1, w);
+  put_be(a.c0, w + 8);
+}
+
+// wasmcurves isNegative / F2 sign: the plain value is > (q-1)/2 = q >> 1; for Fq2 c1 decides, c0 when c1 = 0.
+HD bool y_negative(const Fq& a) {
+  const Fq p = fp_from_mont(a);
+  for (int i = 7; i >= 0; i--) {
+    const uint32_t h = (FqParams::mod(i) >> 1) | (i < 7 ? FqParams::mod(i + 1) << 31 : 0);
+    if (p.v[i] != h) return p.v[i] > h;
+  }
+  return false;
+}
+HD bool y_negative(const Fq2& a) { return a.c1.is_zero() ? y_negative(a.c0) : y_negative(a.c1); }
+
+// U(P) as little-endian words: big-endian plain coordinates; infinity = 0x40 then zeros.
+template <class F>
+HD void u_encode(const Affine<F>& a, uint32_t* w) {
+  constexpr int n = sizeof(Affine<F>) / 4;
+  if (a.is_inf()) {
+    for (int i = 0; i < n; i++) w[i] = 0;
+    w[0] = 0x40;
+    return;
+  }
+  put_be(a.x, w);
+  put_be(a.y, w + n / 2);
+}
+
+// C(P), wasmcurves LEMtoC: big-endian plain x, 0x80 ORed into byte 0 when y is negative; infinity = 0x40 then zeros.
+template <class F>
+HD void c_encode(const Affine<F>& a, uint32_t* w) {
+  constexpr int n = sizeof(Affine<F>) / 8;
+  if (a.is_inf()) {
+    for (int i = 0; i < n; i++) w[i] = 0;
+    w[0] = 0x40;
+    return;
+  }
+  put_be(a.x, w);
+  if (y_negative(a.y)) w[0] |= 0x80;   // byte 0 is the low byte of the first little-endian word
+}
+
+template <class F>
+__global__ void __launch_bounds__(128) u_encode_kernel(const Affine<F>* __restrict__ in, uint32_t* __restrict__ out, uint64_t n) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) u_encode(in[i], out + i * (sizeof(Affine<F>) / 4));
+}
+
+template <class F>
+__global__ void __launch_bounds__(128) c_encode_kernel(const Affine<F>* __restrict__ in, uint32_t* __restrict__ out, uint64_t n) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) c_encode(in[i], out + i * (sizeof(Affine<F>) / 8));
+}
+
+// ------------------------------------------------------------------------------------------------ chunked point hashing
+enum class Enc { U, C };   // uncompressed (hashPubKey, the circuit hash, nextChallenge) or compressed (the response hash)
+
+constexpr uint64_t kHashChunk = 1u << 16;     // points per conversion chunk
+
+// BLAKE2b-512 over a stream of bytes and encoded points.  Device-resident points are encoded in chunks, so the host BLAKE2b
+// of chunk j (one sequential stream) overlaps the conversion and copy of chunk j + 1.  on_host: the same encoders run on
+// the CPU (test hooks).
+struct Hasher {
+  Blake2b512 h;
+  bool host;
+  Enc enc;
+  float kernel_ms = 0, blake_ms = 0;
+  std::unique_ptr<DevMem> d_enc[2];
+  uint8_t* h_enc[2] = {nullptr, nullptr};
+  cudaEvent_t ev[6] = {};   // per buffer: kernel start, kernel end, copy done
+
+  explicit Hasher(bool on_host, Enc e = Enc::U) : host(on_host), enc(e) {
+    if (host) return;
+    for (int b = 0; b < 2; b++) {
+      d_enc[b].reset(new DevMem(kHashChunk * 128));
+      NZCP_CUDA(cudaMallocHost((void**)&h_enc[b], kHashChunk * 128));
+    }
+    for (auto& e : ev) NZCP_CUDA(cudaEventCreate(&e));
+  }
+  ~Hasher() {
+    for (auto p : h_enc) if (p) cudaFreeHost(p);
+    for (auto e : ev) if (e) cudaEventDestroy(e);
+  }
+  Hasher(const Hasher&) = delete;
+  Hasher& operator=(const Hasher&) = delete;
+  template <class F>
+  static constexpr size_t enc_bytes(Enc e) { return e == Enc::U ? sizeof(Affine<F>) : sizeof(Affine<F>) / 2; }
+  void update(const void* p, size_t n) {
+    const auto t0 = std::chrono::steady_clock::now();
+    h.update(p, n);
+    blake_ms += std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  }
+  void u32be(uint32_t v) {
+    const uint8_t b[4] = {(uint8_t)(v >> 24), (uint8_t)(v >> 16), (uint8_t)(v >> 8), (uint8_t)v};
+    update(b, 4);
+  }
+  template <class F>
+  void points_host(const Affine<F>* p, uint64_t n) {
+    const size_t w = enc_bytes<F>(enc) / 4;
+    std::vector<uint32_t> buf(std::min<uint64_t>(n, 4096) * w);
+    for (uint64_t i = 0; i < n; i += 4096) {
+      const uint64_t m = std::min<uint64_t>(4096, n - i);
+      for (uint64_t j = 0; j < m; j++) {
+        Affine<F> a;
+        memcpy(&a, p + i + j, sizeof a);
+        if (enc == Enc::U) u_encode(a, buf.data() + j * w);
+        else c_encode(a, buf.data() + j * w);
+      }
+      update(buf.data(), m * w * 4);
+    }
+  }
+  // n device-resident points: chunk j's host hash overlaps the conversion and copy of chunk j + 1.
+  template <class F>
+  void points_device(const Affine<F>* d, uint64_t n) {
+    const size_t esz = enc_bytes<F>(enc);
+    const uint64_t nch = (n + kHashChunk - 1) / kHashChunk;
+    for (uint64_t j = 0; j <= nch; j++) {
+      if (j < nch) {
+        const int b = j & 1;
+        const uint64_t off = j * kHashChunk, m = std::min(kHashChunk, n - off);
+        uint32_t* dst = static_cast<uint32_t*>(d_enc[b]->p);
+        NZCP_CUDA(cudaEventRecord(ev[3 * b], 0));
+        if (enc == Enc::U) u_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, dst, m);
+        else c_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, dst, m);
+        NZCP_LAUNCH_CHECK();
+        NZCP_CUDA(cudaEventRecord(ev[3 * b + 1], 0));
+        NZCP_CUDA(cudaMemcpyAsync(h_enc[b], d_enc[b]->p, m * esz, cudaMemcpyDeviceToHost, 0));
+        NZCP_CUDA(cudaEventRecord(ev[3 * b + 2], 0));
+      }
+      if (j > 0) {
+        const int b = (j - 1) & 1;
+        const uint64_t m = std::min(kHashChunk, n - (j - 1) * kHashChunk);
+        NZCP_CUDA(cudaEventSynchronize(ev[3 * b + 2]));
+        float ms = 0;
+        NZCP_CUDA(cudaEventElapsedTime(&ms, ev[3 * b], ev[3 * b + 1]));
+        kernel_ms += ms;
+        update(h_enc[b], m * esz);
+      }
+    }
+  }
+  // n points in host memory
+  template <class F>
+  void section(const uint8_t* p, uint64_t n) {
+    const Affine<F>* a = reinterpret_cast<const Affine<F>*>(p);
+    if (host || n == 0) return points_host(a, n);
+    DevMem d(n * sizeof(Affine<F>));
+    NZCP_CUDA(cudaMemcpy(d.p, p, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
+    points_device(static_cast<const Affine<F>*>(d.p), n);
   }
 };
 

@@ -43,9 +43,6 @@
 // and H combinations are variable-base MSMs (msm.cu, table-free), the H scalars pass through the Fr NTT on the device.
 #include <sys/random.h>
 
-#include <chrono>
-#include <memory>
-
 #include "mpc.cuh"
 
 namespace nzcp {
@@ -60,39 +57,10 @@ HD G1Affine h_diff_point(const G1Affine& hi, const G1Affine& lo) {
   return to_affine_fast(acc);
 }
 
-HD uint32_t bswap32(uint32_t v) { return (v >> 24) | ((v >> 8) & 0xff00u) | ((v << 8) & 0xff0000u) | (v << 24); }
-HD void put_be(const Fq& a, uint32_t* w) {
-  const Fq p = fp_from_mont(a);
-  for (int j = 0; j < 8; j++) w[j] = bswap32(p.v[7 - j]);
-}
-HD void put_be(const Fq2& a, uint32_t* w) {   // c1 first
-  put_be(a.c1, w);
-  put_be(a.c0, w + 8);
-}
-
-// U(P) as little-endian words: big-endian plain coordinates; infinity = 0x40 then zeros.
-template <class F>
-HD void u_encode(const Affine<F>& a, uint32_t* w) {
-  constexpr int n = sizeof(Affine<F>) / 4;
-  if (a.is_inf()) {
-    for (int i = 0; i < n; i++) w[i] = 0;
-    w[0] = 0x40;
-    return;
-  }
-  put_be(a.x, w);
-  put_be(a.y, w + n / 2);
-}
-
 __global__ void __launch_bounds__(128) h_diff_kernel(const G1Affine* __restrict__ tau, uint64_t N, G1Affine* __restrict__ out,
                                                      uint64_t n) {
   const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = h_diff_point(tau[i + N], tau[i]);
-}
-
-template <class F>
-__global__ void __launch_bounds__(128) u_encode_kernel(const Affine<F>* __restrict__ in, uint32_t* __restrict__ out, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) u_encode(in[i], out + i * (sizeof(Affine<F>) / 4));
 }
 
 // r[m] <- -2 w^m r[m]: plain r, Montgomery w and -2, plain result.
@@ -109,7 +77,6 @@ __global__ void __launch_bounds__(256) h_scalar_kernel(Fr* __restrict__ r, uint6
 
 namespace {
 
-constexpr uint64_t kHashChunk = 1u << 16;     // points per conversion chunk
 constexpr uint64_t kHashHChunk = 1u << 14;    // hashHPoints CHUNK_SIZE
 
 // Points hashHPoints passes to the hasher for a domain of N (see the header of this file).
@@ -151,87 +118,6 @@ void check_init_sections(const ZkeyIn& z) {
 }
 
 // ------------------------------------------------------------------------------------------------ circuit hash
-struct Hasher {
-  Blake2b512 h;
-  bool host;
-  float kernel_ms = 0, blake_ms = 0;
-  std::unique_ptr<DevMem> d_enc[2];
-  uint8_t* h_enc[2] = {nullptr, nullptr};
-  cudaEvent_t ev[6] = {};   // per buffer: kernel start, kernel end, copy done
-
-  explicit Hasher(bool on_host) : host(on_host) {
-    if (host) return;
-    for (int b = 0; b < 2; b++) {
-      d_enc[b].reset(new DevMem(kHashChunk * 128));
-      NZCP_CUDA(cudaMallocHost((void**)&h_enc[b], kHashChunk * 128));
-    }
-    for (auto& e : ev) NZCP_CUDA(cudaEventCreate(&e));
-  }
-  ~Hasher() {
-    for (auto p : h_enc) if (p) cudaFreeHost(p);
-    for (auto e : ev) if (e) cudaEventDestroy(e);
-  }
-  void update(const void* p, size_t n) {
-    const auto t0 = std::chrono::steady_clock::now();
-    h.update(p, n);
-    blake_ms += std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  }
-  void u32be(uint32_t v) {
-    const uint8_t b[4] = {(uint8_t)(v >> 24), (uint8_t)(v >> 16), (uint8_t)(v >> 8), (uint8_t)v};
-    update(b, 4);
-  }
-  template <class F>
-  void points_host(const Affine<F>* p, uint64_t n) {
-    constexpr size_t w = sizeof(Affine<F>) / 4;
-    std::vector<uint32_t> buf(std::min<uint64_t>(n, 4096) * w);
-    for (uint64_t i = 0; i < n; i += 4096) {
-      const uint64_t m = std::min<uint64_t>(4096, n - i);
-      for (uint64_t j = 0; j < m; j++) {
-        Affine<F> a;
-        memcpy(&a, p + i + j, sizeof a);
-        u_encode(a, buf.data() + j * w);
-      }
-      update(buf.data(), m * w * 4);
-    }
-  }
-  // n device-resident points: chunk j's host hash overlaps the conversion and copy of chunk j + 1.
-  template <class F>
-  void points_device(const Affine<F>* d, uint64_t n) {
-    const size_t psz = sizeof(Affine<F>);
-    const uint64_t nch = (n + kHashChunk - 1) / kHashChunk;
-    for (uint64_t j = 0; j <= nch; j++) {
-      if (j < nch) {
-        const int b = j & 1;
-        const uint64_t off = j * kHashChunk, m = std::min(kHashChunk, n - off);
-        NZCP_CUDA(cudaEventRecord(ev[3 * b], 0));
-        u_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, static_cast<uint32_t*>(d_enc[b]->p), m);
-        NZCP_LAUNCH_CHECK();
-        NZCP_CUDA(cudaEventRecord(ev[3 * b + 1], 0));
-        NZCP_CUDA(cudaMemcpyAsync(h_enc[b], d_enc[b]->p, m * psz, cudaMemcpyDeviceToHost, 0));
-        NZCP_CUDA(cudaEventRecord(ev[3 * b + 2], 0));
-      }
-      if (j > 0) {
-        const int b = (j - 1) & 1;
-        const uint64_t m = std::min(kHashChunk, n - (j - 1) * kHashChunk);
-        NZCP_CUDA(cudaEventSynchronize(ev[3 * b + 2]));
-        float ms = 0;
-        NZCP_CUDA(cudaEventElapsedTime(&ms, ev[3 * b], ev[3 * b + 1]));
-        kernel_ms += ms;
-        update(h_enc[b], m * psz);
-      }
-    }
-  }
-  // n points in host memory
-  template <class F>
-  void section(const uint8_t* p, uint64_t n) {
-    const Affine<F>* a = reinterpret_cast<const Affine<F>*>(p);
-    if (host || n == 0) return points_host(a, n);
-    DevMem d(n * sizeof(Affine<F>));
-    NZCP_CUDA(cudaMemcpy(d.p, p, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-    points_device(static_cast<const Affine<F>*>(d.p), n);
-  }
-};
-
 struct HDiff {
   uint64_t n = 0;                   // h_hash_points(N)
   std::unique_ptr<DevMem> d;        // device run: the differences, resident for the H check

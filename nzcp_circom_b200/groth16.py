@@ -6,7 +6,8 @@ yarn.lock:987-999).  The reference's tests build the prover input at /root/refer
 test/nzcp.js:41-48; `publicSignals` below is that same slice, in the same order, as decimal strings.
 
 `zKey` groups newZKey / contribute / beacon / verifyFromR1cs / verifyFromInit / exportVerificationKey the way snarkjs's
-main.js does (snarkjs.zKey.newZKey, ...); `powersOfTau.preparePhase2` is snarkjs.powersOfTau.preparePhase2.
+main.js does (snarkjs.zKey.newZKey, ...); `powersOfTau` groups newAccumulator / contribute / beacon / preparePhase2
+(snarkjs.powersOfTau.*).
 
 Same names, argument meaning and error text as snarkjs:
   prove(zkeyFileName, witnessFileName, logger=None)   file args: path | bytes-like | {"type": "mem", "data": ...}
@@ -318,6 +319,83 @@ def preparePhase2(oldPtauFilename, newPTauFilename=None, logger=None, *, device=
     return data
 
 
+def newAccumulator(curve, power, fileName=None, logger=None):
+    """snarkjs powersOfTau.newAccumulator(curve, power, fileName): a fresh phase-1 file of 2^power (1..28) on the host.
+    `curve`: "bn128" / "bn254" or None (bn128).  `fileName`: a path to write, a {"type": "mem"} object that receives
+    `.data`, or None.  Returns the 64-byte first challenge hash, as snarkjs does."""
+    if curve is not None and str(curve).lower() not in ("bn128", "bn254"):
+        raise NzcpError(_lib.NZCP_E_CURVE, "Curve not supported: %s" % curve)
+    data, h = api.ptau_new(power)
+    if logger:
+        logger.debug(_format_hash(hashlib.blake2b(digest_size=64).digest(), "Blank Contribution Hash:"))
+        logger.info(_format_hash(h, "First Contribution Hash:"))
+    _write_out(fileName, data)
+    return h
+
+
+def _section_ids(buf):
+    mv = memoryview(buf).cast("B")
+    pos, ids = 12, []
+    for _ in range(struct.unpack_from("<I", mv, 8)[0] if len(mv) >= 12 else 0):
+        if pos + 12 > len(mv):
+            break
+        sid, ln = struct.unpack_from("<IQ", mv, pos)
+        ids.append(sid)
+        pos += 12 + ln
+    return ids
+
+
+def _ptau_step(old, new, logger, run, params_len):
+    """Shared tail of powersOfTau.contribute / beacon: the phase-2 warning, the call, snarkjs's log lines, the output."""
+    pb = api._as_bytes_like(old)
+    if logger and 12 in _section_ids(pb):
+        logger.warn("WARNING: Contributing into a file that has phase2 calculated. You will have to prepare phase2 again.")
+    timings = {} if logger else None
+    data, h = run(pb, timings)
+    if logger:
+        end = len(data) - params_len - 8     # the new record is last: ... nextChallenge, type, paramLength, parameters
+        for k, v in timings.items():
+            logger.debug("%s: %.3f ms" % (k if isinstance(k, str) else "section %d" % k, v))
+        logger.info(_format_hash(h, "Contribution Response Hash imported: "))
+        logger.info(_format_hash(bytes(data[end - 64:end]), "Next Challenge Hash: "))
+    _write_out(new, data)
+    return h
+
+
+def ptauContribute(oldPtauFilename, newPTauFilename, name, entropy, logger=None, *, seed=None, device=0):
+    """snarkjs powersOfTau.contribute(oldPtauFilename, newPTauFilename, name, entropy): one phase-1 contribution; sections
+    2-6 are multiplied on the GPU.  Empty entropy means OS randomness alone (snarkjs would prompt for it).
+    `newPTauFilename`: a path to write, a {"type": "mem"} object that receives `.data`, or None.  Returns the 64-byte
+    response hash.  `seed` (32 bytes) replaces the randomness: for tests only."""
+    nb = api._utf8(name or None)
+    return _ptau_step(oldPtauFilename, newPTauFilename, logger,
+                      lambda pb, t: api.ptau_contribute(pb, name=name or None, entropy=entropy or None, seed=seed,
+                                                        device=device, timings=t),
+                      2 + len(nb) if nb else 0)
+
+
+def _beacon_hash(beaconHashStr):
+    try:
+        hb = bytes.fromhex(beaconHashStr)
+    except (TypeError, ValueError):
+        hb = b""
+    if not hb or len(hb) * 2 != len(beaconHashStr):
+        raise NzcpError(_lib.NZCP_E_ARG, "Invalid Beacon Hash. (It must be a valid hexadecimal sequence)")
+    return hb
+
+
+def ptauBeacon(oldPtauFilename, newPTauFilename, name, beaconHashStr, numIterationsExp, logger=None, *, device=0):
+    """snarkjs powersOfTau.beacon(oldPtauFilename, newPTauFilename, name, beaconHashStr, numIterationsExp): the final,
+    publicly reproducible phase-1 contribution, its key derived from the hex string beaconHashStr hashed
+    2^numIterationsExp times.  Output and return value as ptauContribute."""
+    hb = _beacon_hash(beaconHashStr)
+    nb = api._utf8(name or None)
+    return _ptau_step(oldPtauFilename, newPTauFilename, logger,
+                      lambda pb, t: api.ptau_beacon(pb, hb, int(numIterationsExp), name=name or None, device=device,
+                                                    timings=t),
+                      (2 + len(nb) if nb else 0) + 4 + len(hb))
+
+
 def contribute(zkeyNameOld, zkeyNameNew, name, entropy, logger=None, *, seed=None, device=0):
     """snarkjs zKey.contribute(zkeyNameOld, zkeyNameNew, name, entropy): one phase-2 contribution to delta; sections 8
     and 9 are rescaled on the GPU.  Empty entropy means OS randomness alone (snarkjs would prompt for it).
@@ -335,12 +413,7 @@ def beacon(zkeyNameOld, zkeyNameNew, name, beaconHashStr, numIterationsExp, logg
     """snarkjs zKey.beacon(zkeyNameOld, zkeyNameNew, name, beaconHashStr, numIterationsExp): the final, publicly
     reproducible contribution, its key derived from the hex string beaconHashStr hashed 2^numIterationsExp times.
     Output and return value as contribute."""
-    try:
-        hb = bytes.fromhex(beaconHashStr)
-    except (TypeError, ValueError):
-        hb = b""
-    if not hb or len(hb) * 2 != len(beaconHashStr):
-        raise NzcpError(_lib.NZCP_E_ARG, "Invalid Beacon Hash. (It must be a valid hexadecimal sequence)")
+    hb = _beacon_hash(beaconHashStr)
     timings = {} if logger else None
     data, h = api.zkey_beacon(zkeyNameOld, hb, int(numIterationsExp), name=name or None, device=device, timings=timings)
     _log_sections(logger, timings)
@@ -388,7 +461,10 @@ def verifyFromInit(initFileName, pTauFileName, zkeyFileName, logger=None, *, see
 
 
 class powersOfTau:
-    """snarkjs.powersOfTau namespace: the one entry this library computes."""
+    """snarkjs.powersOfTau namespace: the entries this library computes."""
+    newAccumulator = staticmethod(newAccumulator)
+    contribute = staticmethod(ptauContribute)
+    beacon = staticmethod(ptauBeacon)
     preparePhase2 = staticmethod(preparePhase2)
 
 
