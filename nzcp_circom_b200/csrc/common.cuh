@@ -40,6 +40,10 @@ extern thread_local std::atomic<uint64_t>* t_launch_sink;
 
 static inline unsigned div_up(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
 
+G1Affine g1_generator();   // synth.cu: the BN254 generators, Montgomery affine
+G2Affine g2_generator();
+Fr host_fr_root(int k);    // ntt.cu: ffjavascript's Fr.w[k], Montgomery
+
 // ---------------------------------------------------------------------------------------------- NTT (ntt.cu)
 // Tables for one domain size n = 2^log_n (Montgomery-form Fr, device memory).
 struct NttDomain {

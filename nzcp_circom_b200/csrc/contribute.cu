@@ -45,7 +45,7 @@ __global__ void __launch_bounds__(128) zkey_scale_kernel(G1Affine* __restrict__ 
 namespace {
 
 size_t contribute_size(const ZkeyIn& z, size_t name_len, size_t beacon_len) {
-  size_t total = 12 + 10 * 12 + 4 + kHeaderLen;
+  size_t total = 12 + 10 * 12 + 4 + kZkeyHeaderLen;
   for (int id = 3; id <= 10; id++) total += z.s[id].len;
   return total + kRecFixed + params_len(name_len, beacon_len);
 }
@@ -84,7 +84,7 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
   const size_t total = contribute_size(z, a.name_len, beacon ? a.beacon_len : 0);
   if (cap < total) throw ApiError(NZCP_E_ARG, "output buffer too small");
   const bool host = device < 0;
-  if (host && z.n_l + z.n_h > kHostMaxPoints)
+  if (host && z.n_l() + z.domain_size > kHostMaxPoints)
     throw ApiError(NZCP_E_ARG, "zkey: the host run is limited to 4096 points in sections 8 and 9");
   if (!host) use_device(device);
 
@@ -117,8 +117,8 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
 
   G1Affine d1;
   G2Affine d2;
-  memcpy(&d1, z.s[2].p + kDelta1Off, 64);
-  memcpy(&d2, z.s[2].p + kDelta2Off, 128);
+  memcpy(&d1, z.s[2].p + kZkeyDelta1Off, 64);
+  memcpy(&d2, z.s[2].p + kZkeyDelta2Off, 128);
   d1 = mul_plain(d1, k.v);
   d2 = mul_plain(d2, k.v);
 
@@ -147,19 +147,19 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
   w.u32(10);
   w.section(1, 4);
   w.u32(1);
-  w.section(2, kHeaderLen);
-  uint8_t* hdr = w.reserve(kHeaderLen);
-  memcpy(hdr, z.s[2].p, kHeaderLen);
-  memcpy(hdr + kDelta1Off, &d1, 64);
-  memcpy(hdr + kDelta2Off, &d2, 128);
+  w.section(2, kZkeyHeaderLen);
+  uint8_t* hdr = w.reserve(kZkeyHeaderLen);
+  memcpy(hdr, z.s[2].p, kZkeyHeaderLen);
+  memcpy(hdr + kZkeyDelta1Off, &d1, 64);
+  memcpy(hdr + kZkeyDelta2Off, &d2, 128);
   for (int id = 3; id <= 7; id++) {
     w.section(id, z.s[id].len);
     w.raw(z.s[id].p, z.s[id].len);
   }
   std::unique_ptr<DevMem> d_buf;
-  if (!host) d_buf.reset(new DevMem(std::max(z.n_l, z.n_h) * 64));
+  if (!host) d_buf.reset(new DevMem(std::max<uint64_t>(z.n_l(), z.domain_size) * 64));
   for (int id = 8; id <= 9; id++) {
-    const uint64_t n = id == 8 ? z.n_l : z.n_h;
+    const uint64_t n = id == 8 ? z.n_l() : z.domain_size;
     w.section(id, n * 64);
     uint8_t* dst = w.reserve(n * 64);
     float ms = 0;

@@ -1,7 +1,7 @@
 // Code shared by the ceremony entry points (contribute.cu `zkey contribute` / `zkey beacon`, verify.cu `zkey verify`,
 // setup.cu `zkey new`, ptau_contribute.cu `powersoftau new` / `contribute` / `beacon`): BLAKE2b-512 and SHA-256,
 // ffjavascript's ChaCha, F/G.fromRng, the uncompressed and compressed point encodings (host and device) with the chunked
-// point hasher, the .zkey / contribution-record reader, and the .r1cs / .ptau readers and the key writer of setup.cu.
+// point hasher, and the contribution records with the .zkey input of `zkey contribute` / `zkey verify`.
 #pragma once
 #include <sys/random.h>
 
@@ -11,31 +11,6 @@
 #include "binfile.cuh"
 
 namespace nzcp {
-
-G1Affine g1_generator();  // synth.cu
-G2Affine g2_generator();
-
-// ------------------------------------------------------------------------------------------------ setup.cu
-struct R1cs {
-  uint32_t n_wires = 0, n_pub_out = 0, n_pub_in = 0, n_prv_in = 0, n_constraints = 0, n_public = 0;
-  const uint8_t* cons = nullptr;
-  uint64_t cons_len = 0;
-  uint64_t n_terms[3] = {0, 0, 0};   // A, B, C terms in total
-};
-
-struct Ptau {
-  uint32_t power = 0;
-  Sect s[16];
-};
-
-R1cs parse_r1cs(const uint8_t* b, size_t len);
-Ptau parse_ptau(const uint8_t* b, size_t len);
-uint32_t circuit_power(const R1cs& r);
-size_t zkey_new_size(const R1cs& r, uint32_t cir_power);
-// snarkjs `zkey new` into out[0 .. cap); section 10 holds a zero circuit hash.
-void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b, size_t ptau_len, int device, uint8_t* out,
-                   size_t cap, size_t* written);
-
 namespace {
 
 // ------------------------------------------------------------------------------------------------ hashes (host)
@@ -426,13 +401,9 @@ void hash_pub_key(Blake2b512& h, const uint8_t* rec) {
 }
 
 // ------------------------------------------------------------------------------------------------ input
-constexpr size_t kHeaderLen = 4 + 32 + 4 + 32 + 12 + 64 + 64 + 128 + 128 + 64 + 128;   // 660
-constexpr size_t kDelta1Off = 468, kDelta2Off = 532;
 constexpr uint64_t kHostMaxPoints = 1u << 12;
 
-struct ZkeyIn {
-  Sect s[11];
-  uint64_t n_l = 0, n_h = 0;
+struct ZkeyIn : Zkey {
   std::vector<const uint8_t*> recs;   // section-10 records
   std::vector<size_t> rec_len;
 };
@@ -481,32 +452,23 @@ void parse_records(const uint8_t* p, uint64_t len, uint64_t head, size_t rec_fix
 
 void parse_mpc(ZkeyIn& z) { parse_records(z.s[10].p, z.s[10].len, 64, kRecFixed, "zkey: section 10", z.recs, z.rec_len); }
 
-// check_pts = false: the caller checks the points of sections 2, 8 and 9 itself.
+// The input of `zkey contribute` / `zkey verify`: read_zkey, then a header of exactly 660 bytes, sections 3-10, the sizes
+// of 8 and 9 and the records.  check_pts = false: the caller checks the points of sections 2, 8 and 9 itself.
 ZkeyIn parse_zkey_in(const uint8_t* b, size_t len, bool check_pts = true) {
-  ZkeyIn z;
-  parse_bin(b, len, "zkey", z.s, 10);
-  if (!z.s[1].p || z.s[1].len < 4) throw ApiError(NZCP_E_FORMAT, "zkey: missing header");
-  if (rd32u(z.s[1].p) != 1) throw ApiError(NZCP_E_NOT_GROTH16, "zkey file is not groth16");
-  for (int id = 2; id <= 10; id++)
-    if (!z.s[id].p) throw ApiError(NZCP_E_FORMAT, "Missing section " + std::to_string(id));
-  const uint8_t* h = z.s[2].p;
-  if (z.s[2].len != kHeaderLen) throw ApiError(NZCP_E_FORMAT, "zkey: header section 2 is not 660 bytes");
-  if (rd32u(h) != 32 || memcmp(h + 4, kQBytes, 32) != 0 || rd32u(h + 36) != 32 || memcmp(h + 40, kRBytes, 32) != 0)
-    throw ApiError(NZCP_E_CURVE, "zkey: curve is not bn128");
-  const uint32_t n_vars = rd32u(h + 72), n_public = rd32u(h + 76), domain = rd32u(h + 80);
-  if ((uint64_t)n_public + 1 > n_vars) throw ApiError(NZCP_E_FORMAT, "zkey: more public signals than variables");
-  z.n_l = (uint64_t)n_vars - n_public - 1;
-  z.n_h = domain;
-  if (z.s[8].len != z.n_l * 64) throw ApiError(NZCP_E_FORMAT, "zkey: section 8 size does not match nVars - nPublic - 1");
-  if (z.s[9].len != z.n_h * 64) throw ApiError(NZCP_E_FORMAT, "zkey: section 9 size does not match domainSize");
+  ZkeyIn z{read_zkey(b, len)};
+  if (z.s[2].len != kZkeyHeaderLen) throw ApiError(NZCP_E_FORMAT, "zkey: header section 2 is not 660 bytes");
+  need_sections(z.s, 3, 10);
+  if (z.s[8].len != z.n_l() * 64) throw ApiError(NZCP_E_FORMAT, "zkey: section 8 size does not match nVars - nPublic - 1");
+  if (z.s[9].len != (uint64_t)z.domain_size * 64)
+    throw ApiError(NZCP_E_FORMAT, "zkey: section 9 size does not match domainSize");
   parse_mpc(z);
   if (!check_pts) return z;
   const Fq b1 = curve_b(g1_generator());
   const Fq2 b2 = curve_b(g2_generator());
-  check_points<Fq>("zkey", h + kDelta1Off, 1, 2, b1);
-  check_points<Fq2>("zkey", h + kDelta2Off, 1, 2, b2);
-  check_points<Fq>("zkey", z.s[8].p, z.n_l, 8, b1);
-  check_points<Fq>("zkey", z.s[9].p, z.n_h, 9, b1);
+  check_points<Fq>("zkey", z.s[2].p + kZkeyDelta1Off, 1, 2, b1);
+  check_points<Fq2>("zkey", z.s[2].p + kZkeyDelta2Off, 1, 2, b2);
+  check_points<Fq>("zkey", z.s[8].p, z.n_l(), 8, b1);
+  check_points<Fq>("zkey", z.s[9].p, z.domain_size, 9, b1);
   return z;
 }
 

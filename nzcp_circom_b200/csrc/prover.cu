@@ -12,7 +12,7 @@
 #include <mutex>
 #include <thread>
 
-#include "api_util.cuh"
+#include "binfile.cuh"
 
 namespace nzcp {
 
@@ -31,45 +31,6 @@ std::atomic<int> g_tune_stage_threads{4};      // host threads sharing the copy 
 
 static thread_local std::string t_last_error;
 void set_last_error(const std::string& s) { t_last_error = s; }
-
-// ---------------------------------------------------------------------------------------------- container parsing
-struct Section {
-  const uint8_t* p = nullptr;
-  uint64_t len = 0;
-};
-
-static uint32_t rd32(const uint8_t* p) {
-  uint32_t v;
-  memcpy(&v, p, 4);
-  return v;
-}
-static uint64_t rd64(const uint8_t* p) {
-  uint64_t v;
-  memcpy(&v, p, 8);
-  return v;
-}
-
-// binfileutils readBinFile: magic, version, nSections, then (u32 id, u64 len, payload)*
-static void parse_container(const uint8_t* b, size_t len, const char magic[4], uint32_t max_version, Section* secs,
-                            int max_id) {
-  if (len < 12 || memcmp(b, magic, 4) != 0) throw ApiError(NZCP_E_FORMAT, std::string(magic, 4) + " file: Invalid File format");
-  uint32_t version = rd32(b + 4);
-  if (version > max_version) throw ApiError(NZCP_E_FORMAT, "Version not supported");
-  uint32_t nsec = rd32(b + 8);
-  size_t pos = 12;
-  for (uint32_t i = 0; i < nsec; i++) {
-    if (pos + 12 > len) throw ApiError(NZCP_E_FORMAT, "truncated section table");
-    uint32_t id = rd32(b + pos);
-    uint64_t sl = rd64(b + pos + 4);
-    pos += 12;
-    if (sl > len - pos) throw ApiError(NZCP_E_FORMAT, "section exceeds file size");
-    if (id <= (uint32_t)max_id && secs[id].p == nullptr) {   // unsigned compare: a section id >= 2^31 must not index backwards
-      secs[id].p = b + pos;
-      secs[id].len = sl;
-    }
-    pos += sl;
-  }
-}
 
 }  // namespace nzcp
 
@@ -140,50 +101,38 @@ static T* upload(const void* src, size_t bytes, size_t* total) {
 }
 
 static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
-  Section s[11];
-  parse_container(b, len, "zkey", 1, s, 10);
-  if (!s[1].p || s[1].len < 4) throw ApiError(NZCP_E_FORMAT, "zkey: missing section 1");
-  if (rd32(s[1].p) != 1) throw ApiError(NZCP_E_NOT_GROTH16, "zkey file is not groth16");
-  for (int id = 2; id <= 9; id++)
-    if (!s[id].p) throw ApiError(NZCP_E_FORMAT, "zkey: missing section " + std::to_string(id));
-  // section 2: header (zkey_utils.js readHeaderGroth16)
-  const uint8_t* h = s[2].p;
-  const size_t hdr_len = 4 + 32 + 4 + 32 + 12 + 64 + 64 + 128 + 128 + 64 + 128;
-  if (s[2].len < hdr_len) throw ApiError(NZCP_E_FORMAT, "zkey: short header");
-  if (rd32(h) != 32 || rd32(h + 36) != 32) throw ApiError(NZCP_E_CURVE, "zkey: field size is not 32 bytes (curve is not bn128)");
-  if (memcmp(h + 4, kQBytes, 32) != 0 || memcmp(h + 40, kRBytes, 32) != 0)
-    throw ApiError(NZCP_E_CURVE, "zkey: curve is not bn128");
+  const Zkey z = read_zkey(b, len);
+  const Sect* s = z.s;
+  need_sections(s, 3, 9);
   std::unique_ptr<nzcp_zkey, void (*)(nzcp_zkey*)> zk(new nzcp_zkey(), zkey_release);
   zk->device = device;
-  zk->n_vars = rd32(h + 72);
-  zk->n_public = rd32(h + 76);
-  zk->domain_size = rd32(h + 80);
-  uint32_t n = zk->domain_size;
-  if (n < 2 || (n & (n - 1)) != 0) throw ApiError(NZCP_E_FORMAT, "zkey: domainSize is not a power of two >= 2");
-  if (zk->n_public + 1 > zk->n_vars) throw ApiError(NZCP_E_FORMAT, "zkey: nPublic + 1 > nVars");
-  while ((1u << zk->power) < n) zk->power++;
-  const uint8_t* pp = h + 84;
-  memcpy(&zk->alpha1, pp, 64); pp += 64;
-  memcpy(&zk->beta1, pp, 64); pp += 64;
-  memcpy(&zk->beta2, pp, 128); pp += 128;
-  memcpy(&zk->gamma2, pp, 128); pp += 128;
-  memcpy(&zk->delta1, pp, 64); pp += 64;
-  memcpy(&zk->delta2, pp, 128);
+  zk->n_vars = z.n_vars;
+  zk->n_public = z.n_public;
+  zk->domain_size = z.domain_size;
+  zk->power = zkey_domain_power(z);
+  const uint32_t n = zk->domain_size;
+  const uint8_t* h = s[2].p;
+  memcpy(&zk->alpha1, h + kZkeyAlpha1Off, 64);
+  memcpy(&zk->beta1, h + kZkeyBeta1Off, 64);
+  memcpy(&zk->beta2, h + kZkeyBeta2Off, 128);
+  memcpy(&zk->gamma2, h + kZkeyGamma2Off, 128);
+  memcpy(&zk->delta1, h + kZkeyDelta1Off, 64);
+  memcpy(&zk->delta2, h + kZkeyDelta2Off, 128);
   // section sizes
   const uint64_t m = zk->n_vars;
-  if (s[5].len != m * 64 || s[6].len != m * 64 || s[7].len != m * 128 || s[8].len != (m - zk->n_public - 1) * 64 ||
+  if (s[5].len != m * 64 || s[6].len != m * 64 || s[7].len != m * 128 || s[8].len != z.n_l() * 64 ||
       s[9].len != (uint64_t)n * 64)
     throw ApiError(NZCP_E_FORMAT, "zkey: point section size does not match header");
   // section 4: COO coefficients -> CSR (rows 0..n-1 = A, n..2n-1 = B)
   if (s[4].len < 4) throw ApiError(NZCP_E_FORMAT, "zkey: short coefficient section");
-  uint64_t nc = rd32(s[4].p);
+  uint64_t nc = rd32u(s[4].p);
   if (s[4].len != 4 + nc * 44) throw ApiError(NZCP_E_FORMAT, "zkey: coefficient section size mismatch");
   zk->n_coefs = nc;
   std::vector<uint32_t> row_ptr(2 * (size_t)n + 1, 0);
   const uint8_t* cp = s[4].p + 4;
   for (uint64_t i = 0; i < nc; i++) {
     const uint8_t* rec = cp + i * 44;
-    uint32_t mtx = rd32(rec), c = rd32(rec + 4), sg = rd32(rec + 8);
+    uint32_t mtx = rd32u(rec), c = rd32u(rec + 4), sg = rd32u(rec + 8);
     if (mtx > 1 || c >= n || sg >= zk->n_vars) throw ApiError(NZCP_E_FORMAT, "zkey: coefficient record out of range");
     row_ptr[(size_t)mtx * n + c + 1]++;
   }
@@ -193,7 +142,7 @@ static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
   std::vector<Fr> val(nc ? nc : 1);
   for (uint64_t i = 0; i < nc; i++) {
     const uint8_t* rec = cp + i * 44;
-    uint32_t mtx = rd32(rec), c = rd32(rec + 4), sg = rd32(rec + 8);
+    uint32_t mtx = rd32u(rec), c = rd32u(rec + 4), sg = rd32u(rec + 8);
     uint32_t pos = fill[(size_t)mtx * n + c]++;
     col[pos] = sg;
     memcpy(val[pos].v, rec + 12, 32);
@@ -229,7 +178,7 @@ static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
   // sections 5-9 -> window tables (one-time expansion; the raw section is only staged)
   zk->c_w = g_tune_c_w.load() > 0 ? g_tune_c_w.load() : msm_pick_window(m);
   zk->c_h = g_tune_c_h.load() > 0 ? g_tune_c_h.load() : msm_pick_window(n);
-  auto make_table = [&](MsmTable* t, const Section& sec, size_t count, size_t pad, bool g2, int c) {
+  auto make_table = [&](MsmTable* t, const Sect& sec, size_t count, size_t pad, bool g2, int c) {
     size_t dummy = 0;
     void* raw = upload<unsigned char>(sec.p, sec.len, &dummy);
     try {
@@ -245,7 +194,7 @@ static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
   make_table(&zk->tab_a, s[5], m, 0, false, zk->c_w);
   make_table(&zk->tab_b1, s[6], m, 0, false, zk->c_w);
   make_table(&zk->tab_b2, s[7], m, 0, true, zk->c_w);
-  make_table(&zk->tab_c, s[8], m - zk->n_public - 1, zk->n_public + 1, false, zk->c_w);
+  make_table(&zk->tab_c, s[8], z.n_l(), zk->n_public + 1, false, zk->c_w);
   make_table(&zk->tab_h, s[9], n, 0, false, zk->c_h);
   ntt_domain_create(&zk->dom, (int)zk->power, 0);
   tot += ((size_t)n / 2 * 2 + n) * sizeof(Fr);
@@ -605,13 +554,13 @@ int nzcp_prove(nzcp_prover* p, const uint8_t* wtns, size_t wtns_len, const uint8
                nzcp_proof* proof, nzcp_prove_debug* dbg) {
   return api_guard([&] {
     if (!p || !wtns) throw ApiError(NZCP_E_ARG, "null argument");
-    Section sec[3];
-    parse_container(wtns, wtns_len, "wtns", 2, sec, 2);
+    Sect sec[3];
+    parse_bin(wtns, wtns_len, "wtns", sec, 2, 2);
     if (!sec[1].p || !sec[2].p || sec[1].len < 8) throw ApiError(NZCP_E_FORMAT, "wtns: missing section");
-    uint32_t n8 = rd32(sec[1].p);
+    uint32_t n8 = rd32u(sec[1].p);
     if (n8 != 32 || sec[1].len != 4 + 32 + 4 || memcmp(sec[1].p + 4, kRBytes, 32) != 0)
       throw ApiError(NZCP_E_CURVE, "Curve of the witness does not match the curve of the proving key");
-    uint32_t nw = rd32(sec[1].p + 36);
+    uint32_t nw = rd32u(sec[1].p + 36);
     if (nw != p->zk->n_vars)
       throw ApiError(NZCP_E_WITNESS_LEN, "Invalid witness length. Circuit: " + std::to_string(p->zk->n_vars) +
                                              ", witness: " + std::to_string(nw));

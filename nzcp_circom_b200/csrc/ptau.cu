@@ -31,10 +31,6 @@
 
 namespace nzcp {
 
-G1Affine g1_generator();  // synth.cu
-G2Affine g2_generator();
-Fr host_fr_root(int k);   // ntt.cu
-
 // ------------------------------------------------------------------------------------------------ shared host/device code
 HD int ilog2_u64(uint64_t v) {   // v > 0
 #ifdef __CUDA_ARCH__
@@ -123,39 +119,15 @@ __global__ void __launch_bounds__(128) ptau_stage_kernel(Affine<F>* __restrict__
 // ------------------------------------------------------------------------------------------------ host side
 namespace {
 
-constexpr uint32_t kMaxPower = 27;
 constexpr uint32_t kHostMaxPower = 4;
 
-struct PtauIn {
-  uint32_t power = 0;
-  Sect s[16];
-};
-
 // Everything preparePhase2 needs from its input, validated before any device work.
-PtauIn parse_ptau_in(const uint8_t* b, size_t len) {
-  PtauIn p;
-  parse_bin(b, len, "ptau", p.s, 15);
-  if (!p.s[1].p || p.s[1].len < 4 + 32 + 8) throw ApiError(NZCP_E_FORMAT, "ptau: missing header");
-  if (rd32u(p.s[1].p) != 32 || memcmp(p.s[1].p + 4, kQBytes, 32) != 0) throw ApiError(NZCP_E_CURVE, "ptau: curve is not bn128");
-  p.power = rd32u(p.s[1].p + 36);
-  if (p.power == 28)
+Ptau parse_prepare_in(const uint8_t* b, size_t len) {
+  const Ptau p = read_ptau(b, len);
+  if (p.power == kPtauMaxPower)
     throw ApiError(NZCP_E_ARG, "ptau: power 28 is not supported: its top tauG1 level has 2^29 points, more than the 2^28 "
                                "roots of unity of Fr, and needs the coset branch of snarkjs's lagrangeEvaluations");
-  if (p.power < 1 || p.power > kMaxPower) throw ApiError(NZCP_E_FORMAT, "ptau: power out of range [1, 27]");
-  for (int id = 2; id <= 7; id++)
-    if (!p.s[id].p) throw ApiError(NZCP_E_FORMAT, "ptau: Missing section " + std::to_string(id));
-  const uint64_t n = (uint64_t)1 << p.power;
-  const uint64_t want[7] = {0, 0, (2 * n - 1) * 64, n * 128, n * 64, n * 64, 128};
-  for (int id = 2; id <= 6; id++)
-    if (p.s[id].len != want[id])
-      throw ApiError(NZCP_E_FORMAT, "ptau: section " + std::to_string(id) + " size does not match the header power");
-  const Fq b1 = curve_b(g1_generator());
-  const Fq2 b2 = curve_b(g2_generator());
-  check_points<Fq>("ptau", p.s[2].p, 2 * n - 1, 2, b1);
-  check_points<Fq2>("ptau", p.s[3].p, n, 3, b2);
-  check_points<Fq>("ptau", p.s[4].p, n, 4, b1);
-  check_points<Fq>("ptau", p.s[5].p, n, 5, b1);
-  check_points<Fq2>("ptau", p.s[6].p, 1, 6, b2);
+  check_ptau_sections(p);
   return p;
 }
 
@@ -175,8 +147,8 @@ void out_sects(uint32_t power, OutSect o[4]) {
 
 uint64_t level_points(uint32_t top) { return ((uint64_t)2 << top) - 1; }   // levels 0 .. top back to back
 
-size_t prepare_size(const PtauIn& p) {
-  size_t total = 12 + 11 * 12 + 44;
+size_t prepare_size(const Ptau& p) {
+  size_t total = 12 + 11 * 12 + kPtauHeaderLen;
   for (int id = 2; id <= 7; id++) total += p.s[id].len;
   OutSect o[4];
   out_sects(p.power, o);
@@ -248,7 +220,7 @@ void run_section_host(const uint8_t* src, uint64_t n_src, uint32_t top, const Fr
 
 // device < 0: the host hook.
 void prepare_impl(const uint8_t* b, size_t len, int device, uint8_t* out, size_t cap, size_t* written, float* section_ms) {
-  const PtauIn p = parse_ptau_in(b, len);
+  const Ptau p = parse_prepare_in(b, len);
   const size_t total = prepare_size(p);
   if (cap < total) throw ApiError(NZCP_E_ARG, "output buffer too small");
   const bool host = device < 0;
@@ -275,14 +247,7 @@ void prepare_impl(const uint8_t* b, size_t len, int device, uint8_t* out, size_t
   }
 
   Writer w(out, cap);
-  w.raw("ptau", 4);
-  w.u32(1);
-  w.u32(11);
-  w.section(1, 44);
-  w.u32(32);
-  w.raw(kQBytes, 32);
-  w.u32(p.power);
-  w.u32(p.power);                                           // ceremonyPower = power (writePTauHeader)
+  write_ptau_header(w, p.power, 11);
   for (int id = 2; id <= 7; id++) {
     w.section(id, p.s[id].len);
     w.raw(p.s[id].p, p.s[id].len);
@@ -318,7 +283,7 @@ extern "C" {
 int nzcp_ptau_prepare_size(const uint8_t* ptau, size_t len, size_t* out_size) {
   return api_guard([&] {
     if (!ptau || !out_size) throw ApiError(NZCP_E_ARG, "null argument");
-    *out_size = prepare_size(parse_ptau_in(ptau, len));
+    *out_size = prepare_size(parse_prepare_in(ptau, len));
   });
 }
 

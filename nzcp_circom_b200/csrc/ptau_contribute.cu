@@ -69,78 +69,41 @@ __global__ void __launch_bounds__(128) ptau_key_kernel(Affine<F>* __restrict__ x
 
 namespace {
 
-constexpr uint32_t kMaxPower = 28;
 constexpr uint32_t kHostMaxPower = 4;
-constexpr size_t kHdrLen = 4 + 32 + 4 + 4;
 constexpr size_t kPubKeyLen = 6 * 64 + 3 * 128;                               // 768
 constexpr size_t kPartialLen = 216;
 // pubkey tauG1 tauG2 alphaG1 betaG1 betaG2 partialHash nextChallenge type paramLength
 constexpr size_t kPtauRecFixed = kPubKeyLen + 3 * 64 + 2 * 128 + kPartialLen + 64 + 4 + 4;   // 1504
 
-uint64_t sect_points(uint32_t power, int id) {
-  const uint64_t n = (uint64_t)1 << power;
-  return id == 2 ? 2 * n - 1 : id == 6 ? 1 : n;
-}
-bool sect_g2(int id) { return id == 3 || id == 6; }
-size_t sect_bytes(uint32_t power, int id) { return sect_points(power, id) * (sect_g2(id) ? 128 : 64); }
-
 size_t new_size(uint32_t power) {
-  size_t total = 12 + 7 * 12 + kHdrLen + 4;
+  size_t total = 12 + 7 * 12 + kPtauHeaderLen + 4;
   for (int id = 2; id <= 6; id++) total += sect_bytes(power, id);
   return total;
 }
 
-void check_power(uint32_t power, int code) {
-  if (power < 1 || power > kMaxPower) throw ApiError(code, "ptau: power out of range [1, 28]");
+void check_power(uint32_t power) {
+  if (power < 1 || power > kPtauMaxPower) throw ApiError(NZCP_E_ARG, "ptau: power out of range [1, 28]");
 }
 
-struct PtauIn {
-  uint32_t power = 0;
-  Sect s[16];
+struct ContribIn : Ptau {
   std::vector<const uint8_t*> recs;   // section-7 records
   std::vector<size_t> rec_len;
 };
 
 // Everything contribute / beacon need from their input, validated before any device work.
-PtauIn parse_contrib_in(const uint8_t* b, size_t len) {
-  PtauIn p;
-  parse_bin(b, len, "ptau", p.s, 15);
-  if (!p.s[1].p || p.s[1].len < kHdrLen) throw ApiError(NZCP_E_FORMAT, "ptau: missing header");
-  if (rd32u(p.s[1].p) != 32 || memcmp(p.s[1].p + 4, kQBytes, 32) != 0) throw ApiError(NZCP_E_CURVE, "ptau: curve is not bn128");
-  p.power = rd32u(p.s[1].p + 36);
-  check_power(p.power, NZCP_E_FORMAT);
-  for (int id = 2; id <= 7; id++)
-    if (!p.s[id].p) throw ApiError(NZCP_E_FORMAT, "ptau: Missing section " + std::to_string(id));
-  for (int id = 2; id <= 6; id++)
-    if (p.s[id].len != sect_bytes(p.power, id))
-      throw ApiError(NZCP_E_FORMAT, "ptau: section " + std::to_string(id) + " size does not match the header power");
-  if (rd32u(p.s[1].p + 40) != p.power)
+ContribIn parse_contrib_in(const uint8_t* b, size_t len) {
+  ContribIn p{read_ptau(b, len)};
+  check_ptau_sections(p);
+  if (p.ceremony_power != p.power)
     throw ApiError(NZCP_E_ARG, "This file has been reduced. You cannot contribute into a reduced file.");
   parse_records(p.s[7].p, p.s[7].len, 0, kPtauRecFixed, "ptau: section 7", p.recs, p.rec_len);
-  const Fq b1 = curve_b(g1_generator());
-  const Fq2 b2 = curve_b(g2_generator());
-  for (int id = 2; id <= 6; id++) {
-    if (sect_g2(id)) check_points<Fq2>("ptau", p.s[id].p, sect_points(p.power, id), id, b2);
-    else check_points<Fq>("ptau", p.s[id].p, sect_points(p.power, id), id, b1);
-  }
   return p;
 }
 
-size_t contribute_size(const PtauIn& p, size_t name_len, size_t beacon_len) {
-  size_t total = 12 + 7 * 12 + kHdrLen;
+size_t contribute_size(const ContribIn& p, size_t name_len, size_t beacon_len) {
+  size_t total = 12 + 7 * 12 + kPtauHeaderLen;
   for (int id = 2; id <= 7; id++) total += p.s[id].len;
   return total + kPtauRecFixed + params_len(name_len, beacon_len);
-}
-
-void write_header(Writer& w, uint32_t power) {   // writePTauHeader
-  w.raw("ptau", 4);
-  w.u32(1);
-  w.u32(7);
-  w.section(1, kHdrLen);
-  w.u32(32);
-  w.raw(kQBytes, 32);
-  w.u32(power);
-  w.u32(power);
 }
 
 // calculateFirstChallengeHash; blake_ms += the host time.
@@ -248,7 +211,7 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
                      uint8_t* hash_out, float* ms_out) {
   check_contrib_args("ptau", a);
   const bool beacon = a.beacon != nullptr;
-  const PtauIn p = parse_contrib_in(b, len);
+  const ContribIn p = parse_contrib_in(b, len);
   const size_t total = contribute_size(p, a.name_len, beacon ? a.beacon_len : 0);
   if (cap < total) throw ApiError(NZCP_E_ARG, "output buffer too small");
   const bool host = device < 0;
@@ -270,7 +233,7 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
 
   // ---- sections 2-6 and the response hash
   Writer w(out, cap);
-  write_header(w, p.power);
+  write_ptau_header(w, p.power, 7);
   Hasher resp(host, Enc::C);
   resp.update(challenge, 64);
   std::unique_ptr<DevMem> d_buf;
@@ -355,7 +318,7 @@ extern "C" {
 int nzcp_ptau_new_size(uint32_t power, size_t* out_size) {
   return api_guard([&] {
     if (!out_size) throw ApiError(NZCP_E_ARG, "null argument");
-    check_power(power, NZCP_E_ARG);
+    check_power(power);
     *out_size = new_size(power);
   });
 }
@@ -363,11 +326,11 @@ int nzcp_ptau_new_size(uint32_t power, size_t* out_size) {
 int nzcp_ptau_new(uint32_t power, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]) {
   return api_guard([&] {
     if (!out) throw ApiError(NZCP_E_ARG, "null argument");
-    check_power(power, NZCP_E_ARG);
+    check_power(power);
     const size_t total = new_size(power);
     if (cap < total) throw ApiError(NZCP_E_ARG, "output buffer too small");
     Writer w(out, cap);
-    write_header(w, power);
+    write_ptau_header(w, power, 7);
     const G1Affine g1 = g1_generator();
     const G2Affine g2 = g2_generator();
     for (int id = 2; id <= 6; id++) {

@@ -11,12 +11,9 @@
 // The point checks run on the GPU (one thread per point); the rest is a host scan.
 #include <memory>
 
-#include "api_util.cuh"
+#include "binfile.cuh"
 
 namespace nzcp {
-
-G1Affine g1_generator();  // synth.cu
-G2Affine g2_generator();
 
 // counts[0] += points off the curve (or with a non-canonical coordinate), counts[1] += infinity markers
 template <class F>
@@ -53,42 +50,22 @@ static void check_section(const uint8_t* host, size_t n_points, const F& b, uint
   *infinity = c[1];
 }
 
-static uint32_t rd32s(const uint8_t* p) { uint32_t v; memcpy(&v, p, 4); return v; }
-static uint64_t rd64s(const uint8_t* p) { uint64_t v; memcpy(&v, p, 8); return v; }
-
 static void selfcheck_impl(const uint8_t* b, size_t len, int device, nzcp_zkey_check* rep) {
   memset(rep, 0, sizeof *rep);
-  // container (binfileutils): magic, version, nSections, (u32 id, u64 len, payload)*
-  if (len < 12 || memcmp(b, "zkey", 4) != 0) throw ApiError(NZCP_E_FORMAT, "zkey file: Invalid File format");
-  struct Sec { const uint8_t* p = nullptr; uint64_t len = 0; } s[11];
-  size_t pos = 12;
-  for (uint32_t i = 0, nsec = rd32s(b + 8); i < nsec; i++) {
-    if (pos + 12 > len) throw ApiError(NZCP_E_FORMAT, "truncated section table");
-    const uint32_t id = rd32s(b + pos);
-    const uint64_t sl = rd64s(b + pos + 4);
-    pos += 12;
-    if (sl > len - pos) throw ApiError(NZCP_E_FORMAT, "section exceeds file size");
-    if (id <= 10 && !s[id].p) { s[id].p = b + pos; s[id].len = sl; }
-    pos += sl;
-  }
-  for (int id = 1; id <= 9; id++)
-    if (!s[id].p) throw ApiError(NZCP_E_FORMAT, "zkey: missing section " + std::to_string(id));
-  if (s[1].len < 4 || rd32s(s[1].p) != 1) throw ApiError(NZCP_E_NOT_GROTH16, "zkey file is not groth16");
-  const uint8_t* h = s[2].p;
-  const size_t hdr_len = 4 + 32 + 4 + 32 + 12 + 64 + 64 + 128 + 128 + 64 + 128;
-  if (s[2].len < hdr_len) throw ApiError(NZCP_E_FORMAT, "zkey: short header");
-  rep->header_moduli_ok = rd32s(h) == 32 && rd32s(h + 36) == 32 && memcmp(h + 4, kQBytes, 32) == 0 && memcmp(h + 40, kRBytes, 32) == 0;
-  if (!rep->header_moduli_ok) throw ApiError(NZCP_E_CURVE, "zkey: curve is not bn128");
-  rep->n_vars = rd32s(h + 72);
-  rep->n_public = rd32s(h + 76);
-  rep->domain_size = rd32s(h + 80);
+  const Zkey z = read_zkey(b, len);
+  const Sect* s = z.s;
+  need_sections(s, 3, 9);
+  zkey_domain_power(z);
+  rep->header_moduli_ok = 1;   // read_zkey refuses any other
+  rep->n_vars = z.n_vars;
+  rep->n_public = z.n_public;
+  rep->domain_size = z.domain_size;
   const uint64_t m = rep->n_vars, npub = rep->n_public, n = rep->domain_size;
-  if (n < 2 || (n & (n - 1)) != 0 || npub + 1 > m) throw ApiError(NZCP_E_FORMAT, "zkey: inconsistent header dimensions");
   if (s[3].len != (npub + 1) * 64 || s[5].len != m * 64 || s[6].len != m * 64 || s[7].len != m * 128 ||
-      s[8].len != (m - npub - 1) * 64 || s[9].len != n * 64)
+      s[8].len != z.n_l() * 64 || s[9].len != n * 64)
     throw ApiError(NZCP_E_FORMAT, "zkey: point section size does not match header");
   if (s[4].len < 4) throw ApiError(NZCP_E_FORMAT, "zkey: short coefficient section");
-  const uint64_t nc = rd32s(s[4].p);
+  const uint64_t nc = rd32u(s[4].p);
   if (s[4].len != 4 + nc * 44) throw ApiError(NZCP_E_FORMAT, "zkey: coefficient section size mismatch");
   rep->n_coefs = nc;
   // section 4 scan
@@ -96,7 +73,7 @@ static void selfcheck_impl(const uint8_t* b, size_t len, int device, nzcp_zkey_c
   uint64_t bad_val = 0, bad_idx = 0;
   for (uint64_t i = 0; i < nc; i++) {
     const uint8_t* rec = cp + i * 44;
-    if (rd32s(rec) > 1 || rd32s(rec + 4) >= n || rd32s(rec + 8) >= m) bad_idx++;
+    if (rd32u(rec) > 1 || rd32u(rec + 4) >= n || rd32u(rec + 8) >= m) bad_idx++;
     if (!fr_bytes_canonical(rec + 12)) bad_val++;
   }
   rep->bad_coef_values = bad_val;
@@ -107,11 +84,11 @@ static void selfcheck_impl(const uint8_t* b, size_t len, int device, nzcp_zkey_c
   rep->public_rows_ok = nc >= npub + 1;
   if (rep->public_rows_ok) {
     const uint8_t* tail = cp + (nc - npub - 1) * 44;
-    const uint32_t c0 = rd32s(tail + 4);
+    const uint32_t c0 = rd32u(tail + 4);
     rep->n_constraints = c0;
     for (uint64_t i = 0; i <= npub; i++) {
       const uint8_t* rec = tail + i * 44;
-      if (rd32s(rec) != 0 || rd32s(rec + 4) != c0 + i || rd32s(rec + 8) != i || memcmp(rec + 12, r2b, 32) != 0) rep->public_rows_ok = 0;
+      if (rd32u(rec) != 0 || rd32u(rec + 4) != c0 + i || rd32u(rec + 8) != i || memcmp(rec + 12, r2b, 32) != 0) rep->public_rows_ok = 0;
     }
     if ((uint64_t)c0 + npub + 1 > n) rep->public_rows_ok = 0;
   }
@@ -122,21 +99,18 @@ static void selfcheck_impl(const uint8_t* b, size_t len, int device, nzcp_zkey_c
   check_section<Fq>(s[5].p, m, b1, &rep->off_curve[0], &rep->infinity[0]);
   check_section<Fq>(s[6].p, m, b1, &rep->off_curve[1], &rep->infinity[1]);
   check_section<Fq2>(s[7].p, m, b2, &rep->off_curve[2], &rep->infinity[2]);
-  check_section<Fq>(s[8].p, m - npub - 1, b1, &rep->off_curve[3], &rep->infinity[3]);
+  check_section<Fq>(s[8].p, z.n_l(), b1, &rep->off_curve[3], &rep->infinity[3]);
   check_section<Fq>(s[9].p, n, b1, &rep->off_curve[4], &rep->infinity[4]);
   check_section<Fq>(s[3].p, npub + 1, b1, &rep->off_curve[5], &rep->infinity[5]);
   // header points (host): alpha1, beta1, beta2, gamma2, delta1, delta2 -- on the curve and not infinity
-  const uint8_t* pp = h + 84;
-  bool inf = false, ok = true;
+  const uint8_t* h = s[2].p;
   G1Affine g1p;
   G2Affine g2p;
-  memcpy(&g1p, pp, 64); ok = ok && point_ok(g1p, b1, &inf) && !inf; pp += 64;       // alpha1
-  memcpy(&g1p, pp, 64); ok = ok && point_ok(g1p, b1, &inf) && !inf; pp += 64;       // beta1
-  memcpy(&g2p, pp, 128); ok = ok && point_ok(g2p, b2, &inf) && !inf; pp += 128;     // beta2
-  memcpy(&g2p, pp, 128); ok = ok && point_ok(g2p, b2, &inf) && !inf; pp += 128;     // gamma2
-  memcpy(&g1p, pp, 64); ok = ok && point_ok(g1p, b1, &inf) && !inf; pp += 64;       // delta1
-  memcpy(&g2p, pp, 128); ok = ok && point_ok(g2p, b2, &inf) && !inf;                // delta2
-  rep->header_points_ok = ok;
+  bool inf = false;
+  auto g1_ok = [&](size_t off) { memcpy(&g1p, h + off, 64); return point_ok(g1p, b1, &inf) && !inf; };
+  auto g2_ok = [&](size_t off) { memcpy(&g2p, h + off, 128); return point_ok(g2p, b2, &inf) && !inf; };
+  rep->header_points_ok = g1_ok(kZkeyAlpha1Off) && g1_ok(kZkeyBeta1Off) && g2_ok(kZkeyBeta2Off) && g2_ok(kZkeyGamma2Off) &&
+                          g1_ok(kZkeyDelta1Off) && g2_ok(kZkeyDelta2Off);
   uint64_t off = 0;
   for (int k = 0; k < 6; k++) off += rep->off_curve[k];
   rep->ok = rep->header_moduli_ok && rep->header_points_ok && rep->public_rows_ok && off == 0 && bad_val == 0 && bad_idx == 0;

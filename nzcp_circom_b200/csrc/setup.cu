@@ -31,7 +31,7 @@
 // One-time work per circuit.
 #include <memory>
 
-#include "mpc.cuh"
+#include "binfile.cuh"
 
 namespace nzcp {
 
@@ -71,14 +71,8 @@ R1cs parse_r1cs(const uint8_t* b, size_t len) {
 }
 
 Ptau parse_ptau(const uint8_t* b, size_t len) {
-  Ptau p;
-  parse_bin(b, len, "ptau", p.s, 15);
-  if (!p.s[1].p || p.s[1].len < 4 + 32 + 8) throw ApiError(NZCP_E_FORMAT, "ptau: missing header");
-  if (rd32u(p.s[1].p) != 32 || memcmp(p.s[1].p + 4, kQBytes, 32) != 0) throw ApiError(NZCP_E_CURVE, "ptau: curve is not bn128");
-  p.power = rd32u(p.s[1].p + 36);
-  if (p.power < 1 || p.power > 28) throw ApiError(NZCP_E_FORMAT, "ptau: power out of range");
-  for (int id = 2; id <= 6; id++)
-    if (!p.s[id].p) throw ApiError(NZCP_E_FORMAT, "ptau: missing section " + std::to_string(id));
+  Ptau p = read_ptau(b, len);
+  need_sections(p.s, 2, 6);
   if (!p.s[12].p || !p.s[13].p || !p.s[14].p || !p.s[15].p) throw ApiError(NZCP_E_FORMAT, "Powers of tau is not prepared.");
   const uint64_t n = (uint64_t)1 << p.power;
   // Lagrange sections: levels 0..power back to back (2^(power+1) - 1 points); tauG1 carries one more level (power + 1)
@@ -155,8 +149,8 @@ void run_combo(const Combo& cb, const Fr* d_coefs, const void* d_src0, const voi
 size_t zkey_new_size(const R1cs& r, uint32_t cir_power) {
   const uint64_t n = (uint64_t)1 << cir_power, m = r.n_wires, np = r.n_public;
   const uint64_t n_coefs = r.n_terms[0] + r.n_terms[1] + np + 1;
-  const uint64_t hdr = 4 + 32 + 4 + 32 + 12 + 64 + 64 + 128 + 128 + 64 + 128;
-  return 12 + 10 * 12 + 4 + hdr + (4 + n_coefs * 44) + (np + 1) * 64 + n * 64 + (m - np - 1) * 64 + m * 64 + m * 64 + m * 128 + 68;
+  return 12 + 10 * 12 + 4 + kZkeyHeaderLen + (4 + n_coefs * 44) + (np + 1) * 64 + n * 64 + (m - np - 1) * 64 + m * 64 + m * 64 +
+         m * 128 + 68;
 }
 
 void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b, size_t ptau_len, int device, uint8_t* out,
@@ -254,8 +248,7 @@ void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b
   w.u32(10);
   w.section(1, 4);
   w.u32(1);                                                  // groth16
-  const uint64_t hdr = 4 + 32 + 4 + 32 + 12 + 64 + 64 + 128 + 128 + 64 + 128;
-  w.section(2, hdr);
+  w.section(2, kZkeyHeaderLen);
   w.u32(32); w.raw(kQBytes, 32);
   w.u32(32); w.raw(kRBytes, 32);
   w.u32(m); w.u32(np); w.u32((uint32_t)n);

@@ -13,10 +13,6 @@ extern std::atomic<int> g_tune_pair_stage;
 extern std::atomic<int> g_tune_pair_k[kMsmMaxRounds];
 extern std::atomic<int> g_tune_rounds_w, g_tune_rounds_h;
 
-G1Affine g1_generator();  // synth.cu
-Fr host_fr_root(int k);     // ntt.cu
-G2Affine g2_generator();
-
 struct DevBuf {
   void* p = nullptr;
   explicit DevBuf(size_t bytes) { NZCP_CUDA(cudaMalloc(&p, bytes ? bytes : 16)); }

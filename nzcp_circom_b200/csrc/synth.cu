@@ -13,8 +13,6 @@
 
 namespace nzcp {
 
-Fr host_fr_root(int k);  // ntt.cu
-
 // ------------------------------------------------------------------------------------------------ PRNG
 struct Rng {
   uint64_t s;

@@ -47,8 +47,6 @@
 
 namespace nzcp {
 
-Fr host_fr_root(int k);  // ntt.cu
-
 // ------------------------------------------------------------------------------------------------ shared host/device code
 // d = hi - lo (hi = tauG1[i + N], lo = tauG1[i])
 HD G1Affine h_diff_point(const G1Affine& hi, const G1Affine& lo) {
@@ -98,19 +96,9 @@ void check_ptau_for(const Ptau& pt, uint32_t cir_power) {
   check_points<Fq>("ptau", pt.s[2].p, N + h_hash_points(N), 2, curve_b(g1_generator()));
 }
 
-uint32_t domain_power(const ZkeyIn& z) {
-  const uint64_t n = z.n_h;
-  if (n < 2 || (n & (n - 1))) throw ApiError(NZCP_E_FORMAT, "zkey: domainSize is not a power of two >= 2");
-  uint32_t p = 0;
-  while (((uint64_t)1 << p) < n) p++;
-  return p;
-}
-
-uint32_t hdr_u32(const ZkeyIn& z, int off) { return rd32u(z.s[2].p + off); }
-
 // The initial key: the sections the circuit hash reads must have the sizes its header gives.
 void check_init_sections(const ZkeyIn& z) {
-  const uint64_t m = hdr_u32(z, 72), np = hdr_u32(z, 76);
+  const uint64_t m = z.n_vars, np = z.n_public;
   const uint64_t want[8] = {0, 0, 0, (np + 1) * 64, 0, m * 64, m * 64, m * 128};
   for (int id : {3, 5, 6, 7})
     if (z.s[id].len != want[id])
@@ -127,15 +115,15 @@ struct HDiff {
 // csHash of the initial key zi (zkey_new.js order); the H differences are left in `diff`.
 void circuit_hash(const ZkeyIn& zi, const Ptau& pt, bool host, uint8_t out[64], HDiff& diff, float* kernel_ms, float* blake_ms) {
   const uint8_t* hd = zi.s[2].p;
-  const uint64_t N = zi.n_h, m = hdr_u32(zi, 72), np = hdr_u32(zi, 76);
+  const uint64_t N = zi.domain_size, m = zi.n_vars, np = zi.n_public;
   Hasher hs(host);
   const G1Affine g1 = g1_generator();
   const G2Affine g2 = g2_generator();
-  hs.points_host(reinterpret_cast<const G1Affine*>(hd + 84), 2);     // alpha1, beta1
-  hs.points_host(reinterpret_cast<const G2Affine*>(hd + 212), 1);    // beta2
-  hs.points_host(&g2, 1);                                             // gamma2
-  hs.points_host(&g1, 1);                                             // delta1
-  hs.points_host(&g2, 1);                                             // delta2
+  hs.points_host(reinterpret_cast<const G1Affine*>(hd + kZkeyAlpha1Off), 2);   // alpha1, beta1
+  hs.points_host(reinterpret_cast<const G2Affine*>(hd + kZkeyBeta2Off), 1);    // beta2
+  hs.points_host(&g2, 1);                                                      // gamma2
+  hs.points_host(&g1, 1);                                                      // delta1
+  hs.points_host(&g2, 1);                                                      // delta2
   hs.u32be((uint32_t)(np + 1));
   hs.section<Fq>(zi.s[3].p, np + 1);
   hs.u32be((uint32_t)(N - 1));
@@ -237,12 +225,12 @@ void check_key_points(const ZkeyIn& z, const std::vector<Rec>& recs) {
     if (subgroup && !in_g2_subgroup(a)) throw Verdict{1, -1, "zkey: " + what + " is not in the order-r subgroup of G2"};
   };
   const uint8_t* h = z.s[2].p;
-  g1(h + 84, "header alpha1");
-  g1(h + 148, "header beta1");
-  g2(h + 212, "header beta2", false);
-  g2(h + 340, "header gamma2", false);
-  g1(h + kDelta1Off, "header delta1");
-  g2(h + kDelta2Off, "header delta2", true);
+  g1(h + kZkeyAlpha1Off, "header alpha1");
+  g1(h + kZkeyBeta1Off, "header beta1");
+  g2(h + kZkeyBeta2Off, "header beta2", false);
+  g2(h + kZkeyGamma2Off, "header gamma2", false);
+  g1(h + kZkeyDelta1Off, "header delta1");
+  g2(h + kZkeyDelta2Off, "header delta2", true);
   for (size_t i = 0; i < recs.size(); i++) {
     const std::string w = "section 10 record " + std::to_string(i) + " ";
     g1(recs[i].p, w + "deltaAfter");
@@ -251,8 +239,8 @@ void check_key_points(const ZkeyIn& z, const std::vector<Rec>& recs) {
     g2(recs[i].p + 192, w + "g2_spx", true);
   }
   try {
-    check_points<Fq>("zkey", z.s[8].p, z.n_l, 8, b1);
-    check_points<Fq>("zkey", z.s[9].p, z.n_h, 9, b1);
+    check_points<Fq>("zkey", z.s[8].p, z.n_l(), 8, b1);
+    check_points<Fq>("zkey", z.s[9].p, z.domain_size, 9, b1);
   } catch (const ApiError& e) {
     throw Verdict{1, -1, e.what()};
   }
@@ -369,15 +357,17 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   }
 
   // 2. the headers
-  for (int off : {72, 76, 80})
-    if (hdr_u32(z, off) != hdr_u32(zi, off)) throw Verdict{6, -1, "Different circuit parameters"};
+  if (z.n_vars != zi.n_vars || z.n_public != zi.n_public || z.domain_size != zi.domain_size)
+    throw Verdict{6, -1, "Different circuit parameters"};
   const uint8_t *h = z.s[2].p, *hi = zi.s[2].p;
-  const struct { int off, len; const char* msg; } same[] = {
-      {84, 64, "Invalid alpha1"}, {148, 64, "Invalid beta1"}, {212, 128, "Invalid beta2"}, {340, 128, "Invalid gamma2"}};
+  const struct { size_t off, len; const char* msg; } same[] = {{kZkeyAlpha1Off, 64, "Invalid alpha1"},
+                                                              {kZkeyBeta1Off, 64, "Invalid beta1"},
+                                                              {kZkeyBeta2Off, 128, "Invalid beta2"},
+                                                              {kZkeyGamma2Off, 128, "Invalid gamma2"}};
   for (const auto& s : same)
     if (memcmp(h + s.off, hi + s.off, s.len) != 0) throw Verdict{7, -1, s.msg};
-  if (memcmp(h + kDelta1Off, &cur, 64) != 0) throw Verdict{7, -1, "Invalid delta1"};
-  const G2Affine delta2 = load_pt<Fq2>(h + kDelta2Off), delta2_init = load_pt<Fq2>(hi + kDelta2Off);
+  if (memcmp(h + kZkeyDelta1Off, &cur, 64) != 0) throw Verdict{7, -1, "Invalid delta1"};
+  const G2Affine delta2 = load_pt<Fq2>(h + kZkeyDelta2Off), delta2_init = load_pt<Fq2>(hi + kZkeyDelta2Off);
   cl.add(8, -1, g1, cur, g2, delta2);
 
   // 3. the circuit, 4. the sections that no contribution changes
@@ -399,8 +389,8 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
     }
   }
   ChaCha rng(sd);
-  const uint64_t N = z.n_h;
-  std::vector<Fr> sc(std::max(z.n_l, N));
+  const uint64_t N = z.domain_size, n_l = z.n_l();
+  std::vector<Fr> sc(std::max(n_l, N));
   Events ev;
   auto timed = [&](float& acc_ms, auto&& fn) {   // device time of fn's work on the default stream, added to acc_ms
     NZCP_CUDA(cudaEventRecord(ev.a, 0));
@@ -414,14 +404,14 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   };
 
   // 5. L: sum rho_i L_init[i] and sum rho_i L[i]
-  if (z.n_l) {
-    for (uint64_t i = 0; i < z.n_l; i++) sc[i] = fp_from_rng<FrParams>(rng);
-    DevMem d_sc(z.n_l * sizeof(Fr)), d_b(z.n_l * 64);
-    NZCP_CUDA(cudaMemcpy(d_sc.p, sc.data(), z.n_l * sizeof(Fr), cudaMemcpyHostToDevice));
-    NZCP_CUDA(cudaMemcpy(d_b.p, zi.s[8].p, z.n_l * 64, cudaMemcpyHostToDevice));
-    const G1Affine r1 = timed(ms[2], [&] { return msm_g1(d_b.p, static_cast<const Fr*>(d_sc.p), z.n_l); });
-    NZCP_CUDA(cudaMemcpy(d_b.p, z.s[8].p, z.n_l * 64, cudaMemcpyHostToDevice));
-    const G1Affine r2 = timed(ms[2], [&] { return msm_g1(d_b.p, static_cast<const Fr*>(d_sc.p), z.n_l); });
+  if (n_l) {
+    for (uint64_t i = 0; i < n_l; i++) sc[i] = fp_from_rng<FrParams>(rng);
+    DevMem d_sc(n_l * sizeof(Fr)), d_b(n_l * 64);
+    NZCP_CUDA(cudaMemcpy(d_sc.p, sc.data(), n_l * sizeof(Fr), cudaMemcpyHostToDevice));
+    NZCP_CUDA(cudaMemcpy(d_b.p, zi.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
+    const G1Affine r1 = timed(ms[2], [&] { return msm_g1(d_b.p, static_cast<const Fr*>(d_sc.p), n_l); });
+    NZCP_CUDA(cudaMemcpy(d_b.p, z.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
+    const G1Affine r2 = timed(ms[2], [&] { return msm_g1(d_b.p, static_cast<const Fr*>(d_sc.p), n_l); });
     cl.add(11, -1, r1, r2, delta2, delta2_init);
   }
 
@@ -504,7 +494,7 @@ int nzcp_zkey_circuit_hash(const uint8_t* init, size_t init_len, const uint8_t* 
     const ZkeyIn zi = parse_zkey_in(init, init_len);
     check_init_sections(zi);
     const Ptau pt = parse_ptau(ptau, ptau_len);
-    check_ptau_for(pt, domain_power(zi));
+    check_ptau_for(pt, zkey_domain_power(zi));
     use_device(device);
     HDiff diff;
     circuit_hash(zi, pt, false, hash, diff, ms, ms ? ms + 1 : nullptr);
@@ -517,8 +507,8 @@ int nzcp_host_zkey_circuit_hash(const uint8_t* init, size_t init_len, const uint
     const ZkeyIn zi = parse_zkey_in(init, init_len);
     check_init_sections(zi);
     const Ptau pt = parse_ptau(ptau, ptau_len);
-    check_ptau_for(pt, domain_power(zi));
-    if (zi.n_h > kHostMaxPoints) throw ApiError(NZCP_E_ARG, "zkey: the host run is limited to 4096 H points");
+    check_ptau_for(pt, zkey_domain_power(zi));
+    if (zi.domain_size > kHostMaxPoints) throw ApiError(NZCP_E_ARG, "zkey: the host run is limited to 4096 H points");
     HDiff diff;
     circuit_hash(zi, pt, true, hash, diff, nullptr, nullptr);
   });
@@ -547,7 +537,7 @@ int nzcp_zkey_verify_from_init(const uint8_t* init, size_t init_len, const uint8
     in.init = parse_zkey_in(init, init_len);
     check_init_sections(in.init);
     in.pt = parse_ptau(ptau, ptau_len);
-    in.cir_power = domain_power(in.init);
+    in.cir_power = zkey_domain_power(in.init);
     check_ptau_for(in.pt, in.cir_power);
     use_device(device);
     run(in, in.init.s[10].p, o);
