@@ -6,6 +6,7 @@
 #include <atomic>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "ec.cuh"
@@ -40,6 +41,74 @@ extern thread_local std::atomic<uint64_t>* t_launch_sink;
 
 static inline unsigned div_up(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
 
+// Owner of CUDA device memory, pinned host memory, events and streams.  Each acquire call returns the raw pointer or
+// handle, which the caller keeps in plain non-owning fields; the destructor releases everything in reverse order of
+// acquisition, ignoring return codes (it runs during unwinding).  Sizes are exactly what the caller asks for.
+class CudaResources {
+ public:
+  CudaResources() = default;
+  CudaResources(CudaResources&& o) noexcept { *this = std::move(o); }
+  CudaResources& operator=(CudaResources&& o) noexcept {   // a swap: what this held is released with `o`
+    items_.swap(o.items_);
+    std::swap(device_bytes_, o.device_bytes_);
+    return *this;
+  }
+  ~CudaResources() { release(); }
+
+  template <class T>
+  T* device(size_t count) {
+    void*& p = slot(kDevice);
+    NZCP_CUDA(cudaMalloc(&p, count * sizeof(T)));
+    device_bytes_ += count * sizeof(T);
+    return static_cast<T*>(p);
+  }
+  template <class T>
+  T* pinned(size_t count) {
+    void*& p = slot(kPinned);
+    NZCP_CUDA(cudaMallocHost(&p, count * sizeof(T)));
+    return static_cast<T*>(p);
+  }
+  cudaEvent_t event() {
+    void*& h = slot(kEvent);
+    cudaEvent_t e = nullptr;
+    NZCP_CUDA(cudaEventCreate(&e));
+    h = e;
+    return e;
+  }
+  cudaStream_t stream() {   // non-blocking: never synchronises with the legacy default stream
+    void*& h = slot(kStream);
+    cudaStream_t s = nullptr;
+    NZCP_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    h = s;
+    return s;
+  }
+  size_t device_bytes() const { return device_bytes_; }   // sum of the device() sizes
+
+ private:
+  enum Kind { kDevice, kPinned, kEvent, kStream };
+  struct Item { Kind kind; void* h; };
+  // The record exists before the resource, so a resource that was created is always released.
+  void*& slot(Kind k) {
+    items_.push_back({k, nullptr});
+    return items_.back().h;
+  }
+  void release() noexcept {
+    for (auto it = items_.rbegin(); it != items_.rend(); ++it) {
+      if (!it->h) continue;
+      switch (it->kind) {
+        case kDevice: cudaFree(it->h); break;
+        case kPinned: cudaFreeHost(it->h); break;
+        case kEvent: cudaEventDestroy(static_cast<cudaEvent_t>(it->h)); break;
+        case kStream: cudaStreamDestroy(static_cast<cudaStream_t>(it->h)); break;
+      }
+    }
+    items_.clear();
+    device_bytes_ = 0;
+  }
+  std::vector<Item> items_;
+  size_t device_bytes_ = 0;
+};
+
 G1Affine g1_generator();   // synth.cu: the BN254 generators, Montgomery affine
 G2Affine g2_generator();
 Fr host_fr_root(int k);    // ntt.cu: ffjavascript's Fr.w[k], Montgomery
@@ -54,9 +123,9 @@ struct NttDomain {
   Fr* ninv_scale = nullptr;   // unused slot kept for standalone iNTT: single element n^-1 (device)
   unsigned char* tw_lo_fwd = nullptr;   // log_n >= 10: w^(j n/1024), j < 512, padded layout (ntt.cu tw_pad_off): the twiddles
   unsigned char* tw_lo_inv = nullptr;   // of every stage of a 2^10 tile, bulk-copied into shared memory by the low pass
+  CudaResources res;
 };
 void ntt_domain_create(NttDomain* d, int log_n, cudaStream_t st);
-void ntt_domain_destroy(NttDomain* d);
 // H pipeline on `batch` polynomials laid out back to back (batch * n elements), in place:
 //   evaluations on the 2^log_n subgroup (natural order)  ->  evaluations on the coset inc*subgroup (natural order)
 void ntt_coset_pipeline(const NttDomain& d, Fr* data, int batch, cudaStream_t st);
@@ -87,8 +156,8 @@ struct MsmTable {
   size_t n_points = 0;   // including pad_front leading infinity points
   int c = 0, n_windows = 0;
   bool g2 = false;
-  bool owned = true;     // false: a view over the caller's bases (msm_table_view)
   size_t bytes = 0;
+  CudaResources res;     // empty for a view over the caller's bases (msm_table_view)
 };
 int msm_pick_window(size_t n_points);
 int msm_num_windows(int c);
@@ -97,7 +166,6 @@ int msm_pick_window_free(size_t n_points);
 void msm_table_create(MsmTable* t, const void* d_bases, size_t n_src, size_t pad_front, bool g2, int c, cudaStream_t st);
 // "Table" view of raw bases for the table-free path (one window, memory owned by the caller).
 void msm_table_view(MsmTable* t, void* d_bases, size_t n_points, bool g2, int c);
-void msm_table_destroy(MsmTable* t);
 
 static constexpr int kMsmMaxRounds = 3;
 
@@ -132,11 +200,11 @@ struct MsmSort {
   uint32_t* round_off = nullptr;
   uint32_t* red_count = nullptr;
   size_t round_max[kMsmMaxRounds + 1] = {0, 0, 0, 0};   // upper bound of the point count after round r
+  CudaResources res;
 };
 int msm_pick_rounds(size_t n_points, int c);
 int msm_pick_rounds_prover(size_t n_points, int c);
 void msm_sort_create(MsmSort* s, size_t n_points, int c, int rounds = -1, bool table_free = false);   // rounds < 0: msm_pick_rounds
-void msm_sort_destroy(MsmSort* s);
 void msm_sort_launch(MsmSort* s, const Fr* scalars, size_t n_points, cudaStream_t st);
 // After the stream drained: throws if the device flagged a scalar >= r.  Returns the number of non-zero digits.
 uint32_t msm_sort_check(const MsmSort* s);
@@ -163,9 +231,9 @@ struct MsmRun {
   void* round_ops = nullptr;                 // round 1: the two operands of every addition, staged by the forward pass
   void* round_prod = nullptr;                // per-thread denominator products, inverted in place between the passes
   size_t scratch_bytes = 0;
+  CudaResources res;
 };
 void msm_run_create(MsmRun* r, const MsmSort* sort, bool g2);
-void msm_run_destroy(MsmRun* r);
 void msm_run_launch(MsmRun* r, const MsmSort* sort, const MsmTable* table, cudaStream_t st);
 void msm_run_finish_device(MsmRun* r, cudaStream_t st);
 void msm_sum_points(const void* d_pts, uint32_t count, bool g2, void* d_result, cudaStream_t st);

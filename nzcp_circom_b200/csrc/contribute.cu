@@ -53,16 +53,17 @@ size_t contribute_size(const ZkeyIn& z, size_t name_len, size_t beacon_len) {
 // Scale n points of src by k into dst; returns the kernel's device milliseconds.  d_buf holds at least n points.
 float scale_section_device(const uint8_t* src, uint64_t n, const Fr& k, G1Affine* d_buf, uint8_t* dst) {
   if (n == 0) return 0.f;
-  Events ev;
+  CudaResources res;
+  const cudaEvent_t e0 = res.event(), e1 = res.event();
   NZCP_CUDA(cudaMemcpyAsync(d_buf, src, n * 64, cudaMemcpyHostToDevice, 0));
-  NZCP_CUDA(cudaEventRecord(ev.a, 0));
+  NZCP_CUDA(cudaEventRecord(e0, 0));
   zkey_scale_kernel<<<div_up(n, 128), 128>>>(d_buf, k, n);
   NZCP_LAUNCH_CHECK();
-  NZCP_CUDA(cudaEventRecord(ev.b, 0));
+  NZCP_CUDA(cudaEventRecord(e1, 0));
   NZCP_CUDA(cudaMemcpyAsync(dst, d_buf, n * 64, cudaMemcpyDeviceToHost, 0));
   NZCP_CUDA(cudaStreamSynchronize(0));
   float ms = 0;
-  NZCP_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
+  NZCP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
   return ms;
 }
 
@@ -156,15 +157,16 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
     w.section(id, z.s[id].len);
     w.raw(z.s[id].p, z.s[id].len);
   }
-  std::unique_ptr<DevMem> d_buf;
-  if (!host) d_buf.reset(new DevMem(std::max<uint64_t>(z.n_l(), z.domain_size) * 64));
+  CudaResources res;
+  const size_t buf_bytes = std::max<uint64_t>(z.n_l(), z.domain_size) * 64;
+  G1Affine* d_buf = host ? nullptr : reinterpret_cast<G1Affine*>(res.device<unsigned char>(buf_bytes ? buf_bytes : 16));
   for (int id = 8; id <= 9; id++) {
     const uint64_t n = id == 8 ? z.n_l() : z.domain_size;
     w.section(id, n * 64);
     uint8_t* dst = w.reserve(n * 64);
     float ms = 0;
     if (host) scale_section_host(z.s[id].p, n, k_inv, dst);
-    else ms = scale_section_device(z.s[id].p, n, k_inv, static_cast<G1Affine*>(d_buf->p), dst);
+    else ms = scale_section_device(z.s[id].p, n, k_inv, d_buf, dst);
     if (section_ms) section_ms[id - 8] = ms;
   }
   w.section(10, z.s[10].len + rec.size());

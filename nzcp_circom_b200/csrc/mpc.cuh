@@ -6,7 +6,6 @@
 #include <sys/random.h>
 
 #include <chrono>
-#include <memory>
 
 #include "binfile.cuh"
 
@@ -472,24 +471,6 @@ ZkeyIn parse_zkey_in(const uint8_t* b, size_t len, bool check_pts = true) {
   return z;
 }
 
-struct DevMem {
-  void* p = nullptr;
-  explicit DevMem(size_t bytes) { NZCP_CUDA(cudaMalloc(&p, bytes ? bytes : 16)); }
-  ~DevMem() { cudaFree(p); }
-};
-
-struct Events {
-  cudaEvent_t a = nullptr, b = nullptr;
-  Events() {
-    NZCP_CUDA(cudaEventCreate(&a));
-    NZCP_CUDA(cudaEventCreate(&b));
-  }
-  ~Events() {
-    if (a) cudaEventDestroy(a);
-    if (b) cudaEventDestroy(b);
-  }
-};
-
 // ------------------------------------------------------------------------------------------------ point encodings (device)
 HD uint32_t bswap32(uint32_t v) { return (v >> 24) | ((v >> 8) & 0xff00u) | ((v << 8) & 0xff0000u) | (v << 24); }
 HD void put_be(const Fq& a, uint32_t* w) {
@@ -563,24 +544,19 @@ struct Hasher {
   bool host;
   Enc enc;
   float kernel_ms = 0, blake_ms = 0;
-  std::unique_ptr<DevMem> d_enc[2];
+  uint32_t* d_enc[2] = {nullptr, nullptr};
   uint8_t* h_enc[2] = {nullptr, nullptr};
   cudaEvent_t ev[6] = {};   // per buffer: kernel start, kernel end, copy done
+  CudaResources res;
 
   explicit Hasher(bool on_host, Enc e = Enc::U) : host(on_host), enc(e) {
     if (host) return;
     for (int b = 0; b < 2; b++) {
-      d_enc[b].reset(new DevMem(kHashChunk * 128));
-      NZCP_CUDA(cudaMallocHost((void**)&h_enc[b], kHashChunk * 128));
+      d_enc[b] = res.device<uint32_t>(kHashChunk * 32);
+      h_enc[b] = res.pinned<uint8_t>(kHashChunk * 128);
     }
-    for (auto& e : ev) NZCP_CUDA(cudaEventCreate(&e));
+    for (auto& e : ev) e = res.event();
   }
-  ~Hasher() {
-    for (auto p : h_enc) if (p) cudaFreeHost(p);
-    for (auto e : ev) if (e) cudaEventDestroy(e);
-  }
-  Hasher(const Hasher&) = delete;
-  Hasher& operator=(const Hasher&) = delete;
   template <class F>
   static constexpr size_t enc_bytes(Enc e) { return e == Enc::U ? sizeof(Affine<F>) : sizeof(Affine<F>) / 2; }
   void update(const void* p, size_t n) {
@@ -616,13 +592,13 @@ struct Hasher {
       if (j < nch) {
         const int b = j & 1;
         const uint64_t off = j * kHashChunk, m = std::min(kHashChunk, n - off);
-        uint32_t* dst = static_cast<uint32_t*>(d_enc[b]->p);
+        uint32_t* dst = d_enc[b];
         NZCP_CUDA(cudaEventRecord(ev[3 * b], 0));
         if (enc == Enc::U) u_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, dst, m);
         else c_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, dst, m);
         NZCP_LAUNCH_CHECK();
         NZCP_CUDA(cudaEventRecord(ev[3 * b + 1], 0));
-        NZCP_CUDA(cudaMemcpyAsync(h_enc[b], d_enc[b]->p, m * esz, cudaMemcpyDeviceToHost, 0));
+        NZCP_CUDA(cudaMemcpyAsync(h_enc[b], d_enc[b], m * esz, cudaMemcpyDeviceToHost, 0));
         NZCP_CUDA(cudaEventRecord(ev[3 * b + 2], 0));
       }
       if (j > 0) {
@@ -641,9 +617,10 @@ struct Hasher {
   void section(const uint8_t* p, uint64_t n) {
     const Affine<F>* a = reinterpret_cast<const Affine<F>*>(p);
     if (host || n == 0) return points_host(a, n);
-    DevMem d(n * sizeof(Affine<F>));
-    NZCP_CUDA(cudaMemcpy(d.p, p, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-    points_device(static_cast<const Affine<F>*>(d.p), n);
+    CudaResources staged;
+    Affine<F>* d = staged.device<Affine<F>>(n);   // n > 0
+    NZCP_CUDA(cudaMemcpy(d, p, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
+    points_device(d, n);
   }
 };
 

@@ -860,15 +860,6 @@ int msm_pick_rounds_prover(size_t n_points, int c) {
   return n_points * (size_t)msm_num_windows(c) >= ((size_t)1 << 22) ? kMsmMaxRounds : 0;
 }
 
-template <class T>
-static T* dev_alloc(size_t count, size_t* total) {
-  T* p = nullptr;
-  size_t bytes = (count ? count : 1) * sizeof(T);
-  NZCP_CUDA(cudaMalloc(&p, bytes));
-  *total += bytes;
-  return p;
-}
-
 void msm_table_create(MsmTable* t, const void* d_bases, size_t n_src, size_t pad_front, bool g2, int c, cudaStream_t st) {
   *t = MsmTable();
   if (c < 2 || c > 20) throw std::runtime_error("msm: window size out of range");
@@ -879,7 +870,7 @@ void msm_table_create(MsmTable* t, const void* d_bases, size_t n_src, size_t pad
   size_t psz = g2 ? sizeof(G2Affine) : sizeof(G1Affine);
   if ((size_t)t->n_windows * t->n_points >= ((size_t)1 << 31)) throw std::runtime_error("msm: too many points");
   t->bytes = (size_t)t->n_windows * (t->n_points ? t->n_points : 1) * psz;
-  NZCP_CUDA(cudaMalloc(&t->pts, t->bytes));
+  t->pts = t->res.device<unsigned char>(t->bytes);
   if (t->n_points == 0) return;
   unsigned grid = div_up(t->n_points, 128);
   if (g2)
@@ -898,12 +889,6 @@ void msm_table_view(MsmTable* t, void* d_bases, size_t n_points, bool g2, int c)
   t->c = c;
   t->n_windows = 1;
   t->g2 = g2;
-  t->owned = false;
-}
-
-void msm_table_destroy(MsmTable* t) {
-  if (t->owned) cudaFree(t->pts);
-  *t = MsmTable();
 }
 
 void msm_sort_create(MsmSort* s, size_t n_points, int c, int rounds, bool table_free) {
@@ -924,44 +909,28 @@ void msm_sort_create(MsmSort* s, size_t n_points, int c, int rounds, bool table_
   size_t by_len = max_entries / kTaskLenMax, by_target = 2 * (size_t)kTargetTasks;
   if (max_entries / kTaskLenMin < by_target) by_target = max_entries / kTaskLenMin;
   s->max_tasks = s->n_buckets + (by_len > by_target ? by_len : by_target) + 1;
-  size_t tot = 0;
   s->smem_hist = s->n_buckets <= (size_t)kSmemHistBuckets;
   s->n_copies = s->smem_hist ? 148 : kCopiesGlobal;
   size_t n_ctr = s->n_buckets * s->n_copies;
-  s->counts = dev_alloc<uint32_t>(n_ctr + 1, &tot);
-  s->offsets = dev_alloc<uint32_t>(n_ctr + 1, &tot);
-  s->cursors = dev_alloc<uint32_t>(n_ctr + 1, &tot);
-  s->red_count = dev_alloc<uint32_t>(s->n_buckets + 1, &tot);
-  s->round_off = dev_alloc<uint32_t>((size_t)(kMsmMaxRounds + 1) * (s->n_buckets + 1), &tot);
+  s->counts = s->res.device<uint32_t>(n_ctr + 1);
+  s->offsets = s->res.device<uint32_t>(n_ctr + 1);
+  s->cursors = s->res.device<uint32_t>(n_ctr + 1);
+  s->red_count = s->res.device<uint32_t>(s->n_buckets + 1);
+  s->round_off = s->res.device<uint32_t>((size_t)(kMsmMaxRounds + 1) * (s->n_buckets + 1));
   s->round_max[0] = max_entries;
   for (int r = 1; r <= kMsmMaxRounds; r++) s->round_max[r] = (s->round_max[r - 1] + s->n_buckets) / 2 + 1;
-  s->block_sums = dev_alloc<uint32_t>(2 * (n_ctr / kScanBlock + 2), &tot);
+  s->block_sums = s->res.device<uint32_t>(2 * (n_ctr / kScanBlock + 2));
   if (s->smem_hist) {  // function attributes are per device: set them whenever a plan is created on the current one
     NZCP_CUDA(cudaFuncSetAttribute(msm_digits_smem_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHistBuckets * 4));
     NZCP_CUDA(cudaFuncSetAttribute(msm_digits_smem_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemHistBuckets * 4));
   }
-  s->entries = dev_alloc<uint32_t>(max_entries, &tot);
-  s->task_off = dev_alloc<uint32_t>(s->n_buckets + 1, &tot);
-  s->tasks = dev_alloc<uint2>(s->max_tasks, &tot);
-  s->flags = dev_alloc<uint32_t>(8, &tot);
-  NZCP_CUDA(cudaMallocHost(&s->flags_host, 8 * sizeof(uint32_t)));
+  s->entries = s->res.device<uint32_t>(max_entries ? max_entries : 1);
+  s->task_off = s->res.device<uint32_t>(s->n_buckets + 1);
+  s->tasks = s->res.device<uint2>(s->max_tasks);
+  s->flags = s->res.device<uint32_t>(8);
+  s->flags_host = s->res.pinned<uint32_t>(8);
   memset(s->flags_host, 0, 8 * sizeof(uint32_t));
-  s->scratch_bytes = tot;
-}
-
-void msm_sort_destroy(MsmSort* s) {
-  cudaFree(s->counts);
-  cudaFree(s->offsets);
-  cudaFree(s->cursors);
-  cudaFree(s->red_count);
-  cudaFree(s->round_off);
-  cudaFree(s->block_sums);
-  cudaFree(s->entries);
-  cudaFree(s->task_off);
-  cudaFree(s->tasks);
-  cudaFree(s->flags);
-  if (s->flags_host) cudaFreeHost(s->flags_host);
-  *s = MsmSort();
+  s->scratch_bytes = s->res.device_bytes();
 }
 
 void msm_sort_launch(MsmSort* s, const Fr* scalars, size_t n_points, cudaStream_t st) {
@@ -1037,7 +1006,6 @@ void msm_run_create(MsmRun* r, const MsmSort* sort, bool g2) {
   *r = MsmRun();
   r->g2 = g2;
   size_t psz = g2 ? sizeof(G2XYZZ) : sizeof(G1XYZZ);
-  size_t tot = 0;
   if (g2) {  // > 48 KB of dynamic shared memory; function attributes are per device
     NZCP_CUDA(cudaFuncSetAttribute(msm_combine_heavy_kernel<Fq2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)(kHeavyThreads * sizeof(G2XYZZ))));
@@ -1046,58 +1014,36 @@ void msm_run_create(MsmRun* r, const MsmSort* sort, bool g2) {
     NZCP_CUDA(cudaFuncSetAttribute(msm_marginal_kernel<Fq2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)(kMargThreads * sizeof(G2XYZZ))));
   }
-  r->partial = dev_alloc<unsigned char>(sort->max_tasks * psz, &tot);
-  r->buckets = dev_alloc<unsigned char>(sort->n_buckets * psz, &tot);
+  r->partial = r->res.device<unsigned char>(sort->max_tasks * psz);
+  r->buckets = r->res.device<unsigned char>(sort->n_buckets * psz);
   r->n_groups = sort->n_groups;
   r->c = sort->c;
-  r->marg = dev_alloc<unsigned char>((size_t)r->n_groups * kMaxDigits * 32 * psz, &tot);
-  r->marg_done = dev_alloc<uint32_t>((size_t)r->n_groups * kMaxDigits, &tot);
+  r->marg = r->res.device<unsigned char>((size_t)r->n_groups * kMaxDigits * 32 * psz);
+  r->marg_done = r->res.device<uint32_t>((size_t)r->n_groups * kMaxDigits);
   NZCP_CUDA(cudaMemset(r->marg_done, 0, (size_t)r->n_groups * kMaxDigits * sizeof(uint32_t)));
-  r->result = dev_alloc<unsigned char>(psz, &tot);
-  r->heavy_list = dev_alloc<uint32_t>(sort->n_buckets, &tot);
-  r->heavy_count = dev_alloc<uint32_t>(2, &tot);
-  r->chunk_off = dev_alloc<uint32_t>(sort->n_buckets + 1, &tot);
-  r->chunk_partial = dev_alloc<unsigned char>((sort->max_tasks / kHeavyChunk + sort->n_buckets + 1) * psz, &tot);
-  r->out = dev_alloc<unsigned char>((size_t)r->n_groups * (kMaxDigits + 1) * psz, &tot);
-  NZCP_CUDA(cudaMallocHost(&r->out_host, (size_t)r->n_groups * (kMaxDigits + 1) * psz));
+  r->result = r->res.device<unsigned char>(psz);
+  r->heavy_list = r->res.device<uint32_t>(sort->n_buckets);
+  r->heavy_count = r->res.device<uint32_t>(2);
+  r->chunk_off = r->res.device<uint32_t>(sort->n_buckets + 1);
+  r->chunk_partial = r->res.device<unsigned char>((sort->max_tasks / kHeavyChunk + sort->n_buckets + 1) * psz);
+  r->out = r->res.device<unsigned char>((size_t)r->n_groups * (kMaxDigits + 1) * psz);
+  r->out_host = r->res.pinned<unsigned char>((size_t)r->n_groups * (kMaxDigits + 1) * psz);
   memset(r->out_host, 0, (size_t)r->n_groups * (kMaxDigits + 1) * psz);
   r->n_digits = (sort->c - 1 + 4) / 5;
   NZCP_CUDA(cudaFuncSetAttribute(msm_sum_points_kernel<Fq2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)(kHeavyThreads * sizeof(G2XYZZ))));
   if (sort->rounds > 0) {
     const size_t asz = g2 ? sizeof(G2Affine) : sizeof(G1Affine), fsz = asz / 2, pad = 128 * 64;
-    r->round_pts[0] = dev_alloc<unsigned char>((sort->round_max[1] + pad) * asz, &tot);
-    if (sort->rounds > 1) r->round_pts[1] = dev_alloc<unsigned char>((sort->round_max[2] + pad) * asz, &tot);
-    r->round_prefix = dev_alloc<unsigned char>((sort->round_max[1] + pad) * fsz, &tot);
+    r->round_pts[0] = r->res.device<unsigned char>((sort->round_max[1] + pad) * asz);
+    if (sort->rounds > 1) r->round_pts[1] = r->res.device<unsigned char>((sort->round_max[2] + pad) * asz);
+    r->round_prefix = r->res.device<unsigned char>((sort->round_max[1] + pad) * fsz);
     if (g_tune_pair_stage.load())   // opt-in ("pair_stage", read when the run is created): two operands per round-1 addition
-      r->round_ops = dev_alloc<unsigned char>((sort->round_max[1] + pad) * 2 * asz, &tot);
-    r->round_prod = dev_alloc<unsigned char>((sort->round_max[1] / 4 + pad) * fsz, &tot);   // >= 4 additions per thread
+      r->round_ops = r->res.device<unsigned char>((sort->round_max[1] + pad) * 2 * asz);
+    r->round_prod = r->res.device<unsigned char>((sort->round_max[1] / 4 + pad) * fsz);   // >= 4 additions per thread
   }
-  NZCP_CUDA(cudaEventCreate(&r->ev_acc0));
-  NZCP_CUDA(cudaEventCreate(&r->ev_acc1));
-  r->scratch_bytes = tot;
-}
-
-void msm_run_destroy(MsmRun* r) {
-  cudaFree(r->partial);
-  cudaFree(r->buckets);
-  cudaFree(r->marg);
-  cudaFree(r->marg_done);
-  cudaFree(r->result);
-  cudaFree(r->heavy_list);
-  cudaFree(r->heavy_count);
-  cudaFree(r->chunk_off);
-  cudaFree(r->chunk_partial);
-  cudaFree(r->out);
-  cudaFree(r->round_pts[0]);
-  cudaFree(r->round_pts[1]);
-  cudaFree(r->round_prefix);
-  cudaFree(r->round_ops);
-  cudaFree(r->round_prod);
-  if (r->out_host) cudaFreeHost(r->out_host);
-  if (r->ev_acc0) cudaEventDestroy(r->ev_acc0);
-  if (r->ev_acc1) cudaEventDestroy(r->ev_acc1);
-  *r = MsmRun();
+  r->ev_acc0 = r->res.event();
+  r->ev_acc1 = r->res.event();
+  r->scratch_bytes = r->res.device_bytes();
 }
 
 template <class F>

@@ -26,11 +26,12 @@ struct nzcp_msm_plan {
   size_t n_points = 0;
   void* d_bases = nullptr;    // mode 1: the raw bases stay resident; mode 0: freed after the table is built
   Fr* d_scalars = nullptr;
+  cudaStream_t st = nullptr;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  CudaResources res;          // st, ev0, ev1, d_scalars and the mode-1 bases
   MsmTable tab;
   MsmSort sort;
   MsmRun run;
-  cudaStream_t st = nullptr;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
 namespace nzcp {
@@ -38,14 +39,6 @@ namespace nzcp {
 static void plan_release(nzcp_msm_plan* p) {
   if (!p) return;
   cudaSetDevice(p->device);
-  msm_run_destroy(&p->run);
-  msm_sort_destroy(&p->sort);
-  msm_table_destroy(&p->tab);
-  cudaFree(p->d_bases);
-  cudaFree(p->d_scalars);
-  if (p->ev0) cudaEventDestroy(p->ev0);
-  if (p->ev1) cudaEventDestroy(p->ev1);
-  if (p->st) cudaStreamDestroy(p->st);
   delete p;
 }
 
@@ -63,18 +56,19 @@ static nzcp_msm_plan* plan_create_impl(const uint8_t* bases, size_t n_points, in
   int c = window_bits > 0 ? window_bits : (mode == 1 ? msm_pick_window_free(np) : msm_pick_window(np));
   if (mode == 1 && (size_t)msm_num_windows(c) << (c - 1) > ((size_t)1 << 19))
     throw ApiError(NZCP_E_ARG, "window size too large for the variable-base path (windows * 2^(c-1) must be <= 2^19)");
-  NZCP_CUDA(cudaStreamCreateWithFlags(&p->st, cudaStreamNonBlocking));
-  NZCP_CUDA(cudaEventCreate(&p->ev0));
-  NZCP_CUDA(cudaEventCreate(&p->ev1));
-  NZCP_CUDA(cudaMalloc(&p->d_bases, np * bsz));
-  NZCP_CUDA(cudaMalloc((void**)&p->d_scalars, np * sizeof(Fr)));
+  p->st = p->res.stream();
+  p->ev0 = p->res.event();
+  p->ev1 = p->res.event();
+  CudaResources staged;       // mode 0: the raw bases, freed as soon as the window table is built
+  p->d_bases = (mode == 0 ? staged : p->res).device<unsigned char>(np * bsz);
+  p->d_scalars = p->res.device<Fr>(np);
   const auto t0 = std::chrono::steady_clock::now();
   if (n_points) NZCP_CUDA(cudaMemcpyAsync(p->d_bases, bases, n_points * bsz, cudaMemcpyHostToDevice, p->st));
   try {
     if (mode == 0) {
       msm_table_create(&p->tab, p->d_bases, n_points, 0, p->g2, c, p->st);
       NZCP_CUDA(cudaStreamSynchronize(p->st));
-      cudaFree(p->d_bases);
+      staged = CudaResources();
       p->d_bases = nullptr;
     } else {
       msm_table_view(&p->tab, p->d_bases, n_points, p->g2, c);
@@ -163,9 +157,8 @@ int nzcp_msm_sum_partials(const void* d_partials, size_t count, int g2, int devi
     if (!d_partials || !out || count == 0 || count > (1u << 20)) throw ApiError(NZCP_E_ARG, "bad argument");
     use_device(device);
     const size_t psz = g2 ? sizeof(G2XYZZ) : sizeof(G1XYZZ);
-    void* d_res = nullptr;
-    NZCP_CUDA(cudaMalloc(&d_res, psz));
-    struct Guard { void* p; ~Guard() { cudaFree(p); } } gd{d_res};
+    CudaResources res;
+    void* d_res = res.device<unsigned char>(psz);
     msm_sum_points(d_partials, (uint32_t)count, g2 != 0, d_res, 0);
     alignas(16) unsigned char host[sizeof(G2XYZZ)];
     NZCP_CUDA(cudaMemcpy(host, d_res, psz, cudaMemcpyDeviceToHost));

@@ -464,30 +464,20 @@ void ntt_domain_create(NttDomain* d, int log_n, cudaStream_t st) {
       memcpy(pf.data() + tw_pad_off(j), &fwd[(size_t)j << (log_n - kLoTmaBits)], sizeof(Fr));
       memcpy(pi.data() + tw_pad_off(j), &inv[(size_t)j << (log_n - kLoTmaBits)], sizeof(Fr));
     }
-    NZCP_CUDA(cudaMalloc((void**)&d->tw_lo_fwd, kLoTwBytes));
-    NZCP_CUDA(cudaMalloc((void**)&d->tw_lo_inv, kLoTwBytes));
+    d->tw_lo_fwd = d->res.device<unsigned char>(kLoTwBytes);
+    d->tw_lo_inv = d->res.device<unsigned char>(kLoTwBytes);
     NZCP_CUDA(cudaMemcpy(d->tw_lo_fwd, pf.data(), kLoTwBytes, cudaMemcpyHostToDevice));
     NZCP_CUDA(cudaMemcpy(d->tw_lo_inv, pi.data(), kLoTwBytes, cudaMemcpyHostToDevice));
   }
-  NZCP_CUDA(cudaMalloc(&d->tw_fwd, (n / 2) * sizeof(Fr)));
-  NZCP_CUDA(cudaMalloc(&d->tw_inv, (n / 2) * sizeof(Fr)));
-  NZCP_CUDA(cudaMalloc(&d->coset_scale, n * sizeof(Fr)));
-  NZCP_CUDA(cudaMalloc(&d->ninv_scale, sizeof(Fr)));
+  d->tw_fwd = d->res.device<Fr>(n / 2);
+  d->tw_inv = d->res.device<Fr>(n / 2);
+  d->coset_scale = d->res.device<Fr>(n);
+  d->ninv_scale = d->res.device<Fr>(1);
   NZCP_CUDA(cudaMemcpyAsync(d->tw_fwd, fwd.data(), (n / 2) * sizeof(Fr), cudaMemcpyHostToDevice, st));
   NZCP_CUDA(cudaMemcpyAsync(d->tw_inv, inv.data(), (n / 2) * sizeof(Fr), cudaMemcpyHostToDevice, st));
   NZCP_CUDA(cudaMemcpyAsync(d->coset_scale, scale.data(), n * sizeof(Fr), cudaMemcpyHostToDevice, st));
   NZCP_CUDA(cudaMemcpyAsync(d->ninv_scale, &ninv, sizeof(Fr), cudaMemcpyHostToDevice, st));
   NZCP_CUDA(cudaStreamSynchronize(st));
-}
-
-void ntt_domain_destroy(NttDomain* d) {
-  cudaFree(d->tw_fwd);
-  cudaFree(d->tw_inv);
-  cudaFree(d->coset_scale);
-  cudaFree(d->ninv_scale);
-  cudaFree(d->tw_lo_fwd);
-  cudaFree(d->tw_lo_inv);
-  *d = NttDomain();
 }
 
 // Split bits [lo_bits, log_n) into hi passes of <= kMaxPassBits stages each.

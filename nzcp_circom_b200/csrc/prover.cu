@@ -45,6 +45,7 @@ struct nzcp_zkey {
   G1Affine alpha1, beta1, delta1;  // Montgomery affine, as stored
   G2Affine beta2, gamma2, delta2;
   R1csDevice r1cs;
+  CudaResources res;                             // the r1cs arrays
   int c_w = 0, c_h = 0;                          // MSM window bits for the witness MSMs / the H MSM
   MsmTable tab_a, tab_b1, tab_b2, tab_c, tab_h;  // window tables of sections 5-9 (tab_c front-padded to n_vars)
   NttDomain dom;
@@ -58,8 +59,7 @@ struct nzcp_prover {
   uint8_t* h_stage = nullptr;                   // pinned staging buffer for pageable host witnesses (n_vars * 32 B, lazy)
   cudaStream_t st_main = nullptr;
   cudaStream_t st_msm[4] = {nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t ev[20];
-  int n_ev = 0;
+  cudaEvent_t ev[20] = {};
   Fr* d_wtns = nullptr;
   Fr* d_abc = nullptr;
   Fr* d_h = nullptr;
@@ -67,6 +67,7 @@ struct nzcp_prover {
   MsmSort sort_b2;                              // the G2 MSM's own witness sort when its round count differs ("prover_rounds_b2")
   bool own_b2_sort = false;
   MsmRun run_a, run_b1, run_b2, run_c, run_h;
+  CudaResources res;                            // the streams, events, staging buffer and d_wtns / d_abc / d_h
 };
 
 namespace nzcp {
@@ -76,25 +77,13 @@ static void prover_release(nzcp_prover* p);
 static void zkey_release(nzcp_zkey* zk) {
   if (!zk) return;
   cudaSetDevice(zk->device);
-  for (nzcp_prover* p : zk->pool) prover_release(p);
-  zk->pool.clear();
-  cudaFree(zk->r1cs.row_ptr);
-  cudaFree(zk->r1cs.col);
-  cudaFree(zk->r1cs.val);
-  cudaFree(zk->r1cs.order);
-  msm_table_destroy(&zk->tab_a);
-  msm_table_destroy(&zk->tab_b1);
-  msm_table_destroy(&zk->tab_b2);
-  msm_table_destroy(&zk->tab_c);
-  msm_table_destroy(&zk->tab_h);
-  ntt_domain_destroy(&zk->dom);
+  for (nzcp_prover* p : zk->pool) prover_release(p);   // pooled provers use the key's tables: they go first
   delete zk;
 }
 
 template <class T>
-static T* upload(const void* src, size_t bytes, size_t* total) {
-  T* d = nullptr;
-  NZCP_CUDA(cudaMalloc(&d, bytes ? bytes : 16));
+static T* upload(CudaResources& res, const void* src, size_t bytes, size_t* total) {
+  T* d = reinterpret_cast<T*>(res.device<unsigned char>(bytes ? bytes : 16));
   if (bytes) NZCP_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
   *total += bytes;
   return d;
@@ -151,9 +140,9 @@ static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
   size_t tot = 0;
   zk->r1cs.n = n;
   zk->r1cs.nnz = nc;
-  zk->r1cs.row_ptr = upload<uint32_t>(row_ptr.data(), row_ptr.size() * 4, &tot);
-  zk->r1cs.col = upload<uint32_t>(col.data(), nc * 4, &tot);
-  zk->r1cs.val = upload<Fr>(val.data(), nc * 32, &tot);
+  zk->r1cs.row_ptr = upload<uint32_t>(zk->res, row_ptr.data(), row_ptr.size() * 4, &tot);
+  zk->r1cs.col = upload<uint32_t>(zk->res, col.data(), nc * 4, &tot);
+  zk->r1cs.val = upload<Fr>(zk->res, val.data(), nc * 32, &tot);
   // Constraint order for the evaluation kernel (one thread per constraint): inside every block of 128 consecutive
   // constraints the rows are handed to threads longest first, so the 32 lanes of a warp walk rows of similar length
   // (NZCP rows have 1..8 terms; unsorted, a warp runs as long as its longest row while the average is under 3).
@@ -173,22 +162,16 @@ static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
       for (int l = 63; l >= 0; l--) { start[l] = run; run += hist[l]; }   // counting sort, longest first, stable
       for (size_t j = 0; j < cnt; j++) order[b0 + start[key[j]]++] = (uint32_t)(b0 + j);
     }
-    zk->r1cs.order = upload<uint32_t>(order.data(), (size_t)n * 4, &tot);
+    zk->r1cs.order = upload<uint32_t>(zk->res, order.data(), (size_t)n * 4, &tot);
   }
   // sections 5-9 -> window tables (one-time expansion; the raw section is only staged)
   zk->c_w = g_tune_c_w.load() > 0 ? g_tune_c_w.load() : msm_pick_window(m);
   zk->c_h = g_tune_c_h.load() > 0 ? g_tune_c_h.load() : msm_pick_window(n);
   auto make_table = [&](MsmTable* t, const Sect& sec, size_t count, size_t pad, bool g2, int c) {
+    CudaResources staged;   // the raw section, freed as soon as its table is built
     size_t dummy = 0;
-    void* raw = upload<unsigned char>(sec.p, sec.len, &dummy);
-    try {
-      msm_table_create(t, raw, count, pad, g2, c, 0);
-      NZCP_CUDA(cudaDeviceSynchronize());
-    } catch (...) {
-      cudaFree(raw);
-      throw;
-    }
-    cudaFree(raw);
+    msm_table_create(t, upload<unsigned char>(staged, sec.p, sec.len, &dummy), count, pad, g2, c, 0);
+    NZCP_CUDA(cudaDeviceSynchronize());
     tot += t->bytes;
   };
   make_table(&zk->tab_a, s[5], m, 0, false, zk->c_w);
@@ -205,22 +188,6 @@ static nzcp_zkey* zkey_load_impl(const uint8_t* b, size_t len, int device) {
 static void prover_release(nzcp_prover* p) {
   if (!p) return;
   cudaSetDevice(p->device);
-  if (p->h_stage) cudaFreeHost(p->h_stage);
-  if (p->st_main) cudaStreamDestroy(p->st_main);
-  for (int i = 0; i < 4; i++)
-    if (p->st_msm[i]) cudaStreamDestroy(p->st_msm[i]);
-  for (int i = 0; i < p->n_ev; i++) cudaEventDestroy(p->ev[i]);
-  cudaFree(p->d_wtns);
-  cudaFree(p->d_abc);
-  cudaFree(p->d_h);
-  msm_run_destroy(&p->run_a);
-  msm_run_destroy(&p->run_b1);
-  msm_run_destroy(&p->run_b2);
-  msm_run_destroy(&p->run_c);
-  msm_run_destroy(&p->run_h);
-  msm_sort_destroy(&p->sort_w);
-  msm_sort_destroy(&p->sort_b2);
-  msm_sort_destroy(&p->sort_h);
   delete p;
 }
 
@@ -234,16 +201,13 @@ static nzcp_prover* prover_create_impl(nzcp_zkey* zk, int mode = 0) {
   std::unique_ptr<nzcp_prover, void (*)(nzcp_prover*)> p(new nzcp_prover(), prover_release);
   p->zk = zk;
   p->device = zk->device;
-  NZCP_CUDA(cudaStreamCreateWithFlags(&p->st_main, cudaStreamNonBlocking));
-  for (int i = 0; i < 4; i++) NZCP_CUDA(cudaStreamCreateWithFlags(&p->st_msm[i], cudaStreamNonBlocking));
-  for (int i = 0; i < 20; i++) {
-    NZCP_CUDA(cudaEventCreate(&p->ev[i]));
-    p->n_ev = i + 1;
-  }
+  p->st_main = p->res.stream();
+  for (auto& st : p->st_msm) st = p->res.stream();
+  for (auto& ev : p->ev) ev = p->res.event();
   size_t n = zk->domain_size;
-  NZCP_CUDA(cudaMalloc(&p->d_wtns, (size_t)zk->n_vars * sizeof(Fr)));
-  NZCP_CUDA(cudaMalloc(&p->d_abc, 3 * n * sizeof(Fr)));
-  NZCP_CUDA(cudaMalloc(&p->d_h, n * sizeof(Fr)));
+  p->d_wtns = p->res.device<Fr>(zk->n_vars);
+  p->d_abc = p->res.device<Fr>(3 * n);
+  p->d_h = p->res.device<Fr>(n);
   int rounds_h = g_tune_rounds_h.load(), rounds_w = g_tune_rounds_w.load();
   (void)mode;
   if (rounds_h < 0) rounds_h = msm_pick_rounds_prover(n, zk->c_h);
@@ -302,7 +266,7 @@ static void upload_witness(nzcp_prover* p, const uint8_t* h_witness, size_t byte
     NZCP_CUDA(cudaMemcpyAsync(p->d_wtns, h_witness, bytes, cudaMemcpyHostToDevice, st));
     return;
   }
-  if (!p->h_stage) NZCP_CUDA(cudaHostAlloc((void**)&p->h_stage, (size_t)p->zk->n_vars * sizeof(Fr), cudaHostAllocDefault));
+  if (!p->h_stage) p->h_stage = p->res.pinned<uint8_t>((size_t)p->zk->n_vars * sizeof(Fr));
   size_t chunk = (size_t)g_tune_stage_chunk_kb.load() * 1024;
   if (chunk < 65536) chunk = 65536;
   // A single core copies ~10 GB/s: 2.8 ms for the 28 MB NZCP witness, a quarter of the whole proof.  The copy is shared by

@@ -25,7 +25,6 @@
 //          2^(s+1) whatever the level, so one table w_top^(-k), k < 2^power, serves every level of every section.
 // Sections are computed one after the other (their times are reported apart); all of them are validated on the host
 // first: container, sizes, canonical coordinates and curve membership of every input point.
-#include <memory>
 
 #include "binfile.cuh"
 
@@ -170,39 +169,28 @@ std::vector<Fr> ninv_table(uint32_t top) {
   return t;
 }
 
-struct DevMem {
-  void* p = nullptr;
-  explicit DevMem(size_t bytes) { NZCP_CUDA(cudaMalloc(&p, bytes ? bytes : 16)); }
-  ~DevMem() { cudaFree(p); }
-  template <class T> T* as() { return reinterpret_cast<T*>(p); }
-};
-
 template <class F>
 float run_section_device(const uint8_t* src, uint64_t n_src, uint32_t top, const Fr* d_ninv, const Fr* d_tw, int t_log,
                          uint8_t* out) {
   const uint64_t n = level_points(top);
-  DevMem d_src(n_src * sizeof(Affine<F>)), d_x(n * sizeof(Affine<F>));
-  NZCP_CUDA(cudaMemcpy(d_src.p, src, n_src * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-  cudaEvent_t e0, e1;
-  NZCP_CUDA(cudaEventCreate(&e0));
-  if (cudaEventCreate(&e1) != cudaSuccess) {
-    cudaEventDestroy(e0);
-    throw CudaError("cudaEventCreate failed");
-  }
-  struct Ev { cudaEvent_t a, b; ~Ev() { cudaEventDestroy(a); cudaEventDestroy(b); } } ev{e0, e1};
+  CudaResources res;
+  Affine<F>* d_src = res.device<Affine<F>>(n_src);   // n_src, n > 0
+  Affine<F>* d_x = res.device<Affine<F>>(n);
+  NZCP_CUDA(cudaMemcpy(d_src, src, n_src * sizeof(Affine<F>), cudaMemcpyHostToDevice));
+  const cudaEvent_t e0 = res.event(), e1 = res.event();
   NZCP_CUDA(cudaEventRecord(e0, 0));
-  ptau_load_kernel<F><<<div_up(n, 128), 128>>>(d_src.as<Affine<F>>(), n_src, d_ninv, d_x.as<Affine<F>>(), n);
+  ptau_load_kernel<F><<<div_up(n, 128), 128>>>(d_src, n_src, d_ninv, d_x, n);
   NZCP_LAUNCH_CHECK();
   for (uint32_t s = 0; s < top; s++) {
     const uint64_t nb = ((uint64_t)1 << top) - ((uint64_t)1 << s);
-    ptau_stage_kernel<F><<<div_up(nb, 128), 128>>>(d_x.as<Affine<F>>(), d_tw, t_log, (int)s, nb);
+    ptau_stage_kernel<F><<<div_up(nb, 128), 128>>>(d_x, d_tw, t_log, (int)s, nb);
     NZCP_LAUNCH_CHECK();
   }
   NZCP_CUDA(cudaEventRecord(e1, 0));
   NZCP_CUDA(cudaEventSynchronize(e1));
   float ms = 0;
   NZCP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  NZCP_CUDA(cudaMemcpy(out, d_x.p, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
+  NZCP_CUDA(cudaMemcpy(out, d_x, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
   return ms;
 }
 
@@ -234,15 +222,16 @@ void prepare_impl(const uint8_t* b, size_t len, int device, uint8_t* out, size_t
   const Fr w_inv = fp_inv(host_fr_root(t_log));
   const std::vector<Fr> ninv = ninv_table(p.power + 1);
   std::vector<Fr> tw;
-  std::unique_ptr<DevMem> d_tw, d_ninv;
+  CudaResources res;
+  Fr *d_tw = nullptr, *d_ninv = nullptr;
   if (host) {
     tw.resize(n_tw);
     for (uint64_t k = 0; k < n_tw; k++) tw[k] = pow_u32_plain(w_inv, (uint32_t)k);
   } else {
-    d_tw.reset(new DevMem(n_tw * sizeof(Fr)));
-    d_ninv.reset(new DevMem(ninv.size() * sizeof(Fr)));
-    NZCP_CUDA(cudaMemcpy(d_ninv->p, ninv.data(), ninv.size() * sizeof(Fr), cudaMemcpyHostToDevice));
-    ptau_twiddle_kernel<<<div_up(n_tw, 256), 256>>>(d_tw->as<Fr>(), w_inv, n_tw);
+    d_tw = res.device<Fr>(n_tw);
+    d_ninv = res.device<Fr>(ninv.size());
+    NZCP_CUDA(cudaMemcpy(d_ninv, ninv.data(), ninv.size() * sizeof(Fr), cudaMemcpyHostToDevice));
+    ptau_twiddle_kernel<<<div_up(n_tw, 256), 256>>>(d_tw, w_inv, n_tw);
     NZCP_LAUNCH_CHECK();
   }
 
@@ -264,8 +253,8 @@ void prepare_impl(const uint8_t* b, size_t len, int device, uint8_t* out, size_t
       if (o.g2) run_section_host<Fq2>(p.s[o.src].p, n_src, o.top, ninv.data(), tw.data(), t_log, dst);
       else run_section_host<Fq>(p.s[o.src].p, n_src, o.top, ninv.data(), tw.data(), t_log, dst);
     } else {
-      if (o.g2) ms = run_section_device<Fq2>(p.s[o.src].p, n_src, o.top, d_ninv->as<Fr>(), d_tw->as<Fr>(), t_log, dst);
-      else ms = run_section_device<Fq>(p.s[o.src].p, n_src, o.top, d_ninv->as<Fr>(), d_tw->as<Fr>(), t_log, dst);
+      if (o.g2) ms = run_section_device<Fq2>(p.s[o.src].p, n_src, o.top, d_ninv, d_tw, t_log, dst);
+      else ms = run_section_device<Fq>(p.s[o.src].p, n_src, o.top, d_ninv, d_tw, t_log, dst);
     }
     if (section_ms) section_ms[k] = ms;
   }

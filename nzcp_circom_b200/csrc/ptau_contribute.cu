@@ -193,16 +193,17 @@ void key_section_host(uint8_t* x, uint64_t n, const Fr& first, const Fr& inc) {
 template <class F>
 float key_section_device(const uint8_t* src, uint64_t n, const Fr& first, const Fr& inc, Affine<F>* d_x, Hasher& resp,
                          uint8_t* dst) {
-  Events ev;
+  CudaResources res;
+  const cudaEvent_t e0 = res.event(), e1 = res.event();
   NZCP_CUDA(cudaMemcpy(d_x, src, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-  NZCP_CUDA(cudaEventRecord(ev.a, 0));
+  NZCP_CUDA(cudaEventRecord(e0, 0));
   ptau_key_kernel<F><<<div_up(n, 128), 128>>>(d_x, first, inc, n);
   NZCP_LAUNCH_CHECK();
-  NZCP_CUDA(cudaEventRecord(ev.b, 0));
+  NZCP_CUDA(cudaEventRecord(e1, 0));
   resp.points_device(d_x, n);
   NZCP_CUDA(cudaMemcpy(dst, d_x, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
   float ms = 0;
-  NZCP_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
+  NZCP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
   return ms;
 }
 
@@ -236,8 +237,8 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
   write_ptau_header(w, p.power, 7);
   Hasher resp(host, Enc::C);
   resp.update(challenge, 64);
-  std::unique_ptr<DevMem> d_buf;
-  if (!host) d_buf.reset(new DevMem(sect_bytes(p.power, 3)));   // the largest section: 2^p G2 points
+  CudaResources res;
+  void* d_buf = host ? nullptr : res.device<unsigned char>(sect_bytes(p.power, 3));   // the largest section: 2^p G2 points
   uint8_t* sect[7] = {};
   for (int id = 2; id <= 6; id++) {
     const uint64_t n = sect_points(p.power, id);
@@ -253,9 +254,9 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
         resp.points_host(reinterpret_cast<const G1Affine*>(sect[id]), n);
       }
     } else if (sect_g2(id)) {
-      ms[id - 2] = key_section_device(p.s[id].p, n, *first[id], tau, static_cast<G2Affine*>(d_buf->p), resp, sect[id]);
+      ms[id - 2] = key_section_device(p.s[id].p, n, *first[id], tau, static_cast<G2Affine*>(d_buf), resp, sect[id]);
     } else {
-      ms[id - 2] = key_section_device(p.s[id].p, n, *first[id], tau, static_cast<G1Affine*>(d_buf->p), resp, sect[id]);
+      ms[id - 2] = key_section_device(p.s[id].p, n, *first[id], tau, static_cast<G1Affine*>(d_buf), resp, sect[id]);
     }
   }
   uint8_t partial[kPartialLen], pk[kPubKeyLen], response[64];
@@ -273,9 +274,9 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
       if (sect_g2(id)) nx.points_host(reinterpret_cast<const G2Affine*>(sect[id]), n);
       else nx.points_host(reinterpret_cast<const G1Affine*>(sect[id]), n);
     } else {
-      NZCP_CUDA(cudaMemcpy(d_buf->p, sect[id], p.s[id].len, cudaMemcpyHostToDevice));
-      if (sect_g2(id)) nx.points_device(static_cast<const G2Affine*>(d_buf->p), n);
-      else nx.points_device(static_cast<const G1Affine*>(d_buf->p), n);
+      NZCP_CUDA(cudaMemcpy(d_buf, sect[id], p.s[id].len, cudaMemcpyHostToDevice));
+      if (sect_g2(id)) nx.points_device(static_cast<const G2Affine*>(d_buf), n);
+      else nx.points_device(static_cast<const G1Affine*>(d_buf), n);
     }
   }
   uint8_t next[64];

@@ -34,12 +34,9 @@ static void check_section(const uint8_t* host, size_t n_points, const F& b, uint
   *infinity = 0;
   if (!n_points) return;
   const size_t bytes = n_points * sizeof(Affine<F>);
-  void* d = nullptr;
-  unsigned long long* d_counts = nullptr;
-  NZCP_CUDA(cudaMalloc(&d, bytes));
-  struct Guard { void* a; void* b; ~Guard() { cudaFree(a); cudaFree(b); } } gd{d, nullptr};
-  NZCP_CUDA(cudaMalloc((void**)&d_counts, 2 * sizeof(unsigned long long)));
-  gd.b = d_counts;
+  CudaResources res;
+  void* d = res.device<unsigned char>(bytes);
+  unsigned long long* d_counts = res.device<unsigned long long>(2);
   NZCP_CUDA(cudaMemset(d_counts, 0, 2 * sizeof(unsigned long long)));
   NZCP_CUDA(cudaMemcpy(d, host, bytes, cudaMemcpyHostToDevice));
   curve_check_kernel<F><<<div_up(n_points, 128), 128>>>(reinterpret_cast<const Affine<F>*>(d), n_points, b, d_counts);

@@ -125,14 +125,10 @@ namespace {
 template <class F>
 void run_combo(const Combo& cb, const Fr* d_coefs, const void* d_src0, const void* d_src1, const void* d_src2, uint32_t n_wires,
                uint8_t* host_out) {
-  uint32_t* d_rp = nullptr;
-  Term* d_terms = nullptr;
-  Affine<F>* d_out = nullptr;
-  struct Guard { void** a; void** b; void** c; ~Guard() { cudaFree(*a); cudaFree(*b); cudaFree(*c); } }
-      gd{(void**)&d_rp, (void**)&d_terms, (void**)&d_out};
-  NZCP_CUDA(cudaMalloc((void**)&d_rp, cb.row_ptr.size() * 4));
-  NZCP_CUDA(cudaMalloc((void**)&d_terms, (cb.terms.size() ? cb.terms.size() : 1) * sizeof(Term)));
-  NZCP_CUDA(cudaMalloc((void**)&d_out, (size_t)(n_wires ? n_wires : 1) * sizeof(Affine<F>)));
+  CudaResources res;
+  uint32_t* d_rp = res.device<uint32_t>(cb.row_ptr.size());
+  Term* d_terms = res.device<Term>(cb.terms.size() ? cb.terms.size() : 1);
+  Affine<F>* d_out = res.device<Affine<F>>(n_wires ? n_wires : 1);
   NZCP_CUDA(cudaMemcpy(d_rp, cb.row_ptr.data(), cb.row_ptr.size() * 4, cudaMemcpyHostToDevice));
   if (!cb.terms.empty()) NZCP_CUDA(cudaMemcpy(d_terms, cb.terms.data(), cb.terms.size() * sizeof(Term), cudaMemcpyHostToDevice));
   if (n_wires) {
@@ -224,22 +220,17 @@ void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b
 
   // ---- device: the four Lagrange levels of size n, the coefficient pool
   const uint64_t lvl = n - 1;   // points before level cir_power in a Lagrange section
+  CudaResources res;
   auto up = [&](const uint8_t* src, size_t bytes) {
-    void* d = nullptr;
-    NZCP_CUDA(cudaMalloc(&d, bytes));
-    if (cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice) != cudaSuccess) {
-      cudaFree(d);
-      throw CudaError("cudaMemcpy of a ptau section failed");
-    }
+    void* d = res.device<unsigned char>(bytes);
+    NZCP_CUDA(cudaMemcpy(d, src, bytes, cudaMemcpyHostToDevice));
     return d;
   };
-  struct Dev { void* p = nullptr; ~Dev() { cudaFree(p); } } d_tau1, d_tau2, d_alpha, d_beta, d_pool;
-  d_tau1.p = up(pt.s[12].p + lvl * 64, n * 64);
-  d_tau2.p = up(pt.s[13].p + lvl * 128, n * 128);
-  d_alpha.p = up(pt.s[14].p + lvl * 64, n * 64);
-  d_beta.p = up(pt.s[15].p + lvl * 64, n * 64);
-  d_pool.p = up(reinterpret_cast<const uint8_t*>(pool.data()), pool.size() * sizeof(Fr));
-  const Fr* d_coefs = reinterpret_cast<const Fr*>(d_pool.p);
+  void* d_tau1 = up(pt.s[12].p + lvl * 64, n * 64);
+  void* d_tau2 = up(pt.s[13].p + lvl * 128, n * 128);
+  void* d_alpha = up(pt.s[14].p + lvl * 64, n * 64);
+  void* d_beta = up(pt.s[15].p + lvl * 64, n * 64);
+  const Fr* d_coefs = static_cast<const Fr*>(up(reinterpret_cast<const uint8_t*>(pool.data()), pool.size() * sizeof(Fr)));
 
   // ---- write the file in zkey_new.js's order
   Writer w(out, cap);
@@ -278,7 +269,7 @@ void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b
   }
   // K = beta*A + alpha*B + C per wire -> IC (section 3) and C (section 8)
   std::vector<uint8_t> kbuf((size_t)m * 64);
-  run_combo<Fq>(K, d_coefs, d_tau1.p, d_alpha.p, d_beta.p, m, kbuf.data());
+  run_combo<Fq>(K, d_coefs, d_tau1, d_alpha, d_beta, m, kbuf.data());
   w.section(3, (uint64_t)(np + 1) * 64);
   w.raw(kbuf.data(), (size_t)(np + 1) * 64);
   // section 9: odd entries of the size-2n Lagrange level of tauG1
@@ -291,11 +282,11 @@ void zkey_new_impl(const uint8_t* r1cs_b, size_t r1cs_len, const uint8_t* ptau_b
   w.section(8, (uint64_t)(m - np - 1) * 64);
   w.raw(kbuf.data() + (size_t)(np + 1) * 64, (size_t)(m - np - 1) * 64);
   w.section(5, (uint64_t)m * 64);
-  run_combo<Fq>(A, d_coefs, d_tau1.p, nullptr, nullptr, m, w.reserve((size_t)m * 64));
+  run_combo<Fq>(A, d_coefs, d_tau1, nullptr, nullptr, m, w.reserve((size_t)m * 64));
   w.section(6, (uint64_t)m * 64);
-  run_combo<Fq>(B, d_coefs, d_tau1.p, nullptr, nullptr, m, w.reserve((size_t)m * 64));
+  run_combo<Fq>(B, d_coefs, d_tau1, nullptr, nullptr, m, w.reserve((size_t)m * 64));
   w.section(7, (uint64_t)m * 128);
-  run_combo<Fq2>(B, d_coefs, d_tau2.p, nullptr, nullptr, m, w.reserve((size_t)m * 128));
+  run_combo<Fq2>(B, d_coefs, d_tau2, nullptr, nullptr, m, w.reserve((size_t)m * 128));
   w.section(10, 68);
   w.zeros(64);                                               // csHash: not computed (see the header of this file)
   w.u32(0);                                                  // no contributions

@@ -13,31 +13,17 @@ extern std::atomic<int> g_tune_pair_stage;
 extern std::atomic<int> g_tune_pair_k[kMsmMaxRounds];
 extern std::atomic<int> g_tune_rounds_w, g_tune_rounds_h;
 
-struct DevBuf {
-  void* p = nullptr;
-  explicit DevBuf(size_t bytes) { NZCP_CUDA(cudaMalloc(&p, bytes ? bytes : 16)); }
-  ~DevBuf() { cudaFree(p); }
-  template <class T> T* as() { return reinterpret_cast<T*>(p); }
-};
-
-struct Timer {
-  cudaEvent_t a, b;
+struct Timer {   // device time on stream st from construction to stop()
+  CudaResources res;
+  cudaEvent_t a = res.event(), b = res.event();
   cudaStream_t st;
-  explicit Timer(cudaStream_t s) : st(s) {
-    NZCP_CUDA(cudaEventCreate(&a));
-    NZCP_CUDA(cudaEventCreate(&b));
-    NZCP_CUDA(cudaEventRecord(a, st));
-  }
+  explicit Timer(cudaStream_t s) : st(s) { NZCP_CUDA(cudaEventRecord(a, st)); }
   float stop() {
     float ms = 0;
     NZCP_CUDA(cudaEventRecord(b, st));
     NZCP_CUDA(cudaEventSynchronize(b));
     NZCP_CUDA(cudaEventElapsedTime(&ms, a, b));
     return ms;
-  }
-  ~Timer() {
-    cudaEventDestroy(a);
-    cudaEventDestroy(b);
   }
 };
 
@@ -131,12 +117,15 @@ template <class F>
 static void run_xyzz_op(int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n) {
   const size_t xs = sizeof(XYZZ<F>), as = sizeof(Affine<F>);
   const size_t bs = op == 0 ? xs : (op <= 2 ? as : 0), os = op == 4 ? as : xs;
-  DevBuf da(n * xs), db(n * bs), dout(n * os);
-  NZCP_CUDA(cudaMemcpy(da.p, a, n * xs, cudaMemcpyHostToDevice));
-  if (bs) NZCP_CUDA(cudaMemcpy(db.p, b, n * bs, cudaMemcpyHostToDevice));
-  xyzz_op_kernel<F><<<div_up(n, 128), 128>>>(op, da.as<XYZZ<F>>(), db.p, dout.p, n);
+  CudaResources res;
+  XYZZ<F>* da = res.device<XYZZ<F>>(n);   // n > 0
+  void* db = res.device<unsigned char>(bs ? n * bs : 16);
+  void* dout = res.device<unsigned char>(n * os);
+  NZCP_CUDA(cudaMemcpy(da, a, n * xs, cudaMemcpyHostToDevice));
+  if (bs) NZCP_CUDA(cudaMemcpy(db, b, n * bs, cudaMemcpyHostToDevice));
+  xyzz_op_kernel<F><<<div_up(n, 128), 128>>>(op, da, db, dout, n);
   NZCP_LAUNCH_CHECK();
-  NZCP_CUDA(cudaMemcpy(out, dout.p, n * os, cudaMemcpyDeviceToHost));
+  NZCP_CUDA(cudaMemcpy(out, dout, n * os, cudaMemcpyDeviceToHost));
 }
 
 template <class P>
@@ -170,15 +159,18 @@ static uint32_t selftest_field(uint64_t seed, uint32_t n) {
     a[6] = a[5]; b[6] = Fp<P>::zero();
     a[7] = Fp<P>::zero(); b[7] = a[5];
   }
-  DevBuf da(n * 32), db(n * 32), dout(n * 32);
-  NZCP_CUDA(cudaMemcpy(da.p, a.data(), n * 32, cudaMemcpyHostToDevice));
-  NZCP_CUDA(cudaMemcpy(db.p, b.data(), n * 32, cudaMemcpyHostToDevice));
+  CudaResources res;
+  Fp<P>* da = res.device<Fp<P>>(n);   // n > 0
+  Fp<P>* db = res.device<Fp<P>>(n);
+  Fp<P>* dout = res.device<Fp<P>>(n);
+  NZCP_CUDA(cudaMemcpy(da, a.data(), n * 32, cudaMemcpyHostToDevice));
+  NZCP_CUDA(cudaMemcpy(db, b.data(), n * 32, cudaMemcpyHostToDevice));
   uint32_t bad = 0;
   std::vector<Fp<P>> out(n);
   for (int op = 0; op < 6; op++) {
-    field_op_kernel<P><<<div_up(n, 128), 128>>>(op, da.as<Fp<P>>(), db.as<Fp<P>>(), dout.as<Fp<P>>(), n);
+    field_op_kernel<P><<<div_up(n, 128), 128>>>(op, da, db, dout, n);
     NZCP_LAUNCH_CHECK();
-    NZCP_CUDA(cudaMemcpy(out.data(), dout.p, n * 32, cudaMemcpyDeviceToHost));
+    NZCP_CUDA(cudaMemcpy(out.data(), dout, n * 32, cudaMemcpyDeviceToHost));
     for (uint32_t i = 0; i < n; i++) {
       Fp<P> e = (op % 3 == 0) ? fp_mul_portable(a[i], b[i]) : (op % 3 == 1) ? fp_add_portable(a[i], b[i]) : fp_sub_portable(a[i], b[i]);
       if (e != out[i]) bad++;
@@ -203,12 +195,15 @@ static uint32_t selftest_curve(const Affine<F>& gen, uint64_t seed, uint32_t n) 
     b[0] = a[0];                                   // madd hits the doubling branch
     b[1] = Affine<F>{a[1].x, f_neg(a[1].y)};       // madd hits the cancellation branch
   }
-  DevBuf da(n * sizeof(Affine<F>)), db(n * sizeof(Affine<F>)), dout(n * sizeof(Affine<F>));
-  NZCP_CUDA(cudaMemcpy(da.p, a.data(), n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-  NZCP_CUDA(cudaMemcpy(db.p, b.data(), n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-  curve_op_kernel<F><<<div_up(n, 64), 64>>>(da.as<Affine<F>>(), db.as<Affine<F>>(), dout.as<Affine<F>>(), n);
+  CudaResources res;
+  Affine<F>* da = res.device<Affine<F>>(n);   // n > 0
+  Affine<F>* db = res.device<Affine<F>>(n);
+  Affine<F>* dout = res.device<Affine<F>>(n);
+  NZCP_CUDA(cudaMemcpy(da, a.data(), n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
+  NZCP_CUDA(cudaMemcpy(db, b.data(), n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
+  curve_op_kernel<F><<<div_up(n, 64), 64>>>(da, db, dout, n);
   NZCP_LAUNCH_CHECK();
-  NZCP_CUDA(cudaMemcpy(out.data(), dout.p, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
+  NZCP_CUDA(cudaMemcpy(out.data(), dout, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
   uint32_t bad = 0;
   for (uint32_t i = 0; i < n; i++) {
     XYZZ<F> e = XYZZ<F>::from_affine(a[i]);
@@ -544,14 +539,15 @@ int nzcp_intpipe_modes(int device, int iters, double out[10]) {
     use_device(device);
     cudaDeviceProp prop;
     NZCP_CUDA(cudaGetDeviceProperties(&prop, device));
-    DevBuf sink(64);
+    CudaResources res;
+    uint32_t* sink = res.device<uint32_t>(16);
     const int blocks = prop.multiProcessorCount * 8, threads = 256;
     for (int mode = 0; mode < 9; mode++) {
       int it = mode == 2 ? (iters / 16 > 0 ? iters / 16 : 1) : iters;
       float best = 1e30f;
       for (int rep = 0; rep < 4; rep++) {
         Timer t(0);
-        launch_intpipe(mode, blocks, threads, it, 12345u + rep, sink.as<uint32_t>());
+        launch_intpipe(mode, blocks, threads, it, 12345u + rep, sink);
         NZCP_LAUNCH_CHECK();
         float ms = t.stop();
         if (rep && ms < best) best = ms;
@@ -572,17 +568,18 @@ int nzcp_pipe_probe(int device, int iters, double out[5]) {
     use_device(device);
     cudaDeviceProp prop;
     NZCP_CUDA(cudaGetDeviceProperties(&prop, device));
-    DevBuf sink(64);
+    CudaResources res;
+    uint32_t* sink = res.device<uint32_t>(16);
     const int blocks = prop.multiProcessorCount * 8, threads = 256;
     for (int mode = 0; mode < 4; mode++) {
       float best = 1e30f;
       for (int rep = 0; rep < 4; rep++) {
         Timer t(0);
         switch (mode) {
-          case 0: pipeprobe_kernel<0><<<blocks, threads>>>(iters, 777u + rep, sink.as<uint32_t>()); break;
-          case 1: pipeprobe_kernel<1><<<blocks, threads>>>(iters, 777u + rep, sink.as<uint32_t>()); break;
-          case 2: pipeprobe_kernel<2><<<blocks, threads>>>(iters, 777u + rep, sink.as<uint32_t>()); break;
-          default: pipeprobe_kernel<3><<<blocks, threads>>>(iters, 777u + rep, sink.as<uint32_t>()); break;
+          case 0: pipeprobe_kernel<0><<<blocks, threads>>>(iters, 777u + rep, sink); break;
+          case 1: pipeprobe_kernel<1><<<blocks, threads>>>(iters, 777u + rep, sink); break;
+          case 2: pipeprobe_kernel<2><<<blocks, threads>>>(iters, 777u + rep, sink); break;
+          default: pipeprobe_kernel<3><<<blocks, threads>>>(iters, 777u + rep, sink); break;
         }
         NZCP_LAUNCH_CHECK();
         float ms = t.stop();
@@ -617,14 +614,15 @@ int nzcp_ntt(uint8_t* data, int log_n, int inverse, int device, float* kernel_ms
     size_t n = (size_t)1 << log_n;
     NttDomain dom;
     ntt_domain_create(&dom, log_n, 0);
-    struct Guard { NttDomain* d; ~Guard() { ntt_domain_destroy(d); } } g{&dom};
-    DevBuf d(n * 32), tmp(n * 32);
-    NZCP_CUDA(cudaMemcpy(d.p, data, n * 32, cudaMemcpyHostToDevice));
+    CudaResources res;
+    Fr* d = res.device<Fr>(n);
+    Fr* tmp = res.device<Fr>(n);
+    NZCP_CUDA(cudaMemcpy(d, data, n * 32, cudaMemcpyHostToDevice));
     Timer t(0);
-    if (inverse) ntt_inverse(dom, d.as<Fr>(), tmp.as<Fr>(), 0); else ntt_forward(dom, d.as<Fr>(), tmp.as<Fr>(), 0);
+    if (inverse) ntt_inverse(dom, d, tmp, 0); else ntt_forward(dom, d, tmp, 0);
     float ms = t.stop();
     if (kernel_ms) *kernel_ms = ms;
-    NZCP_CUDA(cudaMemcpy(data, d.p, n * 32, cudaMemcpyDeviceToHost));
+    NZCP_CUDA(cudaMemcpy(data, d, n * 32, cudaMemcpyDeviceToHost));
   });
 }
 
@@ -636,14 +634,14 @@ int nzcp_ntt_coset(uint8_t* data, int log_n, int batch, int device, float* kerne
     size_t n = (size_t)1 << log_n;
     NttDomain dom;
     ntt_domain_create(&dom, log_n, 0);
-    struct Guard { NttDomain* d; ~Guard() { ntt_domain_destroy(d); } } g{&dom};
-    DevBuf d(n * 32 * batch);
-    NZCP_CUDA(cudaMemcpy(d.p, data, n * 32 * batch, cudaMemcpyHostToDevice));
+    CudaResources res;
+    Fr* d = res.device<Fr>(n * batch);
+    NZCP_CUDA(cudaMemcpy(d, data, n * 32 * batch, cudaMemcpyHostToDevice));
     Timer t(0);
-    ntt_coset_pipeline(dom, d.as<Fr>(), batch, 0);
+    ntt_coset_pipeline(dom, d, batch, 0);
     float ms = t.stop();
     if (kernel_ms) *kernel_ms = ms;
-    NZCP_CUDA(cudaMemcpy(data, d.p, n * 32 * batch, cudaMemcpyDeviceToHost));
+    NZCP_CUDA(cudaMemcpy(data, d, n * 32 * batch, cudaMemcpyDeviceToHost));
   });
 }
 
@@ -654,25 +652,23 @@ int nzcp_msm(const uint8_t* bases, const uint8_t* scalars, size_t n_points, int 
     use_device(device);
     size_t bsz = g2 ? 128 : 64;
     int c = window_bits > 0 ? window_bits : msm_pick_window(n_points ? n_points : 1);
-    DevBuf db(n_points * bsz), ds(n_points * 32);
+    CudaResources res;
+    void* db = res.device<unsigned char>(n_points ? n_points * bsz : 16);
+    Fr* ds = reinterpret_cast<Fr*>(res.device<unsigned char>(n_points ? n_points * 32 : 16));
     if (n_points) {
-      NZCP_CUDA(cudaMemcpy(db.p, bases, n_points * bsz, cudaMemcpyHostToDevice));
-      NZCP_CUDA(cudaMemcpy(ds.p, scalars, n_points * 32, cudaMemcpyHostToDevice));
+      NZCP_CUDA(cudaMemcpy(db, bases, n_points * bsz, cudaMemcpyHostToDevice));
+      NZCP_CUDA(cudaMemcpy(ds, scalars, n_points * 32, cudaMemcpyHostToDevice));
     }
     MsmTable tab;
     MsmSort sort;
     MsmRun run;
-    struct Guard {
-      MsmTable* t; MsmSort* s; MsmRun* r;
-      ~Guard() { msm_run_destroy(r); msm_sort_destroy(s); msm_table_destroy(t); }
-    } gd{&tab, &sort, &run};
     // one-time per base set (the prover does this at zkey load); not part of kernel_ms
-    msm_table_create(&tab, db.p, n_points, 0, g2 != 0, c, 0);
+    msm_table_create(&tab, db, n_points, 0, g2 != 0, c, 0);
     msm_sort_create(&sort, n_points, c);
     msm_run_create(&run, &sort, g2 != 0);
     NZCP_CUDA(cudaDeviceSynchronize());
     Timer t(0);
-    msm_sort_launch(&sort, ds.as<Fr>(), n_points, 0);
+    msm_sort_launch(&sort, ds, n_points, 0);
     msm_run_launch(&run, &sort, &tab, 0);
     float ms = t.stop();
     NZCP_CUDA(cudaDeviceSynchronize());
@@ -705,15 +701,17 @@ int nzcp_field_op(int field, int op, const uint8_t* a, const uint8_t* b, uint8_t
     if (!a || !b || !out) throw ApiError(NZCP_E_ARG, "null argument");
     if (op < 0 || op > 7 || field < 0 || field > 1) throw ApiError(NZCP_E_ARG, "bad op/field");
     use_device(device);
-    DevBuf da(n * 32), db(n * 32), dout(n * 32);
-    NZCP_CUDA(cudaMemcpy(da.p, a, n * 32, cudaMemcpyHostToDevice));
-    NZCP_CUDA(cudaMemcpy(db.p, b, n * 32, cudaMemcpyHostToDevice));
+    CudaResources res;
+    const size_t bytes = n ? n * 32 : 16;
+    void *da = res.device<unsigned char>(bytes), *db = res.device<unsigned char>(bytes), *dout = res.device<unsigned char>(bytes);
+    NZCP_CUDA(cudaMemcpy(da, a, n * 32, cudaMemcpyHostToDevice));
+    NZCP_CUDA(cudaMemcpy(db, b, n * 32, cudaMemcpyHostToDevice));
     if (field == 0)
-      field_op_kernel<FrParams><<<div_up(n, 128), 128>>>(op, da.as<Fr>(), db.as<Fr>(), dout.as<Fr>(), n);
+      field_op_kernel<FrParams><<<div_up(n, 128), 128>>>(op, (Fr*)da, (Fr*)db, (Fr*)dout, n);
     else
-      field_op_kernel<FqParams><<<div_up(n, 128), 128>>>(op, da.as<Fq>(), db.as<Fq>(), dout.as<Fq>(), n);
+      field_op_kernel<FqParams><<<div_up(n, 128), 128>>>(op, (Fq*)da, (Fq*)db, (Fq*)dout, n);
     NZCP_LAUNCH_CHECK();
-    NZCP_CUDA(cudaMemcpy(out, dout.p, n * 32, cudaMemcpyDeviceToHost));
+    NZCP_CUDA(cudaMemcpy(out, dout, n * 32, cudaMemcpyDeviceToHost));
   });
 }
 
@@ -730,11 +728,13 @@ int nzcp_arith_op(int op, const uint8_t* in, uint8_t* out, size_t n, int device)
     use_device(device);
     if (!n) return;
     const int iw = kArithIn[op], ow = kArithOut[op];
-    DevBuf din(n * iw), dout(n * ow);
-    NZCP_CUDA(cudaMemcpy(din.p, in, n * iw, cudaMemcpyHostToDevice));
-    arith_op_kernel<<<div_up(n, 128), 128>>>(op, din.as<uint32_t>(), dout.as<uint32_t>(), n, iw / 4, ow / 4);
+    CudaResources res;
+    uint32_t* din = res.device<uint32_t>(n * iw / 4);   // n > 0
+    uint32_t* dout = res.device<uint32_t>(n * ow / 4);
+    NZCP_CUDA(cudaMemcpy(din, in, n * iw, cudaMemcpyHostToDevice));
+    arith_op_kernel<<<div_up(n, 128), 128>>>(op, din, dout, n, iw / 4, ow / 4);
     NZCP_LAUNCH_CHECK();
-    NZCP_CUDA(cudaMemcpy(out, dout.p, n * ow, cudaMemcpyDeviceToHost));
+    NZCP_CUDA(cudaMemcpy(out, dout, n * ow, cudaMemcpyDeviceToHost));
   });
 }
 

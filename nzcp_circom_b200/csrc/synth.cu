@@ -275,16 +275,13 @@ template <class F>
 static void fixed_base_batch(const Affine<F>* d_table, const std::vector<Fr>& scalars, uint8_t* dst) {
   size_t count = scalars.size();
   if (!count) return;
-  Fr* d_s = nullptr;
-  Affine<F>* d_o = nullptr;
-  NZCP_CUDA(cudaMalloc(&d_s, count * sizeof(Fr)));
-  NZCP_CUDA(cudaMalloc(&d_o, count * sizeof(Affine<F>)));
+  CudaResources res;
+  Fr* d_s = res.device<Fr>(count);
+  Affine<F>* d_o = res.device<Affine<F>>(count);
   NZCP_CUDA(cudaMemcpy(d_s, scalars.data(), count * sizeof(Fr), cudaMemcpyHostToDevice));
   fixed_base_mul_kernel<F><<<div_up(count, 128), 128>>>(d_table, d_s, d_o, count);
   NZCP_LAUNCH_CHECK();
   NZCP_CUDA(cudaMemcpy(dst, d_o, count * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
-  cudaFree(d_s);
-  cudaFree(d_o);
 }
 
 // In-place batch inversion (Montgomery trick); zero entries are left untouched.
@@ -388,16 +385,11 @@ static void synth_write_zkey_impl(const nzcp_synth* c, const uint8_t toxic[160],
   // device tables
   std::vector<G1Affine> t1 = fixed_base_table<Fq>(g1_generator());
   std::vector<G2Affine> t2 = fixed_base_table<Fq2>(g2_generator());
-  G1Affine* d_t1 = nullptr;
-  G2Affine* d_t2 = nullptr;
-  NZCP_CUDA(cudaMalloc(&d_t1, t1.size() * sizeof(G1Affine)));
-  NZCP_CUDA(cudaMalloc(&d_t2, t2.size() * sizeof(G2Affine)));
+  CudaResources res;
+  G1Affine* d_t1 = res.device<G1Affine>(t1.size());
+  G2Affine* d_t2 = res.device<G2Affine>(t2.size());
   NZCP_CUDA(cudaMemcpy(d_t1, t1.data(), t1.size() * sizeof(G1Affine), cudaMemcpyHostToDevice));
   NZCP_CUDA(cudaMemcpy(d_t2, t2.data(), t2.size() * sizeof(G2Affine), cudaMemcpyHostToDevice));
-  struct Free {
-    void* a; void* b;
-    ~Free() { cudaFree(a); cudaFree(b); }
-  } fr{d_t1, d_t2};
 
   Writer w(out, cap);
   w.raw("zkey", 4);
@@ -543,9 +535,8 @@ namespace nzcp {
 template <class F>
 static void synth_points_impl(const Affine<F>& gen, uint64_t seed, size_t n, uint8_t* out) {
   std::vector<Affine<F>> tab = fixed_base_table<F>(gen);
-  Affine<F>* d_tab = nullptr;
-  NZCP_CUDA(cudaMalloc(&d_tab, tab.size() * sizeof(Affine<F>)));
-  struct Free { void* p; ~Free() { cudaFree(p); } } fr{d_tab};
+  CudaResources res;
+  Affine<F>* d_tab = res.device<Affine<F>>(tab.size());
   NZCP_CUDA(cudaMemcpy(d_tab, tab.data(), tab.size() * sizeof(Affine<F>), cudaMemcpyHostToDevice));
   Rng g(seed);
   const size_t chunk = (size_t)1 << 20;

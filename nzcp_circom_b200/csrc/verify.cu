@@ -108,7 +108,8 @@ void check_init_sections(const ZkeyIn& z) {
 // ------------------------------------------------------------------------------------------------ circuit hash
 struct HDiff {
   uint64_t n = 0;                   // h_hash_points(N)
-  std::unique_ptr<DevMem> d;        // device run: the differences, resident for the H check
+  G1Affine* d = nullptr;            // device run: the differences, resident for the H check
+  CudaResources res;
   std::vector<G1Affine> h;          // host run
 };
 
@@ -140,17 +141,18 @@ void circuit_hash(const ZkeyIn& zi, const Ptau& pt, bool host, uint8_t out[64], 
     }
     hs.points_host(diff.h.data(), diff.n);
   } else {
-    DevMem d_tau((N + diff.n) * 64);
-    diff.d.reset(new DevMem(diff.n * 64));
-    NZCP_CUDA(cudaMemcpy(d_tau.p, pt.s[2].p, (N + diff.n) * 64, cudaMemcpyHostToDevice));
-    Events ev;
-    NZCP_CUDA(cudaEventRecord(ev.a, 0));
-    h_diff_kernel<<<div_up(diff.n, 128), 128>>>(static_cast<const G1Affine*>(d_tau.p), N, static_cast<G1Affine*>(diff.d->p), diff.n);
+    CudaResources res;
+    G1Affine* d_tau = res.device<G1Affine>(N + diff.n);
+    diff.d = diff.res.device<G1Affine>(diff.n);   // N >= 2: at least one difference
+    NZCP_CUDA(cudaMemcpy(d_tau, pt.s[2].p, (N + diff.n) * 64, cudaMemcpyHostToDevice));
+    const cudaEvent_t e0 = res.event(), e1 = res.event();
+    NZCP_CUDA(cudaEventRecord(e0, 0));
+    h_diff_kernel<<<div_up(diff.n, 128), 128>>>(d_tau, N, diff.d, diff.n);
     NZCP_LAUNCH_CHECK();
-    NZCP_CUDA(cudaEventRecord(ev.b, 0));
-    NZCP_CUDA(cudaEventSynchronize(ev.b));
-    NZCP_CUDA(cudaEventElapsedTime(&diff_ms, ev.a, ev.b));
-    hs.points_device(static_cast<const G1Affine*>(diff.d->p), diff.n);
+    NZCP_CUDA(cudaEventRecord(e1, 0));
+    NZCP_CUDA(cudaEventSynchronize(e1));
+    NZCP_CUDA(cudaEventElapsedTime(&diff_ms, e0, e1));
+    hs.points_device(diff.d, diff.n);
   }
   hs.u32be((uint32_t)(m - np - 1));
   hs.section<Fq>(zi.s[8].p, m - np - 1);
@@ -278,10 +280,6 @@ G1Affine msm_g1(void* d_bases, const Fr* d_scalars, size_t n) {
   MsmTable tab;
   MsmSort sort;
   MsmRun run;
-  struct Guard {
-    MsmTable* t; MsmSort* s; MsmRun* r;
-    ~Guard() { msm_run_destroy(r); msm_sort_destroy(s); msm_table_destroy(t); }
-  } g{&tab, &sort, &run};
   msm_table_view(&tab, d_bases, n, false, c);
   msm_sort_create(&sort, n, c, -1, true);
   msm_run_create(&run, &sort, false);
@@ -391,14 +389,15 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   ChaCha rng(sd);
   const uint64_t N = z.domain_size, n_l = z.n_l();
   std::vector<Fr> sc(std::max(n_l, N));
-  Events ev;
+  CudaResources res;
+  const cudaEvent_t e0 = res.event(), e1 = res.event();
   auto timed = [&](float& acc_ms, auto&& fn) {   // device time of fn's work on the default stream, added to acc_ms
-    NZCP_CUDA(cudaEventRecord(ev.a, 0));
+    NZCP_CUDA(cudaEventRecord(e0, 0));
     const G1Affine r = fn();
-    NZCP_CUDA(cudaEventRecord(ev.b, 0));
-    NZCP_CUDA(cudaEventSynchronize(ev.b));
+    NZCP_CUDA(cudaEventRecord(e1, 0));
+    NZCP_CUDA(cudaEventSynchronize(e1));
     float t = 0;
-    NZCP_CUDA(cudaEventElapsedTime(&t, ev.a, ev.b));
+    NZCP_CUDA(cudaEventElapsedTime(&t, e0, e1));
     acc_ms += t;
     return r;
   };
@@ -406,33 +405,35 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   // 5. L: sum rho_i L_init[i] and sum rho_i L[i]
   if (n_l) {
     for (uint64_t i = 0; i < n_l; i++) sc[i] = fp_from_rng<FrParams>(rng);
-    DevMem d_sc(n_l * sizeof(Fr)), d_b(n_l * 64);
-    NZCP_CUDA(cudaMemcpy(d_sc.p, sc.data(), n_l * sizeof(Fr), cudaMemcpyHostToDevice));
-    NZCP_CUDA(cudaMemcpy(d_b.p, zi.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
-    const G1Affine r1 = timed(ms[2], [&] { return msm_g1(d_b.p, static_cast<const Fr*>(d_sc.p), n_l); });
-    NZCP_CUDA(cudaMemcpy(d_b.p, z.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
-    const G1Affine r2 = timed(ms[2], [&] { return msm_g1(d_b.p, static_cast<const Fr*>(d_sc.p), n_l); });
+    CudaResources l_res;
+    Fr* d_sc = l_res.device<Fr>(n_l);
+    G1Affine* d_b = l_res.device<G1Affine>(n_l);
+    NZCP_CUDA(cudaMemcpy(d_sc, sc.data(), n_l * sizeof(Fr), cudaMemcpyHostToDevice));
+    NZCP_CUDA(cudaMemcpy(d_b, zi.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
+    const G1Affine r1 = timed(ms[2], [&] { return msm_g1(d_b, d_sc, n_l); });
+    NZCP_CUDA(cudaMemcpy(d_b, z.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
+    const G1Affine r2 = timed(ms[2], [&] { return msm_g1(d_b, d_sc, n_l); });
     cl.add(11, -1, r1, r2, delta2, delta2_init);
   }
 
   // 6. H: r_(N-1) = 0, R1 over the differences i <= N - 2, r' = Fr.fft(-2 w_2N^m r_m), R2 over section 9
   for (uint64_t i = 0; i + 1 < N; i++) sc[i] = fp_from_rng<FrParams>(rng);
   sc[N - 1] = Fr::zero();
-  DevMem d_r(N * sizeof(Fr)), d_tmp(N * sizeof(Fr)), d_h(N * 64);
-  NZCP_CUDA(cudaMemcpy(d_r.p, sc.data(), N * sizeof(Fr), cudaMemcpyHostToDevice));
-  NZCP_CUDA(cudaMemcpy(d_h.p, z.s[9].p, N * 64, cudaMemcpyHostToDevice));
+  Fr* d_r = res.device<Fr>(N);
+  Fr* d_tmp = res.device<Fr>(N);
+  G1Affine* d_h = res.device<G1Affine>(N);
+  NZCP_CUDA(cudaMemcpy(d_r, sc.data(), N * sizeof(Fr), cudaMemcpyHostToDevice));
+  NZCP_CUDA(cudaMemcpy(d_h, z.s[9].p, N * 64, cudaMemcpyHostToDevice));
   NttDomain dom;
   ntt_domain_create(&dom, (int)in.cir_power, 0);
-  struct DomGuard { NttDomain* d; ~DomGuard() { ntt_domain_destroy(d); } } dg{&dom};
-  const G1Affine r1 = timed(ms[3], [&] { return msm_g1(diff.d->p, static_cast<const Fr*>(d_r.p), N - 1); });
+  const G1Affine r1 = timed(ms[3], [&] { return msm_g1(diff.d, d_r, N - 1); });
   Fr two = Fr::zero();
   two.v[0] = 2;
   const G1Affine r2 = timed(ms[3], [&] {
-    h_scalar_kernel<<<div_up(N, 256), 256>>>(static_cast<Fr*>(d_r.p), N, host_fr_root((int)in.cir_power + 1),
-                                             fp_neg(fp_to_mont(two)));
+    h_scalar_kernel<<<div_up(N, 256), 256>>>(d_r, N, host_fr_root((int)in.cir_power + 1), fp_neg(fp_to_mont(two)));
     NZCP_LAUNCH_CHECK();
-    ntt_forward(dom, static_cast<Fr*>(d_r.p), static_cast<Fr*>(d_tmp.p), 0);
-    return msm_g1(d_h.p, static_cast<const Fr*>(d_r.p), N);
+    ntt_forward(dom, d_r, d_tmp, 0);
+    return msm_g1(d_h, d_r, N);
   });
   cl.add(12, -1, r1, r2, delta2, delta2_init);
 }
