@@ -3,7 +3,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <string.h>
+
 #include <atomic>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <utility>
@@ -107,6 +110,81 @@ class CudaResources {
   }
   std::vector<Item> items_;
   size_t device_bytes_ = 0;
+};
+
+// Device time on stream st from construction to end(); ms() waits for the end event.  An inactive timer makes no CUDA
+// call and reads 0 ms (the host runs of Exec).
+struct Timer {
+  CudaResources res;
+  cudaEvent_t a = nullptr, b = nullptr;
+  cudaStream_t st;
+  explicit Timer(cudaStream_t s, bool active = true) : st(s) {
+    if (!active) return;
+    a = res.event();
+    b = res.event();
+    NZCP_CUDA(cudaEventRecord(a, st));
+  }
+  void end() {
+    if (b) NZCP_CUDA(cudaEventRecord(b, st));
+  }
+  float ms() {
+    float t = 0;
+    if (!b) return t;
+    NZCP_CUDA(cudaEventSynchronize(b));
+    NZCP_CUDA(cudaEventElapsedTime(&t, a, b));
+    return t;
+  }
+  float stop() {
+    end();
+    return ms();
+  }
+};
+
+// One thread per index: op(i) for i < n.
+template <int THREADS, class Op>
+__global__ void __launch_bounds__(THREADS) for_each_kernel(Op op, uint64_t n) {
+  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) op(i);
+}
+
+// Where a per-index step runs: on the device (for_each_kernel on stream 0, memory from CudaResources) or, for the host
+// test hooks, in a loop on the CPU over host memory, making no CUDA call at all.  Memory from alloc() lives as long as the
+// executor, so a scope that frees its buffers at its end makes an executor of its own.
+class Exec {
+ public:
+  explicit Exec(bool host) : host_(host) {}
+  bool host() const { return host_; }
+
+  template <class T>
+  T* alloc(size_t count) {
+    if (!host_) return res_.device<T>(count);
+    host_mem_.emplace_back(new uint4[div_up(count * sizeof(T), sizeof(uint4))]);   // 16-byte aligned, as Fp is
+    return reinterpret_cast<T*>(host_mem_.back().get());
+  }
+  void upload(void* dst, const void* src, size_t bytes) const {
+    if (host_) memcpy(dst, src, bytes);
+    else NZCP_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyHostToDevice));
+  }
+  void download(void* dst, const void* src, size_t bytes) const {
+    if (host_) memcpy(dst, src, bytes);
+    else NZCP_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost));
+  }
+  // op(i) for i < n, n > 0.
+  template <int THREADS, class Op>
+  void run(uint64_t n, const Op& op) const {
+    if (host_) {
+      for (uint64_t i = 0; i < n; i++) op(i);
+      return;
+    }
+    for_each_kernel<THREADS><<<div_up(n, THREADS), THREADS>>>(op, n);
+    NZCP_LAUNCH_CHECK();
+  }
+  Timer timer() const { return Timer(0, !host_); }
+
+ private:
+  bool host_;
+  CudaResources res_;
+  std::vector<std::unique_ptr<uint4[]>> host_mem_;
 };
 
 G1Affine g1_generator();   // synth.cu: the BN254 generators, Montgomery affine

@@ -37,10 +37,11 @@ HD G1Affine scale_point(const G1Affine& p, const Fr& k) {   // k plain, < r
   return to_affine_fast(acc);
 }
 
-__global__ void __launch_bounds__(128) zkey_scale_kernel(G1Affine* __restrict__ x, Fr k, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) x[i] = scale_point(x[i], k);
-}
+struct ZkeyScale {   // Exec op
+  G1Affine* x;
+  Fr k;
+  HD void operator()(uint64_t i) const { x[i] = scale_point(x[i], k); }
+};
 
 namespace {
 
@@ -48,32 +49,6 @@ size_t contribute_size(const ZkeyIn& z, size_t name_len, size_t beacon_len) {
   size_t total = 12 + 10 * 12 + 4 + kZkeyHeaderLen;
   for (int id = 3; id <= 10; id++) total += z.s[id].len;
   return total + kRecFixed + params_len(name_len, beacon_len);
-}
-
-// Scale n points of src by k into dst; returns the kernel's device milliseconds.  d_buf holds at least n points.
-float scale_section_device(const uint8_t* src, uint64_t n, const Fr& k, G1Affine* d_buf, uint8_t* dst) {
-  if (n == 0) return 0.f;
-  CudaResources res;
-  const cudaEvent_t e0 = res.event(), e1 = res.event();
-  NZCP_CUDA(cudaMemcpyAsync(d_buf, src, n * 64, cudaMemcpyHostToDevice, 0));
-  NZCP_CUDA(cudaEventRecord(e0, 0));
-  zkey_scale_kernel<<<div_up(n, 128), 128>>>(d_buf, k, n);
-  NZCP_LAUNCH_CHECK();
-  NZCP_CUDA(cudaEventRecord(e1, 0));
-  NZCP_CUDA(cudaMemcpyAsync(dst, d_buf, n * 64, cudaMemcpyDeviceToHost, 0));
-  NZCP_CUDA(cudaStreamSynchronize(0));
-  float ms = 0;
-  NZCP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  return ms;
-}
-
-void scale_section_host(const uint8_t* src, uint64_t n, const Fr& k, uint8_t* dst) {
-  for (uint64_t i = 0; i < n; i++) {
-    G1Affine a;
-    memcpy(&a, src + i * 64, 64);
-    a = scale_point(a, k);
-    memcpy(dst + i * 64, &a, 64);
-  }
 }
 
 // device < 0: the host hook.
@@ -157,16 +132,22 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
     w.section(id, z.s[id].len);
     w.raw(z.s[id].p, z.s[id].len);
   }
-  CudaResources res;
+  Exec ex(host);
   const size_t buf_bytes = std::max<uint64_t>(z.n_l(), z.domain_size) * 64;
-  G1Affine* d_buf = host ? nullptr : reinterpret_cast<G1Affine*>(res.device<unsigned char>(buf_bytes ? buf_bytes : 16));
+  G1Affine* buf = reinterpret_cast<G1Affine*>(ex.alloc<unsigned char>(buf_bytes ? buf_bytes : 16));
   for (int id = 8; id <= 9; id++) {
     const uint64_t n = id == 8 ? z.n_l() : z.domain_size;
     w.section(id, n * 64);
     uint8_t* dst = w.reserve(n * 64);
     float ms = 0;
-    if (host) scale_section_host(z.s[id].p, n, k_inv, dst);
-    else ms = scale_section_device(z.s[id].p, n, k_inv, d_buf, dst);
+    if (n) {   // the scale alone is timed
+      ex.upload(buf, z.s[id].p, n * 64);
+      Timer t = ex.timer();
+      ex.run<128>(n, ZkeyScale{buf, k_inv});
+      t.end();
+      ex.download(dst, buf, n * 64);
+      ms = t.ms();
+    }
     if (section_ms) section_ms[id - 8] = ms;
   }
   w.section(10, z.s[10].len + rec.size());

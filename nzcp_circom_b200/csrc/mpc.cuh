@@ -520,28 +520,35 @@ HD void c_encode(const Affine<F>& a, uint32_t* w) {
 }
 
 template <class F>
-__global__ void __launch_bounds__(128) u_encode_kernel(const Affine<F>* __restrict__ in, uint32_t* __restrict__ out, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) u_encode(in[i], out + i * (sizeof(Affine<F>) / 4));
-}
+struct UEncode {   // Exec op: point i of in -> words [i w, (i + 1) w) of out, w = sizeof(Affine<F>) / 4
+  const Affine<F>* in;
+  uint32_t* out;
+  HD void operator()(uint64_t i) const {
+    const Affine<F> a = in[i];   // a copy: the stores to out cannot alias it
+    u_encode(a, out + i * (sizeof(Affine<F>) / 4));
+  }
+};
 
 template <class F>
-__global__ void __launch_bounds__(128) c_encode_kernel(const Affine<F>* __restrict__ in, uint32_t* __restrict__ out, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) c_encode(in[i], out + i * (sizeof(Affine<F>) / 8));
-}
+struct CEncode {   // Exec op: w = sizeof(Affine<F>) / 8
+  const Affine<F>* in;
+  uint32_t* out;
+  HD void operator()(uint64_t i) const {
+    const Affine<F> a = in[i];
+    c_encode(a, out + i * (sizeof(Affine<F>) / 8));
+  }
+};
 
 // ------------------------------------------------------------------------------------------------ chunked point hashing
 enum class Enc { U, C };   // uncompressed (hashPubKey, the circuit hash, nextChallenge) or compressed (the response hash)
 
 constexpr uint64_t kHashChunk = 1u << 16;     // points per conversion chunk
 
-// BLAKE2b-512 over a stream of bytes and encoded points.  Device-resident points are encoded in chunks, so the host BLAKE2b
-// of chunk j (one sequential stream) overlaps the conversion and copy of chunk j + 1.  on_host: the same encoders run on
-// the CPU (test hooks).
+// BLAKE2b-512 over a stream of bytes and encoded points.  Points in the executor's memory are encoded by its ops; on the
+// device in chunks, so the host BLAKE2b of chunk j (one sequential stream) overlaps the conversion and copy of chunk j + 1.
 struct Hasher {
   Blake2b512 h;
-  bool host;
+  const Exec& ex;
   Enc enc;
   float kernel_ms = 0, blake_ms = 0;
   uint32_t* d_enc[2] = {nullptr, nullptr};
@@ -549,8 +556,8 @@ struct Hasher {
   cudaEvent_t ev[6] = {};   // per buffer: kernel start, kernel end, copy done
   CudaResources res;
 
-  explicit Hasher(bool on_host, Enc e = Enc::U) : host(on_host), enc(e) {
-    if (host) return;
+  explicit Hasher(const Exec& x, Enc e = Enc::U) : ex(x), enc(e) {
+    if (ex.host()) return;
     for (int b = 0; b < 2; b++) {
       d_enc[b] = res.device<uint32_t>(kHashChunk * 32);
       h_enc[b] = res.pinned<uint8_t>(kHashChunk * 128);
@@ -568,6 +575,7 @@ struct Hasher {
     const uint8_t b[4] = {(uint8_t)(v >> 24), (uint8_t)(v >> 16), (uint8_t)(v >> 8), (uint8_t)v};
     update(b, 4);
   }
+  // n points in host memory (the header points and other small arrays)
   template <class F>
   void points_host(const Affine<F>* p, uint64_t n) {
     const size_t w = enc_bytes<F>(enc) / 4;
@@ -583,20 +591,27 @@ struct Hasher {
       update(buf.data(), m * w * 4);
     }
   }
-  // n device-resident points: chunk j's host hash overlaps the conversion and copy of chunk j + 1.
   template <class F>
-  void points_device(const Affine<F>* d, uint64_t n) {
+  void encode(const Affine<F>* x, uint32_t* out, uint64_t n) {
+    if (enc == Enc::U) ex.run<128>(n, UEncode<F>{x, out});
+    else ex.run<128>(n, CEncode<F>{x, out});
+  }
+  // n points in the executor's memory.  On the device chunk j's host hash overlaps the conversion and copy of chunk j + 1.
+  template <class F>
+  void points(const Affine<F>* x, uint64_t n) {
     const size_t esz = enc_bytes<F>(enc);
+    if (ex.host()) {
+      std::vector<uint32_t> buf(n * esz / 4);
+      encode(x, buf.data(), n);
+      return update(buf.data(), n * esz);
+    }
     const uint64_t nch = (n + kHashChunk - 1) / kHashChunk;
     for (uint64_t j = 0; j <= nch; j++) {
       if (j < nch) {
         const int b = j & 1;
         const uint64_t off = j * kHashChunk, m = std::min(kHashChunk, n - off);
-        uint32_t* dst = d_enc[b];
         NZCP_CUDA(cudaEventRecord(ev[3 * b], 0));
-        if (enc == Enc::U) u_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, dst, m);
-        else c_encode_kernel<F><<<div_up(m, 128), 128>>>(d + off, dst, m);
-        NZCP_LAUNCH_CHECK();
+        encode(x + off, d_enc[b], m);
         NZCP_CUDA(cudaEventRecord(ev[3 * b + 1], 0));
         NZCP_CUDA(cudaMemcpyAsync(h_enc[b], d_enc[b], m * esz, cudaMemcpyDeviceToHost, 0));
         NZCP_CUDA(cudaEventRecord(ev[3 * b + 2], 0));
@@ -615,12 +630,11 @@ struct Hasher {
   // n points in host memory
   template <class F>
   void section(const uint8_t* p, uint64_t n) {
-    const Affine<F>* a = reinterpret_cast<const Affine<F>*>(p);
-    if (host || n == 0) return points_host(a, n);
-    CudaResources staged;
-    Affine<F>* d = staged.device<Affine<F>>(n);   // n > 0
-    NZCP_CUDA(cudaMemcpy(d, p, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-    points_device(d, n);
+    if (n == 0) return;
+    Exec staged(ex.host());   // freed when the section is hashed
+    Affine<F>* x = staged.alloc<Affine<F>>(n);
+    staged.upload(x, p, n * sizeof(Affine<F>));
+    points(x, n);
   }
 };
 

@@ -95,25 +95,29 @@ HD void prep_butterfly(Affine<F>* x, const Fr* tw, int t_log, int s, uint64_t u)
   x[i1] = to_affine_fast(add_affine(xyzz_neg(t), a));
 }
 
-// ------------------------------------------------------------------------------------------------ kernels
-__global__ void __launch_bounds__(256) ptau_twiddle_kernel(Fr* __restrict__ tw, Fr w, uint64_t n) {
-  const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (k < n) tw[k] = pow_u32_plain(w, (uint32_t)k);
-}
+// ------------------------------------------------------------------------------------------------ Exec ops
+struct PtauTwiddle {
+  Fr* tw;
+  Fr w;
+  HD void operator()(uint64_t k) const { tw[k] = pow_u32_plain(w, (uint32_t)k); }
+};
 
 template <class F>
-__global__ void __launch_bounds__(128) ptau_load_kernel(const Affine<F>* __restrict__ src, uint64_t n_src,
-                                                        const Fr* __restrict__ ninv, Affine<F>* __restrict__ x, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) x[i] = prep_load(src, n_src, ninv, i);
-}
+struct PtauLoad {
+  const Affine<F>* src;
+  uint64_t n_src;
+  const Fr* ninv;
+  Affine<F>* x;
+  HD void operator()(uint64_t i) const { x[i] = prep_load(src, n_src, ninv, i); }
+};
 
 template <class F>
-__global__ void __launch_bounds__(128) ptau_stage_kernel(Affine<F>* __restrict__ x, const Fr* __restrict__ tw, int t_log, int s,
-                                                         uint64_t n) {
-  const uint64_t u = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (u < n) prep_butterfly(x, tw, t_log, s, u);
-}
+struct PtauStage {
+  Affine<F>* x;
+  const Fr* tw;
+  int t_log, s;
+  HD void operator()(uint64_t u) const { prep_butterfly(x, tw, t_log, s, u); }
+};
 
 // ------------------------------------------------------------------------------------------------ host side
 namespace {
@@ -169,41 +173,21 @@ std::vector<Fr> ninv_table(uint32_t top) {
   return t;
 }
 
+// One output section: load, then every stage; returns their device ms.  Its buffers are freed when it is written.
 template <class F>
-float run_section_device(const uint8_t* src, uint64_t n_src, uint32_t top, const Fr* d_ninv, const Fr* d_tw, int t_log,
-                         uint8_t* out) {
+float run_section(bool host, const uint8_t* src, uint64_t n_src, uint32_t top, const Fr* ninv, const Fr* tw, int t_log,
+                  uint8_t* out) {
   const uint64_t n = level_points(top);
-  CudaResources res;
-  Affine<F>* d_src = res.device<Affine<F>>(n_src);   // n_src, n > 0
-  Affine<F>* d_x = res.device<Affine<F>>(n);
-  NZCP_CUDA(cudaMemcpy(d_src, src, n_src * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-  const cudaEvent_t e0 = res.event(), e1 = res.event();
-  NZCP_CUDA(cudaEventRecord(e0, 0));
-  ptau_load_kernel<F><<<div_up(n, 128), 128>>>(d_src, n_src, d_ninv, d_x, n);
-  NZCP_LAUNCH_CHECK();
-  for (uint32_t s = 0; s < top; s++) {
-    const uint64_t nb = ((uint64_t)1 << top) - ((uint64_t)1 << s);
-    ptau_stage_kernel<F><<<div_up(nb, 128), 128>>>(d_x, d_tw, t_log, (int)s, nb);
-    NZCP_LAUNCH_CHECK();
-  }
-  NZCP_CUDA(cudaEventRecord(e1, 0));
-  NZCP_CUDA(cudaEventSynchronize(e1));
-  float ms = 0;
-  NZCP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  NZCP_CUDA(cudaMemcpy(out, d_x, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
+  Exec ex(host);
+  Affine<F>* in = ex.alloc<Affine<F>>(n_src);   // n_src, n > 0
+  Affine<F>* x = ex.alloc<Affine<F>>(n);
+  ex.upload(in, src, n_src * sizeof(Affine<F>));
+  Timer t = ex.timer();
+  ex.run<128>(n, PtauLoad<F>{in, n_src, ninv, x});
+  for (uint32_t s = 0; s < top; s++) ex.run<128>(((uint64_t)1 << top) - ((uint64_t)1 << s), PtauStage<F>{x, tw, t_log, (int)s});
+  const float ms = t.stop();
+  ex.download(out, x, n * sizeof(Affine<F>));
   return ms;
-}
-
-// The same load / stage indexing / butterflies, one "thread" after the other on the CPU (test hook, small powers).
-template <class F>
-void run_section_host(const uint8_t* src, uint64_t n_src, uint32_t top, const Fr* ninv, const Fr* tw, int t_log, uint8_t* out) {
-  const uint64_t n = level_points(top);
-  std::vector<Affine<F>> in(n_src), x(n);
-  memcpy(in.data(), src, n_src * sizeof(Affine<F>));
-  for (uint64_t i = 0; i < n; i++) x[i] = prep_load(in.data(), n_src, ninv, i);
-  for (uint32_t s = 0; s < top; s++)
-    for (uint64_t u = 0; u < ((uint64_t)1 << top) - ((uint64_t)1 << s); u++) prep_butterfly(x.data(), tw, t_log, (int)s, u);
-  memcpy(out, x.data(), n * sizeof(Affine<F>));
 }
 
 // device < 0: the host hook.
@@ -220,20 +204,12 @@ void prepare_impl(const uint8_t* b, size_t len, int device, uint8_t* out, size_t
   const int t_log = (int)p.power + 1;                       // twiddle table: w^(-k), w = Fr.w[power + 1], k < 2^power
   const uint64_t n_tw = (uint64_t)1 << p.power;
   const Fr w_inv = fp_inv(host_fr_root(t_log));
-  const std::vector<Fr> ninv = ninv_table(p.power + 1);
-  std::vector<Fr> tw;
-  CudaResources res;
-  Fr *d_tw = nullptr, *d_ninv = nullptr;
-  if (host) {
-    tw.resize(n_tw);
-    for (uint64_t k = 0; k < n_tw; k++) tw[k] = pow_u32_plain(w_inv, (uint32_t)k);
-  } else {
-    d_tw = res.device<Fr>(n_tw);
-    d_ninv = res.device<Fr>(ninv.size());
-    NZCP_CUDA(cudaMemcpy(d_ninv, ninv.data(), ninv.size() * sizeof(Fr), cudaMemcpyHostToDevice));
-    ptau_twiddle_kernel<<<div_up(n_tw, 256), 256>>>(d_tw, w_inv, n_tw);
-    NZCP_LAUNCH_CHECK();
-  }
+  const std::vector<Fr> ninv_h = ninv_table(p.power + 1);
+  Exec ex(host);
+  Fr* tw = ex.alloc<Fr>(n_tw);
+  Fr* ninv = ex.alloc<Fr>(ninv_h.size());
+  ex.upload(ninv, ninv_h.data(), ninv_h.size() * sizeof(Fr));
+  ex.run<256>(n_tw, PtauTwiddle{tw, w_inv});
 
   Writer w(out, cap);
   write_ptau_header(w, p.power, 11);
@@ -248,14 +224,8 @@ void prepare_impl(const uint8_t* b, size_t len, int device, uint8_t* out, size_t
     w.section(o.id, n * psz);
     uint8_t* dst = w.reserve(n * psz);
     const uint64_t n_src = p.s[o.src].len / psz;           // 2^top, or 2^top - 1 for tauG1 (the top level's pad)
-    float ms = 0;
-    if (host) {
-      if (o.g2) run_section_host<Fq2>(p.s[o.src].p, n_src, o.top, ninv.data(), tw.data(), t_log, dst);
-      else run_section_host<Fq>(p.s[o.src].p, n_src, o.top, ninv.data(), tw.data(), t_log, dst);
-    } else {
-      if (o.g2) ms = run_section_device<Fq2>(p.s[o.src].p, n_src, o.top, d_ninv, d_tw, t_log, dst);
-      else ms = run_section_device<Fq>(p.s[o.src].p, n_src, o.top, d_ninv, d_tw, t_log, dst);
-    }
+    const float ms = o.g2 ? run_section<Fq2>(host, p.s[o.src].p, n_src, o.top, ninv, tw, t_log, dst)
+                          : run_section<Fq>(host, p.s[o.src].p, n_src, o.top, ninv, tw, t_log, dst);
     if (section_ms) section_ms[k] = ms;
   }
   if (w.pos != total) throw ApiError(NZCP_E_INTERNAL, "ptau prepare: size accounting error");

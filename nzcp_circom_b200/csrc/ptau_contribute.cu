@@ -36,12 +36,12 @@
 // input points must be canonical and on their curve (snarkjs does not check).  A G2 point outside the order-r subgroup,
 // which no ceremony file holds, is scaled by the folded window of scalar_mul_accumulate and then differs from snarkjs's.
 //
-// B200 design.  One section at a time resides in HBM (tauG1 at power 28: 2^29 - 1 points, 34 GB).  ptau_key_kernel runs
+// B200 design.  One section at a time resides in HBM (tauG1 at power 28: 2^29 - 1 points, 34 GB).  The PtauKey op runs
 // one thread per point: s = first * tau^i by square-and-multiply over the <= 29 bits of i (~45 Fr products against ~3 300
 // Fq products for the G1 multiplication, so no power table), then the signed 4-bit window of ec.cuh scalar_mul_accumulate
-// and to_affine_fast.  Unlike zkey_scale_kernel every lane has its own scalar.  The response pass encodes the points still
-// resident after the key kernel (c_encode_kernel); the nextChallenge pass re-uploads each finished section from the output
-// (u_encode_kernel); both run through mpc.cuh's chunked Hasher, whose host BLAKE2b of chunk j overlaps the encoding and
+// and to_affine_fast.  Unlike contribute.cu's ZkeyScale every lane has its own scalar.  The response pass encodes the
+// points still resident after the key op (CEncode); the nextChallenge pass re-uploads each finished section from the
+// output (UEncode); both run through mpc.cuh's chunked Hasher, whose host BLAKE2b of chunk j overlaps the encoding and
 // copy of chunk j + 1.  The host BLAKE2b is a single sequential stream and likely takes longer than the kernels.
 #include "mpc.cuh"
 
@@ -62,10 +62,11 @@ HD Affine<F> ptau_key_point(const Affine<F>& p, const Fr& first, const Fr& inc, 
 }
 
 template <class F>
-__global__ void __launch_bounds__(128) ptau_key_kernel(Affine<F>* __restrict__ x, Fr first, Fr inc, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) x[i] = ptau_key_point(x[i], first, inc, i);
-}
+struct PtauKey {   // Exec op
+  Affine<F>* x;
+  Fr first, inc;
+  HD void operator()(uint64_t i) const { x[i] = ptau_key_point(x[i], first, inc, i); }
+};
 
 namespace {
 
@@ -179,32 +180,17 @@ void pub_key(const KeyPart k[3], bool montgomery, uint8_t out[kPubKeyLen]) {
   }
 }
 
+// Upload, key op in place, response-hash the resident points, download; returns the key op's device ms.
 template <class F>
-void key_section_host(uint8_t* x, uint64_t n, const Fr& first, const Fr& inc) {
-  for (uint64_t i = 0; i < n; i++) {
-    Affine<F> a;
-    memcpy(&a, x + i * sizeof a, sizeof a);
-    a = ptau_key_point(a, first, inc, i);
-    memcpy(x + i * sizeof a, &a, sizeof a);
-  }
-}
-
-// Upload, key kernel in place, response-hash the resident points, download; returns the key kernel's device ms.
-template <class F>
-float key_section_device(const uint8_t* src, uint64_t n, const Fr& first, const Fr& inc, Affine<F>* d_x, Hasher& resp,
-                         uint8_t* dst) {
-  CudaResources res;
-  const cudaEvent_t e0 = res.event(), e1 = res.event();
-  NZCP_CUDA(cudaMemcpy(d_x, src, n * sizeof(Affine<F>), cudaMemcpyHostToDevice));
-  NZCP_CUDA(cudaEventRecord(e0, 0));
-  ptau_key_kernel<F><<<div_up(n, 128), 128>>>(d_x, first, inc, n);
-  NZCP_LAUNCH_CHECK();
-  NZCP_CUDA(cudaEventRecord(e1, 0));
-  resp.points_device(d_x, n);
-  NZCP_CUDA(cudaMemcpy(dst, d_x, n * sizeof(Affine<F>), cudaMemcpyDeviceToHost));
-  float ms = 0;
-  NZCP_CUDA(cudaEventElapsedTime(&ms, e0, e1));
-  return ms;
+float key_section(const Exec& ex, const uint8_t* src, uint64_t n, const Fr& first, const Fr& inc, Affine<F>* x, Hasher& resp,
+                  uint8_t* dst) {
+  ex.upload(x, src, n * sizeof(Affine<F>));
+  Timer t = ex.timer();
+  ex.run<128>(n, PtauKey<F>{x, first, inc});
+  t.end();
+  resp.points(x, n);
+  ex.download(dst, x, n * sizeof(Affine<F>));
+  return t.ms();
 }
 
 // device < 0: the host hook.  ms: [0..4] key kernels of sections 2..6, [5] encode kernels, [6] host BLAKE2b.
@@ -235,29 +221,17 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
   // ---- sections 2-6 and the response hash
   Writer w(out, cap);
   write_ptau_header(w, p.power, 7);
-  Hasher resp(host, Enc::C);
+  Exec ex(host);
+  Hasher resp(ex, Enc::C);
   resp.update(challenge, 64);
-  CudaResources res;
-  void* d_buf = host ? nullptr : res.device<unsigned char>(sect_bytes(p.power, 3));   // the largest section: 2^p G2 points
+  void* buf = ex.alloc<unsigned char>(sect_bytes(p.power, 3));   // the largest section: 2^p G2 points
   uint8_t* sect[7] = {};
   for (int id = 2; id <= 6; id++) {
     const uint64_t n = sect_points(p.power, id);
     w.section(id, p.s[id].len);
     sect[id] = w.reserve(p.s[id].len);
-    if (host) {
-      memcpy(sect[id], p.s[id].p, p.s[id].len);
-      if (sect_g2(id)) {
-        key_section_host<Fq2>(sect[id], n, *first[id], tau);
-        resp.points_host(reinterpret_cast<const G2Affine*>(sect[id]), n);
-      } else {
-        key_section_host<Fq>(sect[id], n, *first[id], tau);
-        resp.points_host(reinterpret_cast<const G1Affine*>(sect[id]), n);
-      }
-    } else if (sect_g2(id)) {
-      ms[id - 2] = key_section_device(p.s[id].p, n, *first[id], tau, static_cast<G2Affine*>(d_buf), resp, sect[id]);
-    } else {
-      ms[id - 2] = key_section_device(p.s[id].p, n, *first[id], tau, static_cast<G1Affine*>(d_buf), resp, sect[id]);
-    }
+    if (sect_g2(id)) ms[id - 2] = key_section(ex, p.s[id].p, n, *first[id], tau, static_cast<G2Affine*>(buf), resp, sect[id]);
+    else ms[id - 2] = key_section(ex, p.s[id].p, n, *first[id], tau, static_cast<G1Affine*>(buf), resp, sect[id]);
   }
   uint8_t partial[kPartialLen], pk[kPubKeyLen], response[64];
   resp.h.partial(partial);
@@ -266,18 +240,13 @@ void contribute_impl(const uint8_t* b, size_t len, ContribArgs a, int device, ui
   resp.h.final(response);
 
   // ---- nextChallenge: the new sections again, uncompressed
-  Hasher nx(host, Enc::U);
+  Hasher nx(ex, Enc::U);
   nx.update(response, 64);
   for (int id = 2; id <= 6; id++) {
     const uint64_t n = sect_points(p.power, id);
-    if (host) {
-      if (sect_g2(id)) nx.points_host(reinterpret_cast<const G2Affine*>(sect[id]), n);
-      else nx.points_host(reinterpret_cast<const G1Affine*>(sect[id]), n);
-    } else {
-      NZCP_CUDA(cudaMemcpy(d_buf, sect[id], p.s[id].len, cudaMemcpyHostToDevice));
-      if (sect_g2(id)) nx.points_device(static_cast<const G2Affine*>(d_buf), n);
-      else nx.points_device(static_cast<const G1Affine*>(d_buf), n);
-    }
+    ex.upload(buf, sect[id], p.s[id].len);
+    if (sect_g2(id)) nx.points(static_cast<const G2Affine*>(buf), n);
+    else nx.points(static_cast<const G1Affine*>(buf), n);
   }
   uint8_t next[64];
   nx.h.final(next);

@@ -13,20 +13,6 @@ extern std::atomic<int> g_tune_pair_stage;
 extern std::atomic<int> g_tune_pair_k[kMsmMaxRounds];
 extern std::atomic<int> g_tune_rounds_w, g_tune_rounds_h;
 
-struct Timer {   // device time on stream st from construction to stop()
-  CudaResources res;
-  cudaEvent_t a = res.event(), b = res.event();
-  cudaStream_t st;
-  explicit Timer(cudaStream_t s) : st(s) { NZCP_CUDA(cudaEventRecord(a, st)); }
-  float stop() {
-    float ms = 0;
-    NZCP_CUDA(cudaEventRecord(b, st));
-    NZCP_CUDA(cudaEventSynchronize(b));
-    NZCP_CUDA(cudaEventElapsedTime(&ms, a, b));
-    return ms;
-  }
-};
-
 // ------------------------------------------------------------------------------------------------ self-test kernels
 template <class P>
 __global__ void field_op_kernel(int op, const Fp<P>* a, const Fp<P>* b, Fp<P>* out, size_t n) {

@@ -55,23 +55,26 @@ HD G1Affine h_diff_point(const G1Affine& hi, const G1Affine& lo) {
   return to_affine_fast(acc);
 }
 
-__global__ void __launch_bounds__(128) h_diff_kernel(const G1Affine* __restrict__ tau, uint64_t N, G1Affine* __restrict__ out,
-                                                     uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = h_diff_point(tau[i + N], tau[i]);
-}
+struct HDifference {   // Exec op
+  const G1Affine* tau;
+  uint64_t N;
+  G1Affine* out;
+  HD void operator()(uint64_t i) const { out[i] = h_diff_point(tau[i + N], tau[i]); }
+};
 
-// r[m] <- -2 w^m r[m]: plain r, Montgomery w and -2, plain result.
-__global__ void __launch_bounds__(256) h_scalar_kernel(Fr* __restrict__ r, uint64_t n, Fr w, Fr neg2) {
-  const uint64_t m = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (m >= n) return;
-  Fr p = Fr::one(), b = w;
-  for (uint64_t e = m; e; e >>= 1) {
-    if (e & 1) p = fp_mul(p, b);
-    b = fp_sqr(b);
+// Exec op: r[m] <- -2 w^m r[m]: plain r, Montgomery w and -2, plain result.
+struct HScalar {
+  Fr* r;
+  Fr w, neg2;
+  HD void operator()(uint64_t m) const {
+    Fr p = Fr::one(), b = w;
+    for (uint64_t e = m; e; e >>= 1) {
+      if (e & 1) p = fp_mul(p, b);
+      b = fp_sqr(b);
+    }
+    r[m] = fp_mul(fp_mul(r[m], p), neg2);
   }
-  r[m] = fp_mul(fp_mul(r[m], p), neg2);
-}
+};
 
 namespace {
 
@@ -107,17 +110,17 @@ void check_init_sections(const ZkeyIn& z) {
 
 // ------------------------------------------------------------------------------------------------ circuit hash
 struct HDiff {
+  explicit HDiff(bool host) : ex(host) {}
+  Exec ex;                          // runs the circuit hash and owns d
   uint64_t n = 0;                   // h_hash_points(N)
-  G1Affine* d = nullptr;            // device run: the differences, resident for the H check
-  CudaResources res;
-  std::vector<G1Affine> h;          // host run
+  G1Affine* d = nullptr;            // the differences, resident for the H check
 };
 
 // csHash of the initial key zi (zkey_new.js order); the H differences are left in `diff`.
-void circuit_hash(const ZkeyIn& zi, const Ptau& pt, bool host, uint8_t out[64], HDiff& diff, float* kernel_ms, float* blake_ms) {
+void circuit_hash(const ZkeyIn& zi, const Ptau& pt, uint8_t out[64], HDiff& diff, float* kernel_ms, float* blake_ms) {
   const uint8_t* hd = zi.s[2].p;
   const uint64_t N = zi.domain_size, m = zi.n_vars, np = zi.n_public;
-  Hasher hs(host);
+  Hasher hs(diff.ex);
   const G1Affine g1 = g1_generator();
   const G2Affine g2 = g2_generator();
   hs.points_host(reinterpret_cast<const G1Affine*>(hd + kZkeyAlpha1Off), 2);   // alpha1, beta1
@@ -130,29 +133,15 @@ void circuit_hash(const ZkeyIn& zi, const Ptau& pt, bool host, uint8_t out[64], 
   hs.u32be((uint32_t)(N - 1));
   diff.n = h_hash_points(N);
   float diff_ms = 0;
-  if (host) {
-    diff.h.resize(diff.n);
-    const G1Affine* tau = reinterpret_cast<const G1Affine*>(pt.s[2].p);
-    for (uint64_t i = 0; i < diff.n; i++) {
-      G1Affine a, b;
-      memcpy(&a, tau + i + N, 64);
-      memcpy(&b, tau + i, 64);
-      diff.h[i] = h_diff_point(a, b);
-    }
-    hs.points_host(diff.h.data(), diff.n);
-  } else {
-    CudaResources res;
-    G1Affine* d_tau = res.device<G1Affine>(N + diff.n);
-    diff.d = diff.res.device<G1Affine>(diff.n);   // N >= 2: at least one difference
-    NZCP_CUDA(cudaMemcpy(d_tau, pt.s[2].p, (N + diff.n) * 64, cudaMemcpyHostToDevice));
-    const cudaEvent_t e0 = res.event(), e1 = res.event();
-    NZCP_CUDA(cudaEventRecord(e0, 0));
-    h_diff_kernel<<<div_up(diff.n, 128), 128>>>(d_tau, N, diff.d, diff.n);
-    NZCP_LAUNCH_CHECK();
-    NZCP_CUDA(cudaEventRecord(e1, 0));
-    NZCP_CUDA(cudaEventSynchronize(e1));
-    NZCP_CUDA(cudaEventElapsedTime(&diff_ms, e0, e1));
-    hs.points_device(diff.d, diff.n);
+  {
+    Exec staged(diff.ex.host());   // tauG1, freed once the differences are hashed
+    G1Affine* tau = staged.alloc<G1Affine>(N + diff.n);
+    diff.d = diff.ex.alloc<G1Affine>(diff.n);   // N >= 2: at least one difference
+    staged.upload(tau, pt.s[2].p, (N + diff.n) * 64);
+    Timer t = staged.timer();
+    staged.run<128>(diff.n, HDifference{tau, N, diff.d});
+    diff_ms = t.stop();
+    hs.points(diff.d, diff.n);
   }
   hs.u32be((uint32_t)(m - np - 1));
   hs.section<Fq>(zi.s[8].p, m - np - 1);
@@ -389,29 +378,24 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   ChaCha rng(sd);
   const uint64_t N = z.domain_size, n_l = z.n_l();
   std::vector<Fr> sc(std::max(n_l, N));
-  CudaResources res;
-  const cudaEvent_t e0 = res.event(), e1 = res.event();
+  Exec ex(false);
   auto timed = [&](float& acc_ms, auto&& fn) {   // device time of fn's work on the default stream, added to acc_ms
-    NZCP_CUDA(cudaEventRecord(e0, 0));
+    Timer t = ex.timer();
     const G1Affine r = fn();
-    NZCP_CUDA(cudaEventRecord(e1, 0));
-    NZCP_CUDA(cudaEventSynchronize(e1));
-    float t = 0;
-    NZCP_CUDA(cudaEventElapsedTime(&t, e0, e1));
-    acc_ms += t;
+    acc_ms += t.stop();
     return r;
   };
 
   // 5. L: sum rho_i L_init[i] and sum rho_i L[i]
   if (n_l) {
     for (uint64_t i = 0; i < n_l; i++) sc[i] = fp_from_rng<FrParams>(rng);
-    CudaResources l_res;
-    Fr* d_sc = l_res.device<Fr>(n_l);
-    G1Affine* d_b = l_res.device<G1Affine>(n_l);
-    NZCP_CUDA(cudaMemcpy(d_sc, sc.data(), n_l * sizeof(Fr), cudaMemcpyHostToDevice));
-    NZCP_CUDA(cudaMemcpy(d_b, zi.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
+    Exec l_ex(false);
+    Fr* d_sc = l_ex.alloc<Fr>(n_l);
+    G1Affine* d_b = l_ex.alloc<G1Affine>(n_l);
+    l_ex.upload(d_sc, sc.data(), n_l * sizeof(Fr));
+    l_ex.upload(d_b, zi.s[8].p, n_l * 64);
     const G1Affine r1 = timed(ms[2], [&] { return msm_g1(d_b, d_sc, n_l); });
-    NZCP_CUDA(cudaMemcpy(d_b, z.s[8].p, n_l * 64, cudaMemcpyHostToDevice));
+    l_ex.upload(d_b, z.s[8].p, n_l * 64);
     const G1Affine r2 = timed(ms[2], [&] { return msm_g1(d_b, d_sc, n_l); });
     cl.add(11, -1, r1, r2, delta2, delta2_init);
   }
@@ -419,19 +403,18 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   // 6. H: r_(N-1) = 0, R1 over the differences i <= N - 2, r' = Fr.fft(-2 w_2N^m r_m), R2 over section 9
   for (uint64_t i = 0; i + 1 < N; i++) sc[i] = fp_from_rng<FrParams>(rng);
   sc[N - 1] = Fr::zero();
-  Fr* d_r = res.device<Fr>(N);
-  Fr* d_tmp = res.device<Fr>(N);
-  G1Affine* d_h = res.device<G1Affine>(N);
-  NZCP_CUDA(cudaMemcpy(d_r, sc.data(), N * sizeof(Fr), cudaMemcpyHostToDevice));
-  NZCP_CUDA(cudaMemcpy(d_h, z.s[9].p, N * 64, cudaMemcpyHostToDevice));
+  Fr* d_r = ex.alloc<Fr>(N);
+  Fr* d_tmp = ex.alloc<Fr>(N);
+  G1Affine* d_h = ex.alloc<G1Affine>(N);
+  ex.upload(d_r, sc.data(), N * sizeof(Fr));
+  ex.upload(d_h, z.s[9].p, N * 64);
   NttDomain dom;
   ntt_domain_create(&dom, (int)in.cir_power, 0);
   const G1Affine r1 = timed(ms[3], [&] { return msm_g1(diff.d, d_r, N - 1); });
   Fr two = Fr::zero();
   two.v[0] = 2;
   const G1Affine r2 = timed(ms[3], [&] {
-    h_scalar_kernel<<<div_up(N, 256), 256>>>(d_r, N, host_fr_root((int)in.cir_power + 1), fp_neg(fp_to_mont(two)));
-    NZCP_LAUNCH_CHECK();
+    ex.run<256>(N, HScalar{d_r, host_fr_root((int)in.cir_power + 1), fp_neg(fp_to_mont(two))});
     ntt_forward(dom, d_r, d_tmp, 0);
     return msm_g1(d_h, d_r, N);
   });
@@ -468,8 +451,8 @@ void run(Inputs& in, const uint8_t* init_hash_or_null, const Out& o) {
   fill_records(in, o.records);
   float ms[4] = {0, 0, 0, 0};
   Claims cl{o.claims};
-  HDiff diff;
-  circuit_hash(in.init, in.pt, false, rep.cs_hash, diff, &ms[0], &ms[1]);
+  HDiff diff(false);
+  circuit_hash(in.init, in.pt, rep.cs_hash, diff, &ms[0], &ms[1]);
   try {
     verify_checks(in, init_hash_or_null ? init_hash_or_null : rep.cs_hash, o.seed, cl, diff, ms);
   } catch (const Verdict& v) {
@@ -497,8 +480,8 @@ int nzcp_zkey_circuit_hash(const uint8_t* init, size_t init_len, const uint8_t* 
     const Ptau pt = parse_ptau(ptau, ptau_len);
     check_ptau_for(pt, zkey_domain_power(zi));
     use_device(device);
-    HDiff diff;
-    circuit_hash(zi, pt, false, hash, diff, ms, ms ? ms + 1 : nullptr);
+    HDiff diff(false);
+    circuit_hash(zi, pt, hash, diff, ms, ms ? ms + 1 : nullptr);
   });
 }
 
@@ -510,8 +493,8 @@ int nzcp_host_zkey_circuit_hash(const uint8_t* init, size_t init_len, const uint
     const Ptau pt = parse_ptau(ptau, ptau_len);
     check_ptau_for(pt, zkey_domain_power(zi));
     if (zi.domain_size > kHostMaxPoints) throw ApiError(NZCP_E_ARG, "zkey: the host run is limited to 4096 H points");
-    HDiff diff;
-    circuit_hash(zi, pt, true, hash, diff, nullptr, nullptr);
+    HDiff diff(true);
+    circuit_hash(zi, pt, hash, diff, nullptr, nullptr);
   });
 }
 
