@@ -27,6 +27,7 @@
  *   nzcp_ptau_new*, nzcp_ptau_contribute*, nzcp_ptau_beacon
  *                       snarkjs powersoftau_new.js newAccumulator, powersoftau_contribute.js contribute and
  *                       powersoftau_beacon.js beacon, with keypair.js createPTauKey (yarn.lock:987-999)
+ *   nzcp_ptau_verify*   snarkjs powersoftau_verify.js verify (yarn.lock:987-999); the pairings stay with the caller
  *   nzcp_zkey_contribute*, nzcp_zkey_beacon
  *                       snarkjs zkey_contribute.js phase2contribute and zkey_beacon.js beacon, with the ChaCha of
  *                       ffjavascript random.js (yarn.lock:987-999, 408-416)
@@ -268,6 +269,55 @@ int nzcp_zkey_verify_from_r1cs(const uint8_t* r1cs, size_t r1cs_len, const uint8
                                size_t claims_cap, nzcp_zkey_contribution* records, size_t records_cap,
                                nzcp_zkey_verify_report* report, float section_ms[4]);
 
+/* snarkjs `powersoftau verify` (powersoftau_verify.js verify(tauFilename); csrc/ptau_verify.cu restates it): the
+ * contributions of section 7, the powers of sections 2-6, the last record's next challenge and, for a prepared file
+ * (sections 12-15 all present), the Lagrange sections.  As for nzcp_zkey_verify_*, the pairings are left to the caller: the
+ * library stops at the first check it decides that fails (report->failed_step != 0, report->message) and returns each
+ * pairing check before that point as a claim e(a, d) = e(b, c), in order; the verdict is the first false claim, else the
+ * library's failure, else true.  Record ids in the messages are index + 1 ("challenge #id").
+ * Steps (failed_step and claim.step; record = section-7 index, else -1):
+ *   1 a point of sections 2-6, 12-15 or of a record that is not canonical and on its curve, or a record's g2_spx / tauG2 /
+ *     betaG2 or a random combination of the tauG2 section outside the order-r subgroup of G2 (snarkjs checks none of this)
+ *   2 "This file has no contribution! It cannot be used in production"
+ *   3 "BEACON key (tauG1_s | tauG1_sx | alphaG1_s | ... | betaG2_spx) is not generated correctly in challenge #id  name"
+ *   4, 5, 6 claims "INVALID key (tau | alpha | beta) in challenge #id"
+ *   7, 8, 9, 10, 11 claims "INVALID tau*G1 | tau*G2 | alpha*G1 | beta*G1 | beta*G2. challenge #id It does not follow the
+ *     previous contribution"
+ *   12, 13, 14, 15 claims "tauG1 | tauG2 | alphaTauG1 | betaTauG1 section. Powers do not match"
+ *   16 a first element of sections 2-6 ("First element of tau*G1 section must be the generator", ...)
+ *   17 "Hash of the values does not match the next challenge of the last contributor in the contributions section" (only
+ *     when power == ceremonyPower; a reduced file skips it)
+ *   18 "Phase2 caclutation does not match with powers of tau"   (snarkjs's spellings)
+ * Deviations: the random combinations draw full-width scalars (snarkjs: 32-bit) from a ChaCha seeded by 32 OS-random bytes
+ * or by `seed` (32 bytes, test hook; NULL in use); the points of step 1.
+ * Errors (before any device work): the file rejections of nzcp_ptau_contribute except the point checks (a bad point is a
+ * false verdict) and the reduced-file check; sections 12-15 whose size does not match the power, ceremonyPower outside
+ * [power, 28], a partialHash with c > 128, t >= 2^64 or outlen != 64, a beacon record without its parameters
+ * (NZCP_E_FORMAT); a prepared file of power 28 (NZCP_E_ARG).
+ * nzcp_ptau_verify_size (host-only) gives the claim and record counts the buffers must hold (8 n + 4 and n).
+ * ms (optional): [0] host point checks, [1] device time of the encode kernels, [2] host BLAKE2b of the next challenge,
+ * [3] device time of the section MSMs, [4] device time of the Lagrange transforms and MSMs. */
+typedef struct nzcp_ptau_contribution {
+  uint8_t response_hash[64];   /* BLAKE2b-512 resumed from partialHash over the public key: the hash snarkjs prints */
+  uint8_t next_challenge[64];  /* as the record stores it */
+  uint32_t type;               /* 0 contribute, 1 beacon */
+  uint32_t num_iterations_exp, name_len, beacon_hash_len;
+  char name[256];              /* parameter tag 1, not NUL-terminated */
+  uint8_t beacon_hash[256];    /* parameter tag 3 */
+} nzcp_ptau_contribution;
+typedef struct nzcp_ptau_verify_report {
+  int32_t failed_step;         /* 0: every check the library decides passed */
+  int32_t failed_record;       /* section-7 index for steps 1 (a record's point) and 3, else -1 */
+  char message[256];
+  uint32_t n_contributions, n_claims;
+  uint32_t prepared;           /* sections 12-15 present (and checked); 0: snarkjs only warns */
+  uint8_t next_challenge[64];  /* the computed next challenge, once sections 2-6 were hashed */
+} nzcp_ptau_verify_report;
+int nzcp_ptau_verify_size(const uint8_t* ptau, size_t len, size_t* n_claims, size_t* n_records);
+int nzcp_ptau_verify(const uint8_t* ptau, size_t len, const uint8_t* seed, int device, nzcp_zkey_verify_claim* claims,
+                     size_t claims_cap, nzcp_ptau_contribution* records, size_t records_cap, nzcp_ptau_verify_report* report,
+                     float ms[5]);
+
 /* Work buffers + streams for proofs against `zk`.  Several provers may share one zkey (one per host thread). */
 int nzcp_prover_create(nzcp_zkey* zk, nzcp_prover** out);   /* = mode 0 */
 /* mode 0 = latency (one proof at a time), mode 1 = throughput (meant to run beside other provers on the same GPU;
@@ -405,6 +455,12 @@ int nzcp_host_zkey_contribute(const uint8_t* zkey, size_t len, const char* name,
 int nzcp_host_ptau_contribute(const uint8_t* ptau, size_t len, const char* name, const uint8_t* entropy, size_t entropy_len,
                               const uint8_t* seed, const uint8_t* beacon_hash, size_t beacon_hash_len,
                               uint32_t num_iterations_exp, uint8_t* out, size_t cap, size_t* written, uint8_t hash[64]);
+
+/* nzcp_ptau_verify with the kernels' per-point code (encodings, scalar transforms) and the MSMs' code (nzcp_host_msm_sim)
+ * run on the CPU, for power <= 4 (more: NZCP_E_ARG).  Same validation, same report, records and claims. */
+int nzcp_host_ptau_verify(const uint8_t* ptau, size_t len, const uint8_t* seed, nzcp_zkey_verify_claim* claims,
+                          size_t claims_cap, nzcp_ptau_contribution* records, size_t records_cap,
+                          nzcp_ptau_verify_report* report);
 
 /* nzcp_zkey_circuit_hash with the kernels' per-point code (H differences, point encoding) run on the CPU, for a domain of
  * at most 4096 (more: NZCP_E_ARG).  Same validation, same hash. */

@@ -65,6 +65,18 @@ class VerifyReport(C.Structure):
                 ("n_contributions", C.c_uint32), ("n_claims", C.c_uint32), ("cs_hash", C.c_uint8 * 64)]
 
 
+class PtauContribution(C.Structure):
+    _fields_ = [("response_hash", C.c_uint8 * 64), ("next_challenge", C.c_uint8 * 64), ("type", C.c_uint32),
+                ("num_iterations_exp", C.c_uint32), ("name_len", C.c_uint32), ("beacon_hash_len", C.c_uint32),
+                ("name", C.c_uint8 * 256), ("beacon_hash", C.c_uint8 * 256)]
+
+
+class PtauVerifyReport(C.Structure):
+    _fields_ = [("failed_step", C.c_int32), ("failed_record", C.c_int32), ("message", C.c_char * 256),
+                ("n_contributions", C.c_uint32), ("n_claims", C.c_uint32), ("prepared", C.c_uint32),
+                ("next_challenge", C.c_uint8 * 64)]
+
+
 # every symbol include/nzcp_prover.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 _U8P = C.c_void_p          # raw byte pointers are passed as addresses / buffers
@@ -112,6 +124,10 @@ SIGNATURES = {
     "nzcp_zkey_verify_from_r1cs": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, _U8P, C.c_size_t, _U8P, C.c_int,
                                              C.POINTER(VerifyClaim), C.c_size_t, C.POINTER(Contribution), C.c_size_t,
                                              C.POINTER(VerifyReport), C.POINTER(C.c_float)]),
+    "nzcp_ptau_verify_size": (C.c_int, [_U8P, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
+    "nzcp_ptau_verify": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_int, C.POINTER(VerifyClaim), C.c_size_t,
+                                   C.POINTER(PtauContribution), C.c_size_t, C.POINTER(PtauVerifyReport),
+                                   C.POINTER(C.c_float)]),
     "nzcp_msm_plan_create": (C.c_int, [_U8P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(_P),
                                        C.POINTER(C.c_float)]),
     "nzcp_msm_plan_free": (None, [_P]),
@@ -135,6 +151,8 @@ SIGNATURES = {
                                             C.c_uint32, _U8P, C.c_size_t, C.POINTER(C.c_size_t), _U8P]),
     "nzcp_host_ptau_contribute": (C.c_int, [_U8P, C.c_size_t, C.c_char_p, _U8P, C.c_size_t, _U8P, _U8P, C.c_size_t,
                                             C.c_uint32, _U8P, C.c_size_t, C.POINTER(C.c_size_t), _U8P]),
+    "nzcp_host_ptau_verify": (C.c_int, [_U8P, C.c_size_t, _U8P, C.POINTER(VerifyClaim), C.c_size_t,
+                                        C.POINTER(PtauContribution), C.c_size_t, C.POINTER(PtauVerifyReport)]),
     "nzcp_host_zkey_circuit_hash": (C.c_int, [_U8P, C.c_size_t, _U8P, C.c_size_t, _U8P]),
     "nzcp_host_msm_sim": (C.c_int, [_U8P, _U8P, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, _U8P]),
     "nzcp_tuning_set": (C.c_int, [C.c_char_p, C.c_int]),

@@ -377,6 +377,25 @@ def _plain_g2(b):
     return None if not any(c) else ((c[0], c[1]), (c[2], c[3]))
 
 
+def _verdict(claims, rep, message_of, timings):
+    """The split verdict of `zkey verify` / `powersoftau verify`: the claims the library returned are checked in order on
+    the CPU (verifier.same_ratio); the first false one gives message_of(claim), else the library's failure message, else
+    None (the file verifies).  timings["pairings"] (host ms), when timings is a dict."""
+    import time
+    from . import verifier
+    t0 = time.perf_counter()
+    message = None
+    for k in claims[:rep.n_claims]:
+        if not verifier.same_ratio(_plain_g1(k.a), _plain_g1(k.b), _plain_g2(k.c), _plain_g2(k.d)):
+            message = message_of(k)
+            break
+    if timings is not None:
+        timings["pairings"] = (time.perf_counter() - t0) * 1e3
+    if message is None and rep.failed_step:
+        message = rep.message.decode(errors="replace")
+    return message
+
+
 def zkey_verify(zkey, ptau, *, r1cs=None, init=None, seed=None, device=0, timings=None):
     """snarkjs `zkey verify`: checks `zkey` against the circuit, given as the .r1cs (verifyFromR1cs) or as the initial key
     (verifyFromInit), and the prepared ptau (all: path | bytes-like | {"type": "mem"}).  The library runs every check but
@@ -384,8 +403,6 @@ def zkey_verify(zkey, ptau, *, r1cs=None, init=None, seed=None, device=0, timing
     on the CPU (verifier.same_ratio).  -> dict(ok, message, cs_hash, contributions=[dict(type, name, hash,
     beacon_hash, num_iterations_exp)]).  `seed` (32 bytes, tests) replaces the OS randomness of the L / H scalars;
     `timings` receives VERIFY_TIMINGS in ms plus "pairings" (host ms)."""
-    import time
-    from . import verifier
     if (r1cs is None) == (init is None):
         raise NzcpError(_lib.NZCP_E_ARG, "zkey_verify: give exactly one of r1cs and init")
     if seed is not None and len(bytes(seed)) != 32:
@@ -406,17 +423,10 @@ def zkey_verify(zkey, ptau, *, r1cs=None, init=None, seed=None, device=0, timing
         fn = lib.nzcp_zkey_verify_from_init
     check(fn(addr(cb), _nbytes(cb), addr(pb), _nbytes(pb), addr(zb), _nbytes(zb), sd, int(device), claims,
              n_claims.value, recs, n_recs.value, C.byref(rep), ms))
-    t0 = time.perf_counter()
-    message = None
-    for k in claims[:rep.n_claims]:
-        if not verifier.same_ratio(_plain_g1(k.a), _plain_g1(k.b), _plain_g2(k.c), _plain_g2(k.d)):
-            message = CLAIM_MESSAGES[k.step] % k.record if "%d" in CLAIM_MESSAGES[k.step] else CLAIM_MESSAGES[k.step]
-            break
+    message = _verdict(claims, rep, lambda k: CLAIM_MESSAGES[k.step] % k.record if "%d" in CLAIM_MESSAGES[k.step]
+                       else CLAIM_MESSAGES[k.step], timings)
     if timings is not None:
         timings.update(zip(VERIFY_TIMINGS, [float(x) for x in ms]))
-        timings["pairings"] = (time.perf_counter() - t0) * 1e3
-    if message is None and rep.failed_step:
-        message = rep.message.decode(errors="replace")
     contributions = [{"type": r.type, "name": bytes(r.name[:r.name_len]).decode(errors="replace"), "hash": bytes(r.hash),
                       "beacon_hash": bytes(r.beacon_hash[:r.beacon_hash_len]), "num_iterations_exp": r.num_iterations_exp}
                      for r in recs[:n_recs.value]]
@@ -571,6 +581,75 @@ def host_ptau_contribute(ptau, name=None, entropy=None, seed=None, beacon_hash=N
                                         int(num_iterations_exp), addr(out), len(out), C.byref(written), addr(h)))
     assert written.value == len(out)
     return out, bytes(h)
+
+
+PTAU_VERIFY_TIMINGS = ("point_checks", "encode", "blake2b", "section_msm", "lagrange")
+PTAU_CLAIM_MESSAGES = {4: "INVALID key (tau) in challenge #%d", 5: "INVALID key (alpha) in challenge #%d",
+                       6: "INVALID key (beta) in challenge #%d",
+                       7: "INVALID tau*G1. challenge #%d It does not follow the previous contribution",
+                       8: "INVALID tau*G2. challenge #%d It does not follow the previous contribution",
+                       9: "INVALID alpha*G1. challenge #%d It does not follow the previous contribution",
+                       10: "INVALID beta*G1. challenge #%d It does not follow the previous contribution",
+                       11: "INVALID beta*G2. challenge #%d It does not follow the previous contribution",
+                       12: "tauG1 section. Powers do not match", 13: "tauG2 section. Powers do not match",
+                       14: "alphaTauG1 section. Powers do not match", 15: "betaTauG1 section. Powers do not match"}
+
+
+def _ptau_claim_message(k):
+    m = PTAU_CLAIM_MESSAGES[k.step]
+    return m % (k.record + 1) if "%d" in m else m
+
+
+def _ptau_verify(ptau, seed, run):
+    """Shared part of ptau_verify / host_ptau_verify: buffers, the call run(pb, sd, claims, n_claims, recs, n_recs, rep),
+    the verdict."""
+    if seed is not None and len(bytes(seed)) != 32:
+        raise NzcpError(_lib.NZCP_E_ARG, "seed must be 32 bytes")
+    lib = _lib.load()
+    pb = _as_bytes_like(ptau)
+    n_claims, n_recs = C.c_size_t(), C.c_size_t()
+    check(lib.nzcp_ptau_verify_size(addr(pb), _nbytes(pb), C.byref(n_claims), C.byref(n_recs)))
+    claims = (_lib.VerifyClaim * n_claims.value)()
+    recs = (_lib.PtauContribution * max(1, n_recs.value))()
+    rep = _lib.PtauVerifyReport()
+    check(run(lib, pb, None if seed is None else bytes(seed), claims, n_claims.value, recs, n_recs.value, rep))
+    contributions = [{"type": r.type, "name": bytes(r.name[:r.name_len]).decode(errors="replace"),
+                      "response_hash": bytes(r.response_hash), "next_challenge": bytes(r.next_challenge),
+                      "beacon_hash": bytes(r.beacon_hash[:r.beacon_hash_len]), "num_iterations_exp": r.num_iterations_exp}
+                     for r in recs[:n_recs.value]]
+    return claims, rep, contributions
+
+
+def ptau_verify(ptau, seed=None, device=0, timings=None):
+    """snarkjs `powersoftau verify`: checks a phase-1 .ptau (path | bytes-like | {"type": "mem"}), its contributions and,
+    when prepared, its Lagrange sections (csrc/ptau_verify.cu).  The library runs every check but the pairings on the GPU
+    and returns the pairing claims that precede its first failure; they are checked here, in order, on the CPU.
+    -> dict(ok, message, prepared, next_challenge (computed; None when not reached), contributions=[dict(type, name,
+    response_hash, next_challenge, beacon_hash, num_iterations_exp)]).  `seed` (32 bytes, tests) replaces the OS
+    randomness of the random combinations; `timings` receives PTAU_VERIFY_TIMINGS in ms plus "pairings" (host ms)."""
+    ms = (C.c_float * 5)()
+    claims, rep, contributions = _ptau_verify(
+        ptau, seed, lambda lib, pb, sd, cl, ncl, recs, nrec, rep: lib.nzcp_ptau_verify(
+            addr(pb), _nbytes(pb), sd, int(device), cl, ncl, recs, nrec, C.byref(rep), ms))
+    if timings is not None:
+        timings.update(zip(PTAU_VERIFY_TIMINGS, [float(x) for x in ms]))
+    return _ptau_result(claims, rep, contributions, timings)
+
+
+def host_ptau_verify(ptau, seed=None):
+    """CPU run of ptau_verify (power <= 4): the kernels' per-point code and the MSMs' code (host_msm_sim) on the CPU ->
+    the same dict; test hook."""
+    claims, rep, contributions = _ptau_verify(
+        ptau, seed, lambda lib, pb, sd, cl, ncl, recs, nrec, rep: lib.nzcp_host_ptau_verify(
+            addr(pb), _nbytes(pb), sd, cl, ncl, recs, nrec, C.byref(rep)))
+    return _ptau_result(claims, rep, contributions, None)
+
+
+def _ptau_result(claims, rep, contributions, timings):
+    message = _verdict(claims, rep, _ptau_claim_message, timings)
+    reached = rep.failed_step == 0 or rep.failed_step >= 17
+    return {"ok": message is None, "message": message, "prepared": bool(rep.prepared),
+            "next_challenge": bytes(rep.next_challenge) if reached else None, "contributions": contributions}
 
 
 def zkey_selfcheck(zkey, device=0):

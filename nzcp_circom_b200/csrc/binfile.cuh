@@ -134,6 +134,10 @@ inline uint32_t zkey_domain_power(const Zkey& z) {
 // prepared file.
 constexpr size_t kPtauHeaderLen = 4 + 32 + 4 + 4;
 constexpr uint32_t kPtauMaxPower = 28;
+// Why no Lagrange sections exist at the top power (`prepare phase2` and `powersoftau verify` reject such files).
+constexpr const char* kPtauPower28Phase2 = "ptau: power 28 is not supported: its top tauG1 level has 2^29 points, more "
+                                           "than the 2^28 roots of unity of Fr, and needs the coset branch of snarkjs's "
+                                           "lagrangeEvaluations";
 
 struct Ptau {
   Sect s[16];

@@ -44,6 +44,25 @@ extern thread_local std::atomic<uint64_t>* t_launch_sink;
 
 static inline unsigned div_up(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
 
+HD int ilog2_u64(uint64_t v) {   // v > 0
+#ifdef __CUDA_ARCH__
+  return 63 - __clzll((long long)v);
+#else
+  return 63 - __builtin_clzll(v);
+#endif
+}
+
+HD uint64_t bitrev_bits(uint64_t x, int bits) {
+  if (bits == 0) return 0;
+#ifdef __CUDA_ARCH__
+  return __brevll(x) >> (64 - bits);
+#else
+  uint64_t r = 0;
+  for (int i = 0; i < bits; i++, x >>= 1) r = (r << 1) | (x & 1);
+  return r;
+#endif
+}
+
 // Owner of CUDA device memory, pinned host memory, events and streams.  Each acquire call returns the raw pointer or
 // handle, which the caller keeps in plain non-owning fields; the destructor releases everything in reverse order of
 // acquisition, ignoring return codes (it runs during unwinding).  Sizes are exactly what the caller asks for.
@@ -318,5 +337,10 @@ void msm_sum_points(const void* d_pts, uint32_t count, bool g2, void* d_result, 
 G1XYZZ msm_run_finish_g1(const MsmRun* r);
 G2XYZZ msm_run_finish_g2(const MsmRun* r);
 float msm_run_accumulate_ms(const MsmRun* r);
+// standalone.cu: the MSM data path (window table, signed digits, c-bit buckets, `rounds` pair rounds of k additions per
+// thread, running-sum reduction) run on the CPU with the kernels' own code; instantiated for Fq and Fq2.  Montgomery affine
+// bases, plain scalars (>= r: NZCP_E_RANGE).
+template <class F>
+XYZZ<F> host_msm_sim(const uint8_t* bases, const uint8_t* scalars, size_t n, int c, int rounds, int k);
 
 }  // namespace nzcp

@@ -1,7 +1,8 @@
 // Code shared by the ceremony entry points (contribute.cu `zkey contribute` / `zkey beacon`, verify.cu `zkey verify`,
-// setup.cu `zkey new`, ptau_contribute.cu `powersoftau new` / `contribute` / `beacon`): BLAKE2b-512 and SHA-256,
-// ffjavascript's ChaCha, F/G.fromRng, the uncompressed and compressed point encodings (host and device) with the chunked
-// point hasher, and the contribution records with the .zkey input of `zkey contribute` / `zkey verify`.
+// setup.cu `zkey new`, ptau_contribute.cu `powersoftau new` / `contribute` / `beacon`, ptau_verify.cu `powersoftau verify`):
+// BLAKE2b-512 and SHA-256, ffjavascript's ChaCha, F/G.fromRng, the uncompressed and compressed point encodings (host and
+// device) with the chunked point hasher, the contribution records with the .zkey input of `zkey contribute` / `zkey
+// verify`, the phase-1 key, and the claims and chunked MSM sums of the two verify steps.
 #pragma once
 #include <sys/random.h>
 
@@ -79,6 +80,16 @@ struct Blake2b512 {   // RFC 7693, unkeyed, 64-byte digest
     memcpy(out + 192, tt, 16);
     memcpy(out + 208, &c, 4);
     memcpy(out + 212, &outlen, 4);
+  }
+  // The inverse of partial(): the hasher a partialHash describes, to be resumed with update().  The caller has checked
+  // c <= 128, t[1] = 0 and outlen = 64.
+  static Blake2b512 from_partial(const uint8_t in[216]) {
+    Blake2b512 s;
+    memcpy(s.buf, in, 128);
+    memcpy(s.h, in + 128, 64);
+    memcpy(&s.t, in + 192, 8);
+    s.n = rd32u(in + 208);
+    return s;
   }
 };
 
@@ -637,6 +648,224 @@ struct Hasher {
     points(x, n);
   }
 };
+
+// ------------------------------------------------------------------------------------------------ phase-1 keys and records
+constexpr size_t kPubKeyLen = 6 * 64 + 3 * 128;                               // 768
+constexpr size_t kPartialLen = 216;
+// pubkey tauG1 tauG2 alphaG1 betaG1 betaG2 partialHash nextChallenge type paramLength
+constexpr size_t kPtauRecFixed = kPubKeyLen + 3 * 64 + 2 * 128 + kPartialLen + 64 + 4 + 4;   // 1504
+
+// calculateFirstChallengeHash; blake_ms += the host time.  A caller that no longer needs the hash may set *cancel: the
+// pass then stops within 1024 points and `out` is meaningless.
+void first_challenge(uint32_t power, uint8_t out[64], float* blake_ms, const std::atomic<bool>* cancel = nullptr) {
+  const auto t0 = std::chrono::steady_clock::now();
+  Blake2b512 h;
+  uint8_t empty[64];
+  Blake2b512().final(empty);
+  h.update(empty, 64);
+  const G1Affine g1 = g1_generator();
+  const G2Affine g2 = g2_generator();
+  constexpr int kRep = 1024;
+  std::vector<uint32_t> r1(kRep * 16), r2(kRep * 32);
+  for (int i = 0; i < kRep; i++) {
+    u_encode(g1, r1.data() + 16 * i);
+    u_encode(g2, r2.data() + 32 * i);
+  }
+  auto block = [&](const std::vector<uint32_t>& r, size_t psz, uint64_t count) {
+    for (uint64_t i = 0; i < count && !(cancel && cancel->load(std::memory_order_relaxed)); i += kRep)
+      h.update(r.data(), std::min<uint64_t>(kRep, count - i) * psz);
+  };
+  const uint64_t n = (uint64_t)1 << power;
+  block(r1, 64, 2 * n - 1);
+  block(r2, 128, n);
+  block(r1, 64, n);
+  block(r1, 64, n);
+  block(r2, 128, 1);
+  h.final(out);
+  if (blake_ms) *blake_ms += std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+}
+
+// One of tau, alpha, beta (keypair.js calculatePubKey).
+struct KeyPart {
+  Fr prv;   // Montgomery
+  G1Affine g1_s, g1_sx;
+  G2Affine g2_sp, g2_spx;
+};
+
+void create_key(ChaCha& rng, const uint8_t challenge[64], KeyPart k[3]) {
+  for (int j = 0; j < 3; j++) {
+    k[j].prv = fp_from_rng<FrParams>(rng);
+    if (k[j].prv.is_zero()) throw ApiError(NZCP_E_INTERNAL, "ptau contribute: the rng drew a zero key");
+  }
+  const Fq b1 = curve_b(g1_generator());
+  for (int j = 0; j < 3; j++) {
+    const Fr kp = fp_from_mont(k[j].prv);
+    k[j].g1_s = point_from_rng(rng, b1, nullptr);
+    k[j].g1_sx = mul_plain(k[j].g1_s, kp.v);
+    Blake2b512 h;
+    const uint8_t pers = (uint8_t)j;
+    h.update(&pers, 1);
+    h.update(challenge, 64);
+    hash_g1(h, reinterpret_cast<const uint8_t*>(&k[j].g1_s));
+    hash_g1(h, reinterpret_cast<const uint8_t*>(&k[j].g1_sx));
+    uint8_t d[64];
+    h.final(d);
+    k[j].g2_sp = hash_to_g2(d);
+    k[j].g2_spx = mul_plain(k[j].g2_sp, kp.v);
+  }
+}
+
+// toPtauPubKeyRpr order, Montgomery affine (montgomery = true) or uncompressed (false).
+void pub_key(const KeyPart k[3], bool montgomery, uint8_t out[kPubKeyLen]) {
+  for (int j = 0; j < 3; j++) {
+    if (montgomery) {
+      memcpy(out + 128 * j, &k[j].g1_s, 64);
+      memcpy(out + 128 * j + 64, &k[j].g1_sx, 64);
+      memcpy(out + 384 + 128 * j, &k[j].g2_spx, 128);
+    } else {
+      u_encode(k[j].g1_s, reinterpret_cast<uint32_t*>(out + 128 * j));
+      u_encode(k[j].g1_sx, reinterpret_cast<uint32_t*>(out + 128 * j + 64));
+      u_encode(k[j].g2_spx, reinterpret_cast<uint32_t*>(out + 384 + 128 * j));
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ verification
+// `zkey verify` (verify.cu) and `powersoftau verify` (ptau_verify.cu): the library decides every check but the pairings and
+// returns each pairing check before its first failure as a claim e(a, d) = e(b, c), for the caller to check in order.
+struct Verdict {   // the first failed check the library decides
+  int step, record;
+  std::string msg;
+};
+
+// A record parse_records accepted: rec_fixed bytes ending in u32 type, u32 paramLength, then the parameters.
+struct Rec {
+  const uint8_t* p;
+  uint32_t type, exp = 0;
+  const uint8_t *name = nullptr, *beacon = nullptr;
+  size_t name_len = 0, beacon_len = 0;
+};
+
+// kind: "zkey" or "ptau", for the message.
+Rec read_record(const uint8_t* r, size_t rec_fixed, const char* kind) {
+  Rec c{r, rd32u(r + rec_fixed - 8)};
+  const uint8_t* q = r + rec_fixed;
+  const uint8_t* end = q + rd32u(r + rec_fixed - 4);
+  while (q < end) {   // parse_records has checked the layout
+    const int tag = *q++;
+    if (tag == 2) {
+      c.exp = *q++;
+    } else {
+      const size_t l = *q++;
+      (tag == 1 ? c.name : c.beacon) = q;
+      (tag == 1 ? c.name_len : c.beacon_len) = l;
+      q += l;
+    }
+  }
+  if (c.type == 1 && (!c.beacon || c.beacon_len == 0 || c.exp > 63))
+    throw ApiError(NZCP_E_FORMAT, std::string(kind) + ": beacon record without a beacon hash or with numIterationsExp > 63");
+  return c;
+}
+
+template <class F>
+Affine<F> load_pt(const uint8_t* p) {
+  Affine<F> a;
+  memcpy(&a, p, sizeof a);
+  return a;
+}
+
+bool in_g2_subgroup(const G2Affine& p) {
+  uint32_t r[8];
+  for (int i = 0; i < 8; i++) r[i] = FrParams::mod(i);
+  return xyzz_mul(G2XYZZ::from_affine(p), r).is_inf();
+}
+
+void plain_g1(const G1Affine& a, uint8_t* o) {
+  fp_to_bytes(fp_from_mont(a.x), o);
+  fp_to_bytes(fp_from_mont(a.y), o + 32);
+}
+void plain_g2(const G2Affine& a, uint8_t* o) {
+  fp_to_bytes(fp_from_mont(a.x.c0), o);
+  fp_to_bytes(fp_from_mont(a.x.c1), o + 32);
+  fp_to_bytes(fp_from_mont(a.y.c0), o + 64);
+  fp_to_bytes(fp_from_mont(a.y.c1), o + 96);
+}
+
+struct Claims {
+  nzcp_zkey_verify_claim* out;
+  size_t n = 0;
+  void add(int step, int record, const G1Affine& a, const G1Affine& b, const G2Affine& c, const G2Affine& d) {
+    nzcp_zkey_verify_claim& k = out[n++];
+    k.step = step;
+    k.record = record;
+    plain_g1(a, k.a);
+    plain_g1(b, k.b);
+    plain_g2(c, k.c);
+    plain_g2(d, k.d);
+  }
+};
+
+// The 32 bytes that seed the ChaCha of the random checks: the test seed, or OS randomness.  what: "zkey verify" / "ptau
+// verify", for the message.
+void verify_seed(const char* what, const uint8_t* seed, uint8_t out[32]) {
+  if (seed) {
+    memcpy(out, seed, 32);
+    return;
+  }
+  for (size_t got = 0; got < 32;) {
+    const ssize_t r = getrandom(out + got, 32 - got, 0);
+    if (r <= 0) throw ApiError(NZCP_E_INTERNAL, std::string(what) + ": no OS randomness");
+    got += (size_t)r;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ MSM
+constexpr uint64_t kMsmChunk = 1u << 22;   // bases per table-free MSM: the plan rejects windows x points >= 2^31
+
+template <class F>
+XYZZ<F> msm_finish(const MsmRun* r) {
+  if constexpr (sizeof(F) == sizeof(Fq)) return msm_run_finish_g1(r);
+  else return msm_run_finish_g2(r);
+}
+
+// out[b] = sum_i s_i P_b,i for k base arrays P_b (b < k) of n points against one vector of n plain scalars, all in the
+// executor's memory.  On the device: the table-free MSM of msm_plan.cu in chunks of at most kMsmChunk bases, one bucket
+// sort per chunk for all k runs, the chunk sums added.  On the host: host_msm_sim, the MSM kernels' code on the CPU.
+template <class F>
+void msm_sums(const Exec& ex, const Affine<F>* const* bases, int k, const Fr* scalars, uint64_t n, Affine<F>* out) {
+  std::vector<XYZZ<F>> acc(k, XYZZ<F>::inf());
+  for (uint64_t off = 0; off < n; off += kMsmChunk) {
+    const uint64_t m = std::min(kMsmChunk, n - off);
+    const int c = msm_pick_window_free(m);
+    if (ex.host()) {
+      for (int b = 0; b < k; b++)
+        xyzz_add(acc[b], host_msm_sim<F>(reinterpret_cast<const uint8_t*>(bases[b] + off),
+                                         reinterpret_cast<const uint8_t*>(scalars + off), m, c, msm_pick_rounds(m, c), 4));
+      continue;
+    }
+    MsmSort sort;
+    MsmRun run;
+    msm_sort_create(&sort, m, c, -1, true);
+    msm_run_create(&run, &sort, sizeof(F) != sizeof(Fq));
+    msm_sort_launch(&sort, scalars + off, m, 0);
+    for (int b = 0; b < k; b++) {
+      MsmTable tab;
+      msm_table_view(&tab, const_cast<Affine<F>*>(bases[b] + off), m, sizeof(F) != sizeof(Fq), c);
+      msm_run_launch(&run, &sort, &tab, 0);
+      NZCP_CUDA(cudaStreamSynchronize(0));
+      if (b == 0) msm_sort_check(&sort);
+      xyzz_add(acc[b], msm_finish<F>(&run));
+    }
+  }
+  for (int b = 0; b < k; b++) out[b] = xyzz_to_affine(acc[b]);
+}
+
+template <class F>
+Affine<F> msm_sum(const Exec& ex, const Affine<F>* bases, const Fr* scalars, uint64_t n) {
+  Affine<F> r;
+  msm_sums(ex, &bases, 1, scalars, n, &r);
+  return r;
+}
 
 }  // namespace
 }  // namespace nzcp

@@ -31,25 +31,6 @@
 namespace nzcp {
 
 // ------------------------------------------------------------------------------------------------ shared host/device code
-HD int ilog2_u64(uint64_t v) {   // v > 0
-#ifdef __CUDA_ARCH__
-  return 63 - __clzll((long long)v);
-#else
-  return 63 - __builtin_clzll(v);
-#endif
-}
-
-HD uint64_t bitrev_bits(uint64_t x, int bits) {
-  if (bits == 0) return 0;
-#ifdef __CUDA_ARCH__
-  return __brevll(x) >> (64 - bits);
-#else
-  uint64_t r = 0;
-  for (int i = 0; i < bits; i++, x >>= 1) r = (r << 1) | (x & 1);
-  return r;
-#endif
-}
-
 // tw[k] = w^k, plain form, for a Montgomery-form w
 HD Fr pow_u32_plain(Fr w, uint32_t e) {
   Fr r = Fr::one();
@@ -127,9 +108,7 @@ constexpr uint32_t kHostMaxPower = 4;
 // Everything preparePhase2 needs from its input, validated before any device work.
 Ptau parse_prepare_in(const uint8_t* b, size_t len) {
   const Ptau p = read_ptau(b, len);
-  if (p.power == kPtauMaxPower)
-    throw ApiError(NZCP_E_ARG, "ptau: power 28 is not supported: its top tauG1 level has 2^29 points, more than the 2^28 "
-                               "roots of unity of Fr, and needs the coset branch of snarkjs's lagrangeEvaluations");
+  if (p.power == kPtauMaxPower) throw ApiError(NZCP_E_ARG, kPtauPower28Phase2);
   check_ptau_sections(p);
   return p;
 }

@@ -71,10 +71,6 @@ struct PtauKey {   // Exec op
 namespace {
 
 constexpr uint32_t kHostMaxPower = 4;
-constexpr size_t kPubKeyLen = 6 * 64 + 3 * 128;                               // 768
-constexpr size_t kPartialLen = 216;
-// pubkey tauG1 tauG2 alphaG1 betaG1 betaG2 partialHash nextChallenge type paramLength
-constexpr size_t kPtauRecFixed = kPubKeyLen + 3 * 64 + 2 * 128 + kPartialLen + 64 + 4 + 4;   // 1504
 
 size_t new_size(uint32_t power) {
   size_t total = 12 + 7 * 12 + kPtauHeaderLen + 4;
@@ -105,79 +101,6 @@ size_t contribute_size(const ContribIn& p, size_t name_len, size_t beacon_len) {
   size_t total = 12 + 7 * 12 + kPtauHeaderLen;
   for (int id = 2; id <= 7; id++) total += p.s[id].len;
   return total + kPtauRecFixed + params_len(name_len, beacon_len);
-}
-
-// calculateFirstChallengeHash; blake_ms += the host time.
-void first_challenge(uint32_t power, uint8_t out[64], float* blake_ms) {
-  const auto t0 = std::chrono::steady_clock::now();
-  Blake2b512 h;
-  uint8_t empty[64];
-  Blake2b512().final(empty);
-  h.update(empty, 64);
-  const G1Affine g1 = g1_generator();
-  const G2Affine g2 = g2_generator();
-  constexpr int kRep = 1024;
-  std::vector<uint32_t> r1(kRep * 16), r2(kRep * 32);
-  for (int i = 0; i < kRep; i++) {
-    u_encode(g1, r1.data() + 16 * i);
-    u_encode(g2, r2.data() + 32 * i);
-  }
-  auto block = [&](const std::vector<uint32_t>& r, size_t psz, uint64_t count) {
-    for (uint64_t i = 0; i < count; i += kRep) h.update(r.data(), std::min<uint64_t>(kRep, count - i) * psz);
-  };
-  const uint64_t n = (uint64_t)1 << power;
-  block(r1, 64, 2 * n - 1);
-  block(r2, 128, n);
-  block(r1, 64, n);
-  block(r1, 64, n);
-  block(r2, 128, 1);
-  h.final(out);
-  if (blake_ms) *blake_ms += std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-}
-
-// One of tau, alpha, beta (keypair.js calculatePubKey).
-struct KeyPart {
-  Fr prv;   // Montgomery
-  G1Affine g1_s, g1_sx;
-  G2Affine g2_sp, g2_spx;
-};
-
-void create_key(ChaCha& rng, const uint8_t challenge[64], KeyPart k[3]) {
-  for (int j = 0; j < 3; j++) {
-    k[j].prv = fp_from_rng<FrParams>(rng);
-    if (k[j].prv.is_zero()) throw ApiError(NZCP_E_INTERNAL, "ptau contribute: the rng drew a zero key");
-  }
-  const Fq b1 = curve_b(g1_generator());
-  for (int j = 0; j < 3; j++) {
-    const Fr kp = fp_from_mont(k[j].prv);
-    k[j].g1_s = point_from_rng(rng, b1, nullptr);
-    k[j].g1_sx = mul_plain(k[j].g1_s, kp.v);
-    Blake2b512 h;
-    const uint8_t pers = (uint8_t)j;
-    h.update(&pers, 1);
-    h.update(challenge, 64);
-    hash_g1(h, reinterpret_cast<const uint8_t*>(&k[j].g1_s));
-    hash_g1(h, reinterpret_cast<const uint8_t*>(&k[j].g1_sx));
-    uint8_t d[64];
-    h.final(d);
-    k[j].g2_sp = hash_to_g2(d);
-    k[j].g2_spx = mul_plain(k[j].g2_sp, kp.v);
-  }
-}
-
-// toPtauPubKeyRpr order, Montgomery affine (montgomery = true) or uncompressed (false).
-void pub_key(const KeyPart k[3], bool montgomery, uint8_t out[kPubKeyLen]) {
-  for (int j = 0; j < 3; j++) {
-    if (montgomery) {
-      memcpy(out + 128 * j, &k[j].g1_s, 64);
-      memcpy(out + 128 * j + 64, &k[j].g1_sx, 64);
-      memcpy(out + 384 + 128 * j, &k[j].g2_spx, 128);
-    } else {
-      u_encode(k[j].g1_s, reinterpret_cast<uint32_t*>(out + 128 * j));
-      u_encode(k[j].g1_sx, reinterpret_cast<uint32_t*>(out + 128 * j + 64));
-      u_encode(k[j].g2_spx, reinterpret_cast<uint32_t*>(out + 384 + 128 * j));
-    }
-  }
 }
 
 // Upload, key op in place, response-hash the resident points, download; returns the key op's device ms.

@@ -410,7 +410,7 @@ static void sim_round(bool from_table, const std::vector<Affine<F>>& src, const 
 }
 
 template <class F>
-static XYZZ<F> host_msm_sim(const uint8_t* bases, const uint8_t* scalars, size_t n, int c, int rounds, int k) {
+XYZZ<F> host_msm_sim(const uint8_t* bases, const uint8_t* scalars, size_t n, int c, int rounds, int k) {
   const int n_windows = msm_num_windows(c);
   const uint32_t nb = 1u << (c - 1);
   std::vector<Affine<F>> table((size_t)n_windows * n + 1);
@@ -496,6 +496,8 @@ static XYZZ<F> host_msm_sim(const uint8_t* bases, const uint8_t* scalars, size_t
   }
   return tot;
 }
+template XYZZ<Fq> host_msm_sim<Fq>(const uint8_t*, const uint8_t*, size_t, int, int, int);
+template XYZZ<Fq2> host_msm_sim<Fq2>(const uint8_t*, const uint8_t*, size_t, int, int, int);
 
 }  // namespace nzcp
 

@@ -157,51 +157,6 @@ void circuit_hash(const ZkeyIn& zi, const Ptau& pt, uint8_t out[64], HDiff& diff
 }
 
 // ------------------------------------------------------------------------------------------------ verification
-struct Verdict {   // the first failed check this file decides
-  int step, record;
-  std::string msg;
-};
-
-struct Rec {
-  const uint8_t* p;
-  uint32_t type, exp = 0;
-  const uint8_t *name = nullptr, *beacon = nullptr;
-  size_t name_len = 0, beacon_len = 0;
-};
-
-Rec read_record(const uint8_t* r) {
-  Rec c{r, rd32u(r + 384)};
-  const uint8_t* q = r + kRecFixed;
-  const uint8_t* end = q + rd32u(r + 388);
-  while (q < end) {   // parse_mpc has checked the layout
-    const int tag = *q++;
-    if (tag == 2) {
-      c.exp = *q++;
-    } else {
-      const size_t l = *q++;
-      (tag == 1 ? c.name : c.beacon) = q;
-      (tag == 1 ? c.name_len : c.beacon_len) = l;
-      q += l;
-    }
-  }
-  if (c.type == 1 && (!c.beacon || c.beacon_len == 0 || c.exp > 63))
-    throw ApiError(NZCP_E_FORMAT, "zkey: beacon record without a beacon hash or with numIterationsExp > 63");
-  return c;
-}
-
-template <class F>
-Affine<F> load_pt(const uint8_t* p) {
-  Affine<F> a;
-  memcpy(&a, p, sizeof a);
-  return a;
-}
-
-bool in_g2_subgroup(const G2Affine& p) {
-  uint32_t r[8];
-  for (int i = 0; i < 8; i++) r[i] = FrParams::mod(i);
-  return xyzz_mul(G2XYZZ::from_affine(p), r).is_inf();
-}
-
 // The points of the key under verification: a bad one is a false verdict (step 1) naming it.
 void check_key_points(const ZkeyIn& z, const std::vector<Rec>& recs) {
   const Fq b1 = curve_b(g1_generator());
@@ -235,48 +190,6 @@ void check_key_points(const ZkeyIn& z, const std::vector<Rec>& recs) {
   } catch (const ApiError& e) {
     throw Verdict{1, -1, e.what()};
   }
-}
-
-void plain_g1(const G1Affine& a, uint8_t* o) {
-  fp_to_bytes(fp_from_mont(a.x), o);
-  fp_to_bytes(fp_from_mont(a.y), o + 32);
-}
-void plain_g2(const G2Affine& a, uint8_t* o) {
-  fp_to_bytes(fp_from_mont(a.x.c0), o);
-  fp_to_bytes(fp_from_mont(a.x.c1), o + 32);
-  fp_to_bytes(fp_from_mont(a.y.c0), o + 64);
-  fp_to_bytes(fp_from_mont(a.y.c1), o + 96);
-}
-
-struct Claims {
-  nzcp_zkey_verify_claim* out;
-  size_t n = 0;
-  void add(int step, int record, const G1Affine& a, const G1Affine& b, const G2Affine& c, const G2Affine& d) {
-    nzcp_zkey_verify_claim& k = out[n++];
-    k.step = step;
-    k.record = record;
-    plain_g1(a, k.a);
-    plain_g1(b, k.b);
-    plain_g2(c, k.c);
-    plain_g2(d, k.d);
-  }
-};
-
-// Sum s_i P_i over n device-resident G1 bases with device-resident plain scalars (the table-free MSM of msm_plan.cu).
-G1Affine msm_g1(void* d_bases, const Fr* d_scalars, size_t n) {
-  if (n == 0) return G1Affine::inf();
-  const int c = msm_pick_window_free(n);
-  MsmTable tab;
-  MsmSort sort;
-  MsmRun run;
-  msm_table_view(&tab, d_bases, n, false, c);
-  msm_sort_create(&sort, n, c, -1, true);
-  msm_run_create(&run, &sort, false);
-  msm_sort_launch(&sort, d_scalars, n, 0);
-  msm_run_launch(&run, &sort, &tab, 0);
-  NZCP_CUDA(cudaStreamSynchronize(0));
-  msm_sort_check(&sort);
-  return xyzz_to_affine(msm_run_finish_g1(&run));
 }
 
 struct Inputs {
@@ -366,15 +279,7 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
 
   // the random scalars: L first, then H
   uint8_t sd[32];
-  if (seed) {
-    memcpy(sd, seed, 32);
-  } else {
-    for (size_t got = 0; got < sizeof sd;) {
-      const ssize_t r = getrandom(sd + got, sizeof sd - got, 0);
-      if (r <= 0) throw ApiError(NZCP_E_INTERNAL, "zkey verify: no OS randomness");
-      got += (size_t)r;
-    }
-  }
+  verify_seed("zkey verify", seed, sd);
   ChaCha rng(sd);
   const uint64_t N = z.domain_size, n_l = z.n_l();
   std::vector<Fr> sc(std::max(n_l, N));
@@ -394,9 +299,9 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
     G1Affine* d_b = l_ex.alloc<G1Affine>(n_l);
     l_ex.upload(d_sc, sc.data(), n_l * sizeof(Fr));
     l_ex.upload(d_b, zi.s[8].p, n_l * 64);
-    const G1Affine r1 = timed(ms[2], [&] { return msm_g1(d_b, d_sc, n_l); });
+    const G1Affine r1 = timed(ms[2], [&] { return msm_sum(ex, d_b, d_sc, n_l); });
     l_ex.upload(d_b, z.s[8].p, n_l * 64);
-    const G1Affine r2 = timed(ms[2], [&] { return msm_g1(d_b, d_sc, n_l); });
+    const G1Affine r2 = timed(ms[2], [&] { return msm_sum(ex, d_b, d_sc, n_l); });
     cl.add(11, -1, r1, r2, delta2, delta2_init);
   }
 
@@ -410,13 +315,13 @@ void verify_checks(const Inputs& in, const uint8_t* init_hash, const uint8_t* se
   ex.upload(d_h, z.s[9].p, N * 64);
   NttDomain dom;
   ntt_domain_create(&dom, (int)in.cir_power, 0);
-  const G1Affine r1 = timed(ms[3], [&] { return msm_g1(diff.d, d_r, N - 1); });
+  const G1Affine r1 = timed(ms[3], [&] { return msm_sum(ex, diff.d, d_r, N - 1); });
   Fr two = Fr::zero();
   two.v[0] = 2;
   const G1Affine r2 = timed(ms[3], [&] {
     ex.run<256>(N, HScalar{d_r, host_fr_root((int)in.cir_power + 1), fp_neg(fp_to_mont(two))});
     ntt_forward(dom, d_r, d_tmp, 0);
-    return msm_g1(d_h, d_r, N);
+    return msm_sum(ex, d_h, d_r, N);
   });
   cl.add(12, -1, r1, r2, delta2, delta2_init);
 }
@@ -440,7 +345,7 @@ void check_out(const Out& o, size_t n_recs) {
 // The key under verification: parsed, its points left to verify_checks.
 void parse_key(Inputs& in, const uint8_t* key, size_t key_len) {
   in.key = parse_zkey_in(key, key_len, false);
-  for (const uint8_t* r : in.key.recs) in.recs.push_back(read_record(r));
+  for (const uint8_t* r : in.key.recs) in.recs.push_back(read_record(r, kRecFixed, "zkey"));
 }
 
 void run(Inputs& in, const uint8_t* init_hash_or_null, const Out& o) {

@@ -460,12 +460,39 @@ def verifyFromInit(initFileName, pTauFileName, zkeyFileName, logger=None, *, see
     return _verify(api.zkey_verify(zkeyFileName, pTauFileName, init=initFileName, seed=seed, device=device), logger)
 
 
+def ptauVerify(tauFilename, logger=None, *, seed=None, device=0):
+    """snarkjs powersOfTau.verify(tauFilename): the contributions, the powers and the next challenge of a phase-1 file and,
+    when prepared, its Lagrange sections (random combinations on the GPU, pairings on the CPU).  Returns a bool; the
+    logger gets snarkjs's lines.  `seed` (32 bytes) replaces the OS randomness: for tests only."""
+    res = api.ptau_verify(tauFilename, seed=seed, device=device)
+    if logger:
+        for i in range(len(res["contributions"]) - 1, -1, -1):
+            c = res["contributions"][i]
+            logger.info("-----------------------------------------------------")
+            logger.info("Contribution #%d: %s" % (i + 1, c["name"]))
+            logger.info(_format_hash(c["next_challenge"], "Next Challenge: "))
+            logger.info(_format_hash(c["response_hash"], "Response Hash: "))
+            if c["type"] == 1:
+                logger.info("Beacon generator: %s" % c["beacon_hash"].hex())
+                logger.info("Beacon iterations Exp: %d" % c["num_iterations_exp"])
+        logger.info("-----------------------------------------------------")
+        if not res["ok"]:
+            logger.error(res["message"])
+        elif not res["prepared"]:
+            logger.warn("this file does not contain phase2 precalculated values. Please run: \n"
+                        "   snarkjs \"powersoftau preparephase2\" to prepare this file to be used in the phase2 ceremony.")
+        if res["ok"]:
+            logger.info("Powers of Tau Ok!")
+    return res["ok"]
+
+
 class powersOfTau:
     """snarkjs.powersOfTau namespace: the entries this library computes."""
     newAccumulator = staticmethod(newAccumulator)
     contribute = staticmethod(ptauContribute)
     beacon = staticmethod(ptauBeacon)
     preparePhase2 = staticmethod(preparePhase2)
+    verify = staticmethod(ptauVerify)
 
 
 class zKey:
